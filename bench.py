@@ -6,6 +6,7 @@
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU arm (oracle port; + the reference
                                                                    #   itself when its checkout is present)
     torchrun ... bench.py --gpus N ...                             # N > 1, one rank per GPU
+    python bench.py --dump-outputs DIR ...                         # + what the timed solve returned (.npy)
 
 Workload (BASELINE.json configs[2], the configuration the metric and target are quoted on):
 net3, coupled SMPS Norton equivalent, fundamental + odd harmonics to the 25th (N = 101),
@@ -38,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the tree may be read-only: no bytecode caches next to the sources
 
 NET, H_MAX, COUPLED, SPREAD = "net3", 25, True, "tight"
 B_PER_GPU = 65536
@@ -377,6 +379,33 @@ def measure_fp64_peak(torch, dev):
 
 
 RESULT_KEYS = ("V_m", "V_a", "I_inj", "n_iter_f", "n_iter_h", "err_h", "status")
+DUMP_BYTES = 60 * 10 ** 6            # --dump-outputs: the sample of scenarios is as large as this allows
+
+
+def dump_outputs(res, dirname):
+    """Write what the timed solve returned (the BatchResult fields, batch innermost) as DIR/<name>.npy,
+    all float64: complex fields as <name>_re / <name>_im, integer fields converted.  Only a fixed,
+    seeded sample of the batch's scenarios is kept (all 65,536 of net3 come to ~70 MB); scenario.npy
+    holds their indices.  Same arguments, same inputs: two builds compare file for file."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for k in RESULT_KEYS:
+        v = getattr(res, k)
+        if v is None:
+            continue
+        if v.is_complex():
+            arrays[k + "_re"], arrays[k + "_im"] = v.real, v.imag
+        else:
+            arrays[k] = v
+    per_scenario = 8 * (1 + sum(v[..., 0].numel() for v in arrays.values()))
+    S = min(res.B, DUMP_BYTES // per_scenario)
+    idx = np.sort(np.random.default_rng(0).choice(res.B, S, replace=False))
+    sel = torch.as_tensor(idx, device=res.status.device)
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, "scenario.npy"), idx.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), v.index_select(-1, sel).to(torch.float64).cpu().numpy())
 
 
 class E2E:
@@ -565,6 +594,8 @@ def run_ours(a):
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = sol.launch_count - l0
+    if a.dump_outputs and rank == 0:
+        dump_outputs(out, a.dump_outputs)
     ms_fund = sum(k[0] for k in kms) / a.steps
     ms_harm = sum(k[1] for k in kms) / a.steps
     conv = int((out.status == 0).sum().item())
@@ -911,7 +942,11 @@ def main():
     ap.add_argument("--no-other", action="store_true", help="skip the other BASELINE configurations")
     ap.add_argument("--no-kernels", action="store_true", help="skip the standalone-kernel rooflines")
     ap.add_argument("--no-exec", action="store_true", help="reference arm: skip timing the reference's own code")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0) as DIR/<name>.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
     if a.impl == "reference":
         run_reference(a)

@@ -3,8 +3,7 @@
 TEST INFRASTRUCTURE ONLY.  Nothing in the product path imports this file.  It
 only works where the reference checkout is mounted (``/root/reference``); it is
 used by ``oracle/make_golden.py`` to generate the committed fixtures under
-``tests/golden/`` and by ``tests/test_oracle_vs_reference.py`` (auto-skipped
-when the reference is absent, e.g. on the GPU box).
+``tests/golden/``; the tests compare against those fixtures.
 
 Nothing is copied: the reference text of
 ``Harmonic Power Flow/hcne_generalized.py`` (``HG``) is read at run time,
