@@ -1043,6 +1043,8 @@ __global__ void bus_currents_kernel(const DevNet net, int B, const double* __res
 #define HPF_HOST_RAMP 4096, 8192, 12288, 16384   // default chunk plan (sizes in scenarios; the last one repeats)
 #define HPF_HOST_RAMP_MIN_B 8192        // smaller batches go in one chunk
 #define HPF_HOST_STREAMS_DEFAULT 2
+#define HPF_LS_AUTO_MIN_B 128           // large networks: batches of at least this many scenarios take the lock-step path
+#define HPF_HW_SERVICE_EPOCH 3          // service interval of finished lanes in the one-warp-per-harmonic kernel (profiles/r2_small_batch_ab.txt)
 struct hpf_handle {
     int device = 0;
     int sm_count = 0;
@@ -1074,10 +1076,6 @@ struct hpf_handle {
     double* d_gstate = nullptr;   // variant 3: per-CTA scenario state slabs
     size_t gstate_doubles = 0;
     size_t wN_elems = 0;
-    int harm_warps = 8;           // warps per 32-scenario tile of the harmonic kernel (8 or 16)
-    int gmem_threads = 0;         // $HPF_GMEM_THREADS: threads per CTA of the global-memory-state kernels (0 = by system size)
-    size_t gmem_cap = 0;          // $HPF_GMEM_SMEM_KB: shared-memory budget per CTA of those kernels (0 = all of it)
-    int harm_minb = 1;
     int no_specialise = 0;        // $HPF_NO_SPECIALISE=1: always use the runtime-dimension kernels
     int mismatch_tile = 0;        // $HPF_MISMATCH_TILE=1: standalone mismatch through the tile kernel
     int gj_single_max = 768;      // $HPF_GJ_SINGLE_MAX: largest order inverted by the one-CTA Gauss-Jordan kernel (tests: 0 forces the multi-CTA paths)
@@ -1085,25 +1083,20 @@ struct hpf_handle {
     int setup_gj = 0;             // $HPF_SETUP=gj: variant 3 set-up by Gauss-Jordan inversion of the whole A_ZZ (round-1 path) instead of the Woodbury form
     int wn_kernel = 0;            // $HPF_WN_KERNEL=fma|dmma: generic w_N = W_NL I_N product on the CUDA-core pipe (wn_tile_kernel) or on the FP64 tensor cores (zgemm_dmma_kernel); 0 = default
     int lu_classic = 0;           // $HPF_LU_CLASSIC=1: shared-memory LU with rank-1 updates (lu_solve_smem) instead of the panel LU
-    int dense_blocked = 0;        // $HPF_DENSE_BLOCKED=1: blocked tensor-core LU also for smem-sized systems
     int force_variant = 0;        // $HPF_STRUCT_VARIANT=2|3: force a per-CTA variant of the harmonic stage
     // lock-step batched harmonic stage of the large networks (hpf_lockstep.cuh)
-    int lockstep = -1;            // $HPF_LOCKSTEP=0|1: never / always; default (-1): batches of at least lockstep_min scenarios
-    int lockstep_min = 128;
+    int lockstep = -1;            // $HPF_LOCKSTEP=0|1: never / always; default (-1): batches of at least HPF_LS_AUTO_MIN_B scenarios
     size_t ls_budget = 0;         // $HPF_LOCKSTEP_GB: device memory the lock-step work areas may take (0 = 40 % of the free memory, at most 64 GB)
     void* d_ls = nullptr;         // one allocation: state slabs | border systems | X | GX | U0 | ints
     size_t ls_bytes = 0;
     int ls_slots = 0;
     int last_path = 0;            // hpf_last_solve_path
-    int ls_upd = 0;               // $HPF_LS_UPD=big|direct: rank-64 update with 128 x 64 tiles of 8 warps, 2 CTAs per SM (1) / barrier-free, fragments straight from L1 / L2 (2); default: 64 x 64 tiles of 4 warps, 3 CTAs per SM (A/B: profiles/r2_lockstep_ab.txt)
-    int ls_no_pair = 0;           // $HPF_LS_NO_PAIR=1: rank-32 update after every panel (A/B against the paired rank-64 update)
     // host mirror of the network constants for kernels that take them as parameters
     // (constant bank): fetched lazily from the device tables, see host_consts()
     std::vector<double2> hY, hYN, hWNL, hG;
     std::vector<char> hw_consts;  // HwConsts<D, coupled> of the one-warp-per-harmonic kernel (hw_shape != 0)
     int hw_shape = 0;             // 0 none, 1 = Dims<4,3,2,13,1>, 2 = Dims<4,2,1,10,2>
     int harm_tile_only = 0;       // $HPF_HARM_KERNEL=tile: 32-scenario tile kernel instead (A/B measurements)
-    int hw_epoch = 3;             // $HPF_HW_EPOCH: service interval of finished lanes in the one-warp-per-harmonic kernel
     int hw_minb = 2;              // $HPF_HW_MINB: register budget of the one-warp-per-harmonic kernel (CTAs per SM)
     int max_ctas = 0;             // $HPF_MAX_CTAS: cap on the grid of the persistent kernels (tests: forces queue refills on small batches)
     std::vector<int> hdev;
@@ -1219,30 +1212,12 @@ static bool fits_smem_lu(const hpf_t* h, const DevNet& net) {
            scn_smem_bytes(net.n, net.H, net.q, net.N, true) <= (size_t)h->smem_optin;
 }
 
-// Blocked tensor-core LU on a matrix that still fits shared memory (N <= 192): chosen with
-// $HPF_DENSE_BLOCKED=1 instead of the classic shared-memory LU.  Returns the LU work area in
-// doubles (even), or 0 if it does not fit.
-static size_t smem_blocked_lub_doubles(const hpf_t* h, const DevNet& net) {
-    if (!h->dense_blocked) return 0;
-    const size_t state = scn_smem_doubles_aligned(net.n, net.H, net.q, net.N);
-    const size_t mat = (size_t)lub_ld(net.N) * (net.N + 1);
-    const size_t cap = (size_t)h->smem_optin / sizeof(double);
-    if (state + mat + LUB_SMEM_DOUBLES + 4 > cap) return 0;
-    size_t lubd = lub_smem_doubles_for(net.N, (cap - state - mat - 4) * sizeof(double));
-    return lubd & ~(size_t)1;
-}
-
 static int ensure_workspace(hpf_t* h, size_t doubles) {
     if (doubles <= h->work_doubles) return HPF_OK;
     if (h->d_work) { CK(cudaDeviceSynchronize()); cudaFree(h->d_work); h->d_work = nullptr; h->work_doubles = 0; }
     CK(cudaMalloc((void**)&h->d_work, doubles * sizeof(double)));
     h->work_doubles = doubles;
     return HPF_OK;
-}
-
-// shared-memory budget per CTA of the global-memory-state kernels ($HPF_GMEM_SMEM_KB; default: all of it)
-static size_t gmem_smem_cap(const hpf_t* h) {
-    return (h->gmem_cap && h->gmem_cap < (size_t)h->smem_optin) ? h->gmem_cap : (size_t)h->smem_optin;
 }
 
 template <class K>
@@ -1286,23 +1261,15 @@ static int solve_common(hpf_t* h, int mode, int B, const double* P, const double
         net.H = 1; net.nH = net.n;
         gm = !fits_smem_lu(h, net);
     }
-    const size_t lubs = gm ? 0 : smem_blocked_lub_doubles(h, net);     // > 0: blocked LU, matrix in smem
-    const bool ws_smem = lubs > 0;
-    if (ws_smem) gm = true;
-    // the reduced budget / thread count of $HPF_GMEM_* applies when the scenario state leaves room for the LU work area
-    const bool reduced = gm && !ws_smem &&
-                         gmem_kernel_smem_bytes(net.n, net.H, net.q, net.N) + 32 * 1024 <= gmem_smem_cap(h);
-    const size_t lubd = ws_smem ? lubs : (gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N,
-                                                                      reduced ? gmem_smem_cap(h) : (size_t)h->smem_optin) : 0);
-    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd +
-                              (ws_smem ? (size_t)lub_ld(net.N) * (net.N + 1) : 0)) * sizeof(double) + 16
+    // gm: matrix in a per-CTA global workspace, scenario state + blocked-LU staging in shared memory
+    const size_t lubd = gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin) : 0;
+    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd) * sizeof(double) + 16
                            : scn_smem_bytes(net.n, net.H, net.q, net.N, true);
     int occ = 0;
     const bool big = gm && lub_needs_big(net.N, lubd);
-    const int gthreads = (reduced && h->gmem_threads) ? h->gmem_threads : HPF_THREADS_GMEM;
     rc = !gm ? prep_kernel(h, solve_kernel<0>, smem, who, &occ)
-             : big ? prep_kernel(h, solve_kernel<2>, smem, who, &occ, gthreads)
-                   : prep_kernel(h, solve_kernel<1>, smem, who, &occ, gthreads);
+             : big ? prep_kernel(h, solve_kernel<2>, smem, who, &occ, HPF_THREADS_GMEM)
+                   : prep_kernel(h, solve_kernel<1>, smem, who, &occ, HPF_THREADS_GMEM);
     if (rc) return rc;
     SolveArgs a;
     a.B = B; a.mode = mode; a.flags = flags; a.P = P; a.Q = Q; a.I_N = (const double2*)I_N;
@@ -1318,15 +1285,15 @@ static int solve_common(hpf_t* h, int mode, int B, const double* P, const double
     if (grid > B) grid = B;
     if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
     a.workspace = nullptr;
-    if (gm && !ws_smem) {
+    if (gm) {
         rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
         if (rc) return rc;
         a.workspace = h->d_work;
     }
     if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
     if (!gm) solve_kernel<0><<<(unsigned)grid, HPF_THREADS, smem, st>>>(net, a);
-    else if (big) solve_kernel<2><<<(unsigned)grid, gthreads, smem, st>>>(net, a);
-    else solve_kernel<1><<<(unsigned)grid, gthreads, smem, st>>>(net, a);
+    else if (big) solve_kernel<2><<<(unsigned)grid, HPF_THREADS_GMEM, smem, st>>>(net, a);
+    else solve_kernel<1><<<(unsigned)grid, HPF_THREADS_GMEM, smem, st>>>(net, a);
     if (net.H != H_full) {
         const size_t cnt = (size_t)(H_full - 1) * net.n * B;
         flat_start_fill_kernel<<<(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st>>>(
@@ -1359,8 +1326,9 @@ static int launch_zgemm(hpf_t* h, int M, int N, int K, const double2* A, size_t 
                         double2* C, size_t ldc, cudaStream_t st, bool subtract = false, const int* n_dev = nullptr);
 
 // In-place complex Gauss-Jordan inverse with partial pivoting of one matrix of order nn (row-major):
-// one CTA for nn <= 768, else four small launches per pivot over the whole GPU.  info[0] = 0 or
-// k + 1 (zero pivot), pr[0..1] = min / max pivot modulus.  ipiv: nn ints, tmp: 2 nn + 1 double2.
+// one CTA for nn <= gj_single_max (768), else four small launches per pivot over the whole GPU.  info[0] = 0
+// or k + 1 (zero pivot), pr[0..1] = min / max pivot modulus.  ipiv: nn ints, tmp: 2 nn + 1 double2 (only
+// read for nn > gj_single_max).
 static int gj_invert(hpf_t* h, double2* A, int nn, int* ipiv, int* info, double* pr, double2* tmp, cudaStream_t st,
                      double2* FR = nullptr) {
     if (nn <= h->gj_single_max) {
@@ -1574,7 +1542,7 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
     const int nZ = net.nH - net.m;
     if (nZ < 1) return HPF_OK;
     int variant = 1;
-    if (harm_tile_smem_bytes(net.n, net.H, net.m, net.c, net.q, h->harm_warps,
+    if (harm_tile_smem_bytes(net.n, net.H, net.m, net.c, net.q, 8,
                              h->n_dev * (h->coupled ? h->H * h->H : h->H)) > (size_t)h->smem_optin ||
         fund_tile_doubles_per_warp(net.n, net.Nf) * sizeof(double) > (size_t)h->smem_optin)
         variant = 2;
@@ -1660,24 +1628,9 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
     SK(pr, 2 * sizeof(double), true);
     struct_assemble_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, h->d_Ainv, AZF);
     h->launches++;
-    if (nZ <= 768) {
-        cinv_gj_kernel<<<1, 1024, 0, st>>>(nZ, h->d_Ainv, ipiv, ipiv + nZ, pr);
-        h->launches++;
-    } else {
-        SK(tmp, ((size_t)2 * nZ + 1) * sizeof(double2), true);
-        double2 *rowk = tmp, *colk = tmp + nZ, *pinv = tmp + 2 * (size_t)nZ;
-        const int g1 = (nZ + 255) / 256;
-        int gy = (h->sm_count * 8 + g1 - 1) / g1;
-        if (gy > nZ) gy = nZ;
-        for (int k = 0; k < nZ; ++k) {
-            gjm_pivot_kernel<<<1, 1024, 0, st>>>(nZ, k, h->d_Ainv, ipiv, ipiv + nZ, pr, pinv);
-            gjm_row_kernel<<<g1, 256, 0, st>>>(nZ, k, h->d_Ainv, ipiv, pinv, rowk);
-            gjm_col_kernel<<<g1, 256, 0, st>>>(nZ, k, h->d_Ainv, colk);
-            gjm_elim_kernel<<<dim3(g1, gy), 256, 0, st>>>(nZ, k, h->d_Ainv, rowk, colk);
-        }
-        gjm_unpermute_kernel<<<g1, 256, 0, st>>>(nZ, h->d_Ainv, ipiv);
-        h->launches += 4LL * nZ + 1;
-    }
+    if (nZ > h->gj_single_max) SK(tmp, ((size_t)2 * nZ + 1) * sizeof(double2), true);
+    const int rcg = gj_invert(h, h->d_Ainv, nZ, ipiv, ipiv + nZ, pr, tmp, st);
+    if (rcg) return rcg;
     {
         const size_t tot = (size_t)nZ * net.m;
         struct_G_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(nZ, net.m, net.q < nZ ? net.q : nZ,
@@ -1843,12 +1796,12 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
                        bool persistent, cudaStream_t st) {
     if (h->struct_state >= 2) {
         const bool gst = h->struct_state == 3;
-        const size_t lubd = gst ? harm_cta_gmem_lub_doubles(sn.nx, gmem_smem_cap(h)) : 0;
+        const size_t lubd = gst ? harm_cta_gmem_lub_doubles(sn.nx, (size_t)h->smem_optin) : 0;
         // threads per CTA: every phase of this kernel is barrier- / latency-bound, and a border system whose
         // panels fit one row per thread of 8 warps runs faster with 8 warps than with 16 (measured, 200-bus
         // feeder, nx = 238: 217 -> 183 ms per 2,048 scenarios; 1000-bus network, nx = 1198: 2.40 -> 2.78 s
         // the other way round) - profiles/r2_gmem_ctas_ab.txt
-        const int gthreads = h->gmem_threads ? h->gmem_threads : (sn.nx <= 256 ? 256 : HPF_THREADS_GMEM);
+        const int gthreads = sn.nx <= 256 ? 256 : HPF_THREADS_GMEM;
         const size_t smem = gst ? (lubd + 80) * sizeof(double)
                                 : harm_cta_smem_bytes(net.n, net.H, net.m, net.c, net.q, net.N);
         int occ = 0;
@@ -1937,7 +1890,7 @@ static LsTimer g_ls_timer;
 static bool use_lockstep(const hpf_t* h, const StructNet& sn, int B) {
     if (h->struct_state != 3 || h->lockstep == 0) return false;
     if (sn.nx < 1 || sn.nx > 2048) return false;             // panel kernel: at most 4 rows per thread of 512
-    return h->lockstep == 1 || B >= h->lockstep_min;
+    return h->lockstep == 1 || B >= HPF_LS_AUTO_MIN_B;
 }
 
 template <class K>
@@ -2005,13 +1958,7 @@ static int launch_ls_lu(hpf_t* h, const LsArgs& la, int cur, int N, int nwave, c
             kernel<<<grid, NT, usm, st>>>(la, cur, N, kb, rlo, clo, chi);
             return HPF_OK;
         };
-        if (K == 64 && h->ls_upd == 2) {
-            const long long nsr = (N - rlo + 31) / 32, nsc = (chi + 1 - clo + 31) / 32;
-            rc = ls_grid(h, ls_update_direct_kernel<64>, 128, 0, ((long long)nwave * nsr * nsc + 3) / 4, &grid);
-            if (rc) return rc;
-            ls_update_direct_kernel<64><<<grid, 128, 0, st>>>(la, cur, N, kb, rlo, clo, chi);
-        } else if (K == 64) rc = h->ls_upd == 1 ? go(ls_update_kernel<64, 128, 64, 256, 2>, 128, 64, 256)
-                                                : go(ls_update_kernel<64, 64, 64, 128, 3>, 64, 64, 128);
+        if (K == 64) rc = go(ls_update_kernel<64, 64, 64, 128, 3>, 64, 64, 128);
         else rc = go(ls_update_kernel<32, 128, 128, 256, 2>, 128, 128, 256);
         if (rc) return rc;
         g_ls_timer.mark(6);
@@ -2021,7 +1968,7 @@ static int launch_ls_lu(hpf_t* h, const LsArgs& la, int cur, int N, int nwave, c
     int rc;
     for (int k0 = 0; k0 < N;) {
         const int rows = N - k0, nb = rows < LS_NB ? rows : LS_NB, cr = k0 + nb;
-        const bool pair = nb == LS_NB && N - cr >= LS_NB && !h->ls_no_pair;
+        const bool pair = nb == LS_NB && N - cr >= LS_NB;
         if ((rc = panel(k0, 0))) return rc;
         if ((rc = swap_trsm(k0, 0))) return rc;
         if (!pair) {
@@ -2135,7 +2082,7 @@ static bool use_lockstep_fund(const hpf_t* h, int B) {
     if (h->struct_state != 3 || h->lockstep == 0) return false;
     const int Nf = 2 * h->n - 1 - h->c;
     if (Nf < 1 || Nf > 2048) return false;
-    return h->lockstep == 1 || B >= h->lockstep_min;
+    return h->lockstep == 1 || B >= HPF_LS_AUTO_MIN_B;
 }
 
 static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* Q, double thresh_f, int max_f,
@@ -2337,7 +2284,7 @@ static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, c
         ha.wN = h->d_wN + h->wN_off;
         ha.thresh_h = thresh_h; ha.max_h = max_h; ha.V_m = V_m; ha.V_a = V_a; ha.I_inj = (double2*)I_inj;
         ha.n_iter_h = n_iter_h; ha.status = status; ha.err_h = err_h; ha.work_counter = h->d_counter + h->cur_slot;
-        ha.dx_out = nullptr; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0; ha.hist_h = hist_h; ha.epoch = h->hw_epoch;
+        ha.dx_out = nullptr; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0; ha.hist_h = hist_h; ha.epoch = HPF_HW_SERVICE_EPOCH;
         const bool ls = use_lockstep(h, sn, B);
         rc = ls ? launch_lockstep(h, net, sn, ha, st) : launch_harm(h, net, sn, ha, true, st);
         if (rc) return rc;
@@ -2412,28 +2359,19 @@ int hpf_create(hpf_t** out, int device) {
         delete h;
         return fail(nullptr, HPF_E_UNSUPPORTED, "hpf_create: this library is built for sm_100a (B200) only");
     }
-    if (const char* ev = getenv("HPF_HARM_WARPS")) h->harm_warps = (atoi(ev) == 16) ? 16 : 8;
-    if (const char* ev = getenv("HPF_HARM_MINB")) h->harm_minb = (atoi(ev) == 2) ? 2 : 1;
     if (const char* ev = getenv("HPF_NO_SPECIALISE")) h->no_specialise = atoi(ev) ? 1 : 0;
     if (const char* ev = getenv("HPF_MISMATCH_TILE")) h->mismatch_tile = atoi(ev) ? 1 : 0;
     if (const char* ev = getenv("HPF_STRUCT_VARIANT")) h->force_variant = atoi(ev);
     if (const char* ev = getenv("HPF_LOCKSTEP")) h->lockstep = atoi(ev) ? 1 : 0;
-    if (const char* ev = getenv("HPF_LS_UPD")) h->ls_upd = (strcmp(ev, "big") == 0) ? 1 : (strcmp(ev, "direct") == 0) ? 2 : 0;
-    if (const char* ev = getenv("HPF_LS_NO_PAIR")) h->ls_no_pair = atoi(ev) ? 1 : 0;
-    if (const char* ev = getenv("HPF_LOCKSTEP_MIN")) h->lockstep_min = atoi(ev) > 0 ? atoi(ev) : 1;
     if (const char* ev = getenv("HPF_LOCKSTEP_GB")) h->ls_budget = (size_t)(atof(ev) > 0 ? atof(ev) * 1073741824.0 : 0);
-    if (const char* ev = getenv("HPF_DENSE_BLOCKED")) h->dense_blocked = atoi(ev) ? 1 : 0;
     if (const char* ev = getenv("HPF_LU_CLASSIC")) h->lu_classic = atoi(ev) ? 1 : 0;
     if (const char* ev = getenv("HPF_GJ_SINGLE_MAX")) h->gj_single_max = atoi(ev);
     if (const char* ev = getenv("HPF_GJ_UNBLOCKED")) h->gj_unblocked = atoi(ev) ? 1 : 0;
     if (const char* ev = getenv("HPF_SETUP")) h->setup_gj = (strcmp(ev, "gj") == 0) ? 1 : 0;
     if (const char* ev = getenv("HPF_WN_KERNEL")) h->wn_kernel = (strcmp(ev, "dmma") == 0) ? 2 : (strcmp(ev, "fma") == 0) ? 1 : 0;
     if (const char* ev = getenv("HPF_HARM_KERNEL")) h->harm_tile_only = (strcmp(ev, "tile") == 0) ? 1 : 0;
-    if (const char* ev = getenv("HPF_HW_EPOCH")) h->hw_epoch = atoi(ev) >= 1 ? atoi(ev) : 1;
     if (const char* ev = getenv("HPF_HW_MINB")) h->hw_minb = (atoi(ev) == 1) ? 1 : 2;
     if (const char* ev = getenv("HPF_MAX_CTAS")) h->max_ctas = atoi(ev) > 0 ? atoi(ev) : 0;
-    if (const char* ev = getenv("HPF_GMEM_THREADS")) { const int t = atoi(ev); if (t == 128 || t == 256 || t == 512) h->gmem_threads = t; }
-    if (const char* ev = getenv("HPF_GMEM_SMEM_KB")) h->gmem_cap = (size_t)(atoi(ev) > 0 ? atoi(ev) : 0) * 1024;
     h->sm_count = prop.multiProcessorCount;
     h->smem_optin = (int)prop.sharedMemPerBlockOptin;
     e = cudaMalloc((void**)&h->d_counter, HPF_HOST_MAX_CHUNKS * sizeof(int));
@@ -2820,7 +2758,8 @@ int hpf_fund_solve(hpf_t* h, int B, const double* P, const double* Q, double thr
 // Chunk plan of hpf_solve_host: boundaries cb[0..nchunk] (multiples of 32 scenarios except the end) and
 // the number of compute streams the chunks rotate over.  $HPF_HOST_PLAN = comma-separated chunk sizes
 // (the last size repeats until the batch is covered; at most HPF_HOST_MAX_CHUNKS chunks, the last one
-// takes the rest), $HPF_HOST_CHUNKS = number of equal chunks, $HPF_HOST_STREAMS = 1..4 compute streams.
+// takes the rest), else HPF_HOST_RAMP for batches of at least HPF_HOST_RAMP_MIN_B, else one chunk;
+// $HPF_HOST_STREAMS = 1..4 compute streams.
 static int host_chunk_plan(size_t Bs, size_t* cb, int* streams) {
     static const size_t ramp_default[] = {HPF_HOST_RAMP};
     size_t sizes[HPF_HOST_MAX_CHUNKS];
@@ -2835,16 +2774,9 @@ static int host_chunk_plan(size_t Bs, size_t* cb, int* streams) {
             if (*end != ',') break;
         }
     }
-    int equal = 0;
-    if (const char* ev = getenv("HPF_HOST_CHUNKS")) { const int v = atoi(ev); if (v >= 1 && v <= HPF_HOST_MAX_CHUNKS) equal = v; }
-    if (ns == 0 && equal == 0) {
-        if (Bs >= HPF_HOST_RAMP_MIN_B) {
-            for (size_t i = 0; i < sizeof(ramp_default) / sizeof(ramp_default[0]); ++i) sizes[ns++] = ramp_default[i];
-        } else {
-            equal = 1;
-        }
-    }
-    if (ns == 0) { sizes[0] = (Bs + equal - 1) / equal; ns = 1; }
+    if (ns == 0 && Bs >= HPF_HOST_RAMP_MIN_B)
+        for (size_t i = 0; i < sizeof(ramp_default) / sizeof(ramp_default[0]); ++i) sizes[ns++] = ramp_default[i];
+    if (ns == 0) { sizes[0] = Bs; ns = 1; }
     int k = 0;
     size_t b = 0;
     cb[0] = 0;
@@ -2856,7 +2788,6 @@ static int host_chunk_plan(size_t Bs, size_t* cb, int* streams) {
     }
     int st = HPF_HOST_STREAMS_DEFAULT;
     if (const char* ev = getenv("HPF_HOST_STREAMS")) { const int v = atoi(ev); if (v >= 1 && v <= 4) st = v; }
-    if (getenv("HPF_HOST_SINGLE_STREAM")) st = 1;
     *streams = st;
     return k;
 }
@@ -3138,13 +3069,9 @@ static int lu_solve_impl(hpf_t* h, int B, const double* J, const double* f, doub
     const DevNet net = devnet(h);
     LuArgs a;
     a.B = B; a.J = J; a.f = f; a.dx = dx; a.info = info; a.stride = hpf_jacobian_stride(h);
-    bool gm = !fits_smem_lu(h, net);
-    const size_t lubs = gm ? 0 : smem_blocked_lub_doubles(h, net);
-    const bool ws_smem = lubs > 0;
-    if (ws_smem) gm = true;
-    const size_t lubd = ws_smem ? lubs : (gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin) : 0);
-    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd +
-                              (ws_smem ? (size_t)lub_ld(net.N) * (net.N + 1) : 0)) * sizeof(double) + 16
+    const bool gm = !fits_smem_lu(h, net);
+    const size_t lubd = gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin) : 0;
+    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd) * sizeof(double) + 16
                            : scn_smem_bytes(net.n, net.H, net.q, net.N, true);
     a.lub_doubles = (int)lubd;
     a.lu_classic = h->lu_classic;
@@ -3154,17 +3081,15 @@ static int lu_solve_impl(hpf_t* h, int B, const double* J, const double* f, doub
              : big ? prep_kernel(h, lu_solve_kernel<2>, smem, "hpf_lu_solve", &occ, HPF_THREADS_GMEM)
                    : prep_kernel(h, lu_solve_kernel<1>, smem, "hpf_lu_solve", &occ, HPF_THREADS_GMEM);
     if (rc) return rc;
-    if (gm && !ws_smem && net.N <= 2048 && (h->lockstep == 1 || (h->lockstep != 0 && B >= h->lockstep_min)))
+    if (gm && net.N <= 2048 && (h->lockstep == 1 || (h->lockstep != 0 && B >= HPF_LS_AUTO_MIN_B)))
         return lu_solve_batched(h, net.N, B, J, a.stride, f, dx, info, (cudaStream_t)stream);
     long long grid = (long long)occ * h->sm_count;
     if (grid > B) grid = B;
     a.workspace = nullptr;
     if (gm) {
-        if (!ws_smem) {
-            rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
-            if (rc) return rc;
-            a.workspace = h->d_work;
-        }
+        rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
+        if (rc) return rc;
+        a.workspace = h->d_work;
         if (big) lu_solve_kernel<2><<<(unsigned)grid, HPF_THREADS_GMEM, smem, (cudaStream_t)stream>>>(net, a);
         else lu_solve_kernel<1><<<(unsigned)grid, HPF_THREADS_GMEM, smem, (cudaStream_t)stream>>>(net, a);
     } else {

@@ -802,87 +802,6 @@ ls_update_kernel(const LsArgs a, const int cur, const int N, const int kb, const
     }
 }
 
-// step 3, barrier-free variant ($HPF_LS_UPD=direct): every WARP takes its own 32 x 32 sub-tiles and reads
-// the L / U fragments straight from global memory (read-only path, served by L1 / L2: a fragment load of
-// a warp covers whole 32-byte sectors) one k step ahead of the DMMAs - no shared memory, no block
-// barrier, warps of a CTA run on consecutive column sub-tiles of one row block (they share its L slice).
-template <int K>
-__global__ void __launch_bounds__(128, 3)
-ls_update_direct_kernel(const LsArgs a, const int cur, const int N, const int kb, const int rlo, const int clo, const int chi) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int ld = a.ldb;
-    const int nact = a.nact[cur];
-    const int* act = a.act + (size_t)cur * a.S;
-    const int nsr = (N - rlo + 31) / 32, nsc = (chi + 1 - clo + 31) / 32;
-    const long long items = (long long)nact * nsr * nsc;
-    long long per = (items + gridDim.x - 1) / gridDim.x;
-    per = (per + 3) & ~3LL;
-    const long long w0 = (long long)blockIdx.x * per, w1 = (w0 + per < items) ? w0 + per : items;
-    const int fr = lane >> 2, fk = lane & 3;
-    for (long long w = w0 + warp; w < w1; w += 4) {
-        const long long key = w / nsc;
-        const int sc = (int)(w - key * nsc);
-        const int ai = (int)(key / nsr), sr = (int)(key - (long long)ai * nsr);
-        double* A = a.M + (size_t)act[ai] * a.mat_stride;
-        const int rbb = rlo + sr * 32, cb = clo + sc * 32;
-        bool cok[4], rok[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) { cok[i] = cb + 8 * i + fr <= chi; rok[i] = rbb + 8 * i + fr < N; }
-        const double* pu = A + (size_t)(cb + fr) * ld + kb + fk;          // af[ic] = pu[8 ic ld + kk]
-        const double* pl = A + (size_t)(kb + fk) * ld + rbb + fr;         // bf[ir] = pl[kk ld + 8 ir]
-        double af[4], bf[4], an[4], bn[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            af[i] = cok[i] ? __ldg(pu + (size_t)(8 * i) * ld) : 0.0;
-            bf[i] = rok[i] ? __ldg(pl + 8 * i) : 0.0;
-        }
-        double acc[4][4][2];
-#pragma unroll
-        for (int ic = 0; ic < 4; ++ic)
-#pragma unroll
-            for (int ir = 0; ir < 4; ++ir) {
-                const int cc = cb + 8 * ic + fr, r = rbb + 8 * ir + 2 * fk;
-                if (cc <= chi && r + 1 < N) {
-                    const double2 v2 = *reinterpret_cast<const double2*>(A + (size_t)cc * ld + r);
-                    acc[ic][ir][0] = v2.x; acc[ic][ir][1] = v2.y;
-                } else {
-                    acc[ic][ir][0] = (cc <= chi && r < N) ? A[(size_t)cc * ld + r] : 0.0;
-                    acc[ic][ir][1] = 0.0;
-                }
-            }
-#pragma unroll
-        for (int kk = 0; kk < K; kk += 4) {
-            if (kk + 4 < K) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    an[i] = cok[i] ? __ldg(pu + (size_t)(8 * i) * ld + kk + 4) : 0.0;
-                    bn[i] = rok[i] ? __ldg(pl + (size_t)(kk + 4) * ld + 8 * i) : 0.0;
-                }
-            }
-#pragma unroll
-            for (int ir = 0; ir < 4; ++ir)
-                bf[ir] = __hiloint2double(__double2hiint(bf[ir]) ^ (int)0x80000000, __double2loint(bf[ir]));
-#pragma unroll
-            for (int ic = 0; ic < 4; ++ic)
-#pragma unroll
-                for (int ir = 0; ir < 4; ++ir) dmma884(acc[ic][ir][0], acc[ic][ir][1], af[ic], bf[ir]);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) { af[i] = an[i]; bf[i] = bn[i]; }
-        }
-#pragma unroll
-        for (int ic = 0; ic < 4; ++ic)
-#pragma unroll
-            for (int ir = 0; ir < 4; ++ir) {
-                const int cc = cb + 8 * ic + fr, r = rbb + 8 * ir + 2 * fk;
-                if (cc <= chi && r + 1 < N) {
-                    *reinterpret_cast<double2*>(A + (size_t)cc * ld + r) = make_double2(acc[ic][ir][0], acc[ic][ir][1]);
-                } else if (cc <= chi && r < N) {
-                    A[(size_t)cc * ld + r] = acc[ic][ir][0];
-                }
-            }
-    }
-}
-
 // step 4: blocked back substitution U x = y (y = column N), one CTA per matrix
 __global__ void __launch_bounds__(256)
 ls_backsub_kernel(const LsArgs a, const int cur, const int N) {

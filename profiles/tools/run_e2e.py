@@ -1,4 +1,4 @@
-"""hpf_solve_host end to end (pinned host buffers) for config 3 - chunk-count sweep via $HPF_HOST_CHUNKS."""
+"""hpf_solve_host end to end (pinned host buffers) for config 3 - chunk-plan sweep via $HPF_HOST_PLAN."""
 import os, sys, tempfile, time
 R = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 for p in (R, os.path.join(R, "tests"), os.path.join(R, "oracle")):
@@ -15,5 +15,5 @@ for _ in range(3):
 best = 1e9
 for _ in range(10):
     t0 = time.perf_counter(); r = sol.solve_host(hP, hQ, hI); best = min(best, time.perf_counter() - t0)
-print("chunks=%s B=%d solve_host best %.3f ms (%.1f M solves/s) conv %d" % (os.environ.get("HPF_HOST_CHUNKS", "default"), B, best * 1e3,
+print("plan=%s B=%d solve_host best %.3f ms (%.1f M solves/s) conv %d" % (os.environ.get("HPF_HOST_PLAN", "default"), B, best * 1e3,
       B / best / 1e6, int((r["status"] == 0).sum())))

@@ -1,5 +1,5 @@
 """Kernel 4 standalone (hpf_lu_solve) on config-3 Jacobians - target of ncu captures / A-B timings.
-usage: run_lu.py [B] [reps]   env: HPF_LU_CLASSIC=1 (rank-1 LU), HPF_DENSE_BLOCKED=1 (DMMA blocked LU)"""
+usage: run_lu.py [B] [reps]   env: HPF_LU_CLASSIC=1 (rank-1 LU)"""
 import os
 import sys
 import tempfile

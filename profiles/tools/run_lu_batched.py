@@ -1,6 +1,6 @@
 """Batched LU of hpf_lockstep.cuh standalone (hpf_lu_solve with $HPF_LOCKSTEP=1) on random systems of
 order N = 1038 (net1, H <= 51) - target of ncu captures / A-B timings of the panel / interchange /
-tensor-core update kernels.  usage: run_lu_batched.py [B] [reps]   env: HPF_LS_NO_PAIR=1"""
+tensor-core update kernels.  usage: run_lu_batched.py [B] [reps]"""
 import os
 import sys
 import tempfile

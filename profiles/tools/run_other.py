@@ -1,5 +1,5 @@
 """One of the large BASELINE configurations (radial200 / meshed1000) on cuda:0: set-up + timed solves.
-usage: run_other.py kind B reps   env: HPF_GMEM_THREADS, HPF_GMEM_SMEM_KB (CTAs per SM of the per-CTA kernels)"""
+usage: run_other.py kind B reps"""
 import os, sys, time
 R = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 for p in (R, os.path.join(R, "tests"), os.path.join(R, "oracle")):
@@ -22,6 +22,6 @@ for _ in range(reps):
     k = sol.last_kernel_ms(); ms = e0.elapsed_time(e1)
     if best is None or ms < best[0]: best = (ms, k)
 it = r.n_iter_h.double()
-print("%s B=%d threads=%s smemKB=%s setup %.2fs step %.1f ms (fund %.1f harm %.1f) %.1f solves/s mean it %.2f conv %d checksum %.13e" % (
-    kind, B, os.environ.get("HPF_GMEM_THREADS", "512"), os.environ.get("HPF_GMEM_SMEM_KB", "all"), ts, best[0], best[1][0], best[1][1],
+print("%s B=%d setup %.2fs step %.1f ms (fund %.1f harm %.1f) %.1f solves/s mean it %.2f conv %d checksum %.13e" % (
+    kind, B, ts, best[0], best[1][0], best[1][1],
     B / best[0] * 1e3, it.mean().item(), int((r.status == 0).sum().item()), float(r.V_m.sum())))
