@@ -1044,6 +1044,7 @@ __global__ void bus_currents_kernel(const DevNet net, int B, const double* __res
 #define HPF_HOST_RAMP_MIN_B 8192        // smaller batches go in one chunk
 #define HPF_HOST_STREAMS_DEFAULT 2
 #define HPF_LS_AUTO_MIN_B 128           // large networks: batches of at least this many scenarios take the lock-step path
+#define HPF_LS_MAX_ORDER 2048           // largest system of the lock-step LU (panel kernel: at most 4 rows per thread of 512)
 #define HPF_HW_SERVICE_EPOCH 3          // service interval of finished lanes in the one-warp-per-harmonic kernel (profiles/r2_small_batch_ab.txt)
 struct hpf_handle {
     int device = 0;
@@ -1077,6 +1078,8 @@ struct hpf_handle {
     size_t gstate_doubles = 0;
     size_t wN_elems = 0;
     int no_specialise = 0;        // $HPF_NO_SPECIALISE=1: always use the runtime-dimension kernels
+    int shape = 0;                // shape-specialised instances of the network (see with_shape), 0 = none
+    int fund_shape = 0;           // the same for fund_tile_kernel, matched on (n, c) only: it reads no other dimension
     int mismatch_tile = 0;        // $HPF_MISMATCH_TILE=1: standalone mismatch through the tile kernel
     int gj_single_max = 768;      // $HPF_GJ_SINGLE_MAX: largest order inverted by the one-CTA Gauss-Jordan kernel (tests: 0 forces the multi-CTA paths)
     int gj_unblocked = 0;         // $HPF_GJ_UNBLOCKED=1: multi-CTA Gauss-Jordan with one rank-1 update of the whole matrix per pivot (round-1 kernel) instead of the blocked one
@@ -1094,10 +1097,8 @@ struct hpf_handle {
     // host mirror of the network constants for kernels that take them as parameters
     // (constant bank): fetched lazily from the device tables, see host_consts()
     std::vector<double2> hY, hYN, hWNL, hG;
-    std::vector<char> hw_consts;  // HwConsts<D, coupled> of the one-warp-per-harmonic kernel (hw_shape != 0)
-    int hw_shape = 0;             // 0 none, 1 = Dims<4,3,2,13,1>, 2 = Dims<4,2,1,10,2>
+    std::vector<char> hw_consts;  // HwConsts<D, coupled> of the one-warp-per-harmonic kernel (empty: not built)
     int harm_tile_only = 0;       // $HPF_HARM_KERNEL=tile: 32-scenario tile kernel instead (A/B measurements)
-    int hw_minb = 2;              // $HPF_HW_MINB: register budget of the one-warp-per-harmonic kernel (CTAs per SM)
     int max_ctas = 0;             // $HPF_MAX_CTAS: cap on the grid of the persistent kernels (tests: forces queue refills on small batches)
     std::vector<int> hdev;
     bool host_consts_valid = false;
@@ -1236,6 +1237,49 @@ static int prep_kernel(hpf_t* h, K kernel, size_t smem, const char* who, int* ct
     return HPF_OK;
 }
 
+// Shape-specialised instances exist for the BASELINE configurations' 4-bus networks: shape 1 is
+// config 3 (net3, 13 harmonics), shape 2 config 2 (net2 with two nonlinear buses, 10 harmonics).
+// with_shape(s, f) calls f(Dims<...>{}) of shape s = 1..HPF_SHAPES; with_dims also takes s = 0 and
+// then calls f(DynDims{}), the runtime-dimension instance.
+#define HPF_SHAPES 2
+template <class F>
+static auto with_shape(int shape, F&& f) {
+    return shape == 1 ? f(Dims<4, 3, 2, 13, 1>{}) : f(Dims<4, 2, 1, 10, 2>{});
+}
+template <class F>
+static auto with_dims(int shape, F&& f) {
+    return shape ? with_shape(shape, f) : f(DynDims{});
+}
+
+// LU of the per-scenario kernels (solve_kernel, lu_solve_kernel, harm_cta_kernel): kind 0 = matrix
+// in shared memory; 1 = matrix in a per-CTA global workspace, scenario state + blocked-LU staging
+// (lubd doubles) in shared memory; 2 = the same with oversized panels.  with_lu_kind calls
+// f(std::integral_constant<int, kind>{}).
+struct LuPlan {
+    int kind;
+    size_t lubd, smem;
+};
+static LuPlan lu_plan(const hpf_t* h, const DevNet& net) {
+    if (fits_smem_lu(h, net)) return {0, 0, scn_smem_bytes(net.n, net.H, net.q, net.N, true)};
+    const size_t lubd = gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin);
+    const size_t smem = (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd) * sizeof(double) + 16;
+    return {lub_needs_big(net.N, lubd) ? 2 : 1, lubd, smem};
+}
+template <class F>
+static auto with_lu_kind(int kind, F&& f) {
+    return kind == 0 ? f(std::integral_constant<int, 0>{})
+                     : kind == 1 ? f(std::integral_constant<int, 1>{}) : f(std::integral_constant<int, 2>{});
+}
+
+// Flat start (HG:183) of the harmonic rows h = 2..H of a batch whose fundamental stage ran on the
+// one-harmonic view.
+static void flat_start_harmonics(hpf_t* h, int n, int H, int B, double* V_m, double* V_a, cudaStream_t st) {
+    const size_t cnt = (size_t)(H - 1) * n * B;
+    flat_start_fill_kernel<<<(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st>>>(
+        V_m + (size_t)n * B, V_a + (size_t)n * B, cnt);
+    h->launches++;
+}
+
 static int solve_common(hpf_t* h, int mode, int B, const double* P, const double* Q, const double* I_N,
                         double thresh_f, int max_f, double thresh_h, int max_h, int flags, double* V_m,
                         double* V_a, double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h,
@@ -1252,24 +1296,18 @@ static int solve_common(hpf_t* h, int mode, int B, const double* P, const double
     cudaStream_t st = (cudaStream_t)stream;
     DevNet net = devnet(h);
     if (mode == 1) net.N = net.Nf;      // fundamental only: size the matrix for Nf
-    bool gm = !fits_smem_lu(h, net);
     const int H_full = net.H;
-    if (mode == 1 && gm) {
+    if (mode == 1 && !fits_smem_lu(h, net)) {
         // large network: the fundamental stage only needs the h = 1 block of the state, so the
         // kernel sees a one-harmonic view (its per-scenario arrays are sized by nH) and the
-        // flat start of the harmonic rows (HG:183) is written by a fill kernel
+        // flat start of the harmonic rows is written by a fill kernel
         net.H = 1; net.nH = net.n;
-        gm = !fits_smem_lu(h, net);
     }
-    // gm: matrix in a per-CTA global workspace, scenario state + blocked-LU staging in shared memory
-    const size_t lubd = gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin) : 0;
-    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd) * sizeof(double) + 16
-                           : scn_smem_bytes(net.n, net.H, net.q, net.N, true);
+    const LuPlan lu = lu_plan(h, net);
+    const auto kernel = with_lu_kind(lu.kind, [](auto k) { return solve_kernel<decltype(k)::value>; });
+    const int threads = lu.kind ? HPF_THREADS_GMEM : HPF_THREADS;
     int occ = 0;
-    const bool big = gm && lub_needs_big(net.N, lubd);
-    rc = !gm ? prep_kernel(h, solve_kernel<0>, smem, who, &occ)
-             : big ? prep_kernel(h, solve_kernel<2>, smem, who, &occ, HPF_THREADS_GMEM)
-                   : prep_kernel(h, solve_kernel<1>, smem, who, &occ, HPF_THREADS_GMEM);
+    rc = prep_kernel(h, kernel, lu.smem, who, &occ, threads);
     if (rc) return rc;
     SolveArgs a;
     a.B = B; a.mode = mode; a.flags = flags; a.P = P; a.Q = Q; a.I_N = (const double2*)I_N;
@@ -1278,28 +1316,21 @@ static int solve_common(hpf_t* h, int mode, int B, const double* P, const double
     a.V_m = V_m; a.V_a = V_a; a.I_inj = (double2*)I_inj;
     a.n_iter_f = n_iter_f; a.n_iter_h = n_iter_h; a.status = status; a.err_h = err_h; a.err_f = err_f;
     a.work_counter = h->d_counter + h->cur_slot;
-    a.lub_doubles = (int)lubd;
+    a.lub_doubles = (int)lu.lubd;
     a.lu_classic = h->lu_classic;
     CK(cudaMemsetAsync(h->d_counter + h->cur_slot, 0, sizeof(int), st));
     long long grid = (long long)occ * h->sm_count;
     if (grid > B) grid = B;
     if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
     a.workspace = nullptr;
-    if (gm) {
+    if (lu.kind) {
         rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
         if (rc) return rc;
         a.workspace = h->d_work;
     }
     if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
-    if (!gm) solve_kernel<0><<<(unsigned)grid, HPF_THREADS, smem, st>>>(net, a);
-    else if (big) solve_kernel<2><<<(unsigned)grid, HPF_THREADS_GMEM, smem, st>>>(net, a);
-    else solve_kernel<1><<<(unsigned)grid, HPF_THREADS_GMEM, smem, st>>>(net, a);
-    if (net.H != H_full) {
-        const size_t cnt = (size_t)(H_full - 1) * net.n * B;
-        flat_start_fill_kernel<<<(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st>>>(
-            V_m + (size_t)net.n * B, V_a + (size_t)net.n * B, cnt);
-        h->launches++;
-    }
+    kernel<<<(unsigned)grid, threads, lu.smem, st>>>(net, a);
+    if (net.H != H_full) flat_start_harmonics(h, net.n, H_full, B, V_m, V_a, st);
     if (h->profiling) { CK(cudaEventRecord(h->ev[2], st)); h->ev_valid = 2; }
     h->launches++;
     CK(cudaGetLastError());
@@ -1472,8 +1503,7 @@ static int setup_woodbury(hpf_t* h, const DevNet& net, cudaStream_t st, int* inf
 // Constants of the one-warp-per-harmonic kernel (hpf_harmonic_warp.cuh) for a shape-specialised
 // network, from the host mirrors of Y(h), Y_N and G: kept in the handle, passed BY VALUE at launch.
 template <class D>
-static bool build_hw_consts(hpf_t* h, int shape_id) {
-    if (!(h->n == D::n && h->m == D::m && h->c == D::c && h->H == D::H && h->q == D::q)) return false;
+static void build_hw_consts(hpf_t* h) {
     constexpr int n = D::n, m = D::m, H = D::H, q = D::q;
     auto fill = [&](auto* C) {
         for (int t = 0; t < H * n * n; ++t) C->Y[t] = h->hY[(size_t)t];
@@ -1500,8 +1530,6 @@ static bool build_hw_consts(hpf_t* h, int shape_id) {
         h->hw_consts.assign(sizeof(HwConsts<D, false>), 0);
         fill(reinterpret_cast<HwConsts<D, false>*>(h->hw_consts.data()));
     }
-    h->hw_shape = shape_id;
-    return true;
 }
 
 // Structured set-up, once per network.  Variants of the harmonic stage:
@@ -1617,7 +1645,7 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
         double wpr[2] = {0.0, 0.0};
         int rcw = setup_woodbury(h, net, st, &winfo, wpr);
         if (rcw) return rcw;
-        h->hWNL.clear(); h->hG.clear(); h->hw_shape = 0;
+        h->hWNL.clear(); h->hG.clear(); h->hw_consts.clear();
         h->pivot_min = wpr[0]; h->pivot_max = wpr[1];
         if (winfo == 0 && wpr[0] > 0.0 && wpr[1] / wpr[0] < 1e12) h->struct_state = variant;
         return HPF_OK;
@@ -1649,7 +1677,7 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     h->hWNL.clear();
     h->hG.clear();
-    h->hw_shape = 0;
+    h->hw_consts.clear();
     if (variant == 1 && e == cudaSuccess && qH > 0 && (size_t)nZ * qH <= 1024) {   // small operators: host mirror
         h->hWNL.resize((size_t)nZ * qH);
         e = cudaMemcpy(h->hWNL.data(), h->d_WNL, h->hWNL.size() * sizeof(double2), cudaMemcpyDeviceToHost);
@@ -1662,9 +1690,8 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
     h->pivot_min = prh[0]; h->pivot_max = prh[1];
     // usable when the inversion met no zero pivot and the pivots span < 1e12 (well conditioned)
     if (info == 0 && prh[0] > 0.0 && prh[1] / prh[0] < 1e12) h->struct_state = variant;
-    if (h->struct_state == 1 && !h->hG.empty() && !h->no_specialise) {
-        if (!build_hw_consts<Dims<4, 3, 2, 13, 1>>(h, 1)) build_hw_consts<Dims<4, 2, 1, 10, 2>>(h, 2);
-    }
+    if (h->struct_state == 1 && !h->hG.empty() && h->shape)
+        with_shape(h->shape, [&](auto d) { build_hw_consts<decltype(d)>(h); return 0; });
     return HPF_OK;
 #undef SK
 }
@@ -1707,21 +1734,18 @@ static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, co
     if (qH == 0) { CK(cudaMemsetAsync(h->d_wN + off, 0, (need - off) * sizeof(double2), st)); return HPF_OK; }
     WnArgs wa;
     wa.B = B; wa.I_N = (const double2*)I_N; wa.wN = h->d_wN + off;
-    if (!h->no_specialise && h->struct_state == 1 && !h->hWNL.empty()) {
-        auto lane = [&](auto dims) -> bool {
-            using D = decltype(dims);
-            if (!(net.n == D::n && net.m == D::m && net.c == D::c && net.H == D::H && net.q == D::q)) return false;
+    if (h->shape && h->struct_state == 1 && !h->hWNL.empty()) {
+        with_shape(h->shape, [&](auto d) {
+            using D = decltype(d);
             static_assert(sizeof(WnConsts<D>) + sizeof(WnArgs) <= 32000, "kernel parameter space");
             WnConsts<D> C;
             memcpy(C.W, h->hWNL.data(), sizeof(C.W));
             wn_lane_kernel<D><<<(unsigned)((B + 127) / 128), 128, 0, st>>>(C, wa);
-            return true;
-        };
-        if (lane(Dims<4, 3, 2, 13, 1>()) || lane(Dims<4, 2, 1, 10, 2>())) {
-            h->launches++;
-            CK(cudaGetLastError());
-            return HPF_OK;
-        }
+            return 0;
+        });
+        h->launches++;
+        CK(cudaGetLastError());
+        return HPF_OK;
     }
     if (wn_use_dmma(h, sn.nZ, qH, B)) {
         int rcz = launch_zgemm(h, sn.nZ, B, qH, sn.WNL, (size_t)qH, (const double2*)I_N, (size_t)B, wa.wN, (size_t)B, st);
@@ -1780,18 +1804,10 @@ static int launch_harm_hw(hpf_t* h, const HarmTileArgs& ha, cudaStream_t st) {
         CK(cudaGetLastError());
         return HPF_OK;
     };
-    // two register budgets are compiled: 2 CTAs per SM (default) and 1 CTA per SM ($HPF_HW_MINB=1)
-    if (h->coupled) {
-        const auto* C = reinterpret_cast<const HwConsts<D, true>*>(h->hw_consts.data());
-        return h->hw_minb == 1 ? go(harm_hw_kernel<D, true, 1>, C) : go(harm_hw_kernel<D, true, 2>, C);
-    }
-    const auto* C = reinterpret_cast<const HwConsts<D, false>*>(h->hw_consts.data());
-    return h->hw_minb == 1 ? go(harm_hw_kernel<D, false, 1>, C) : go(harm_hw_kernel<D, false, 2>, C);
+    if (h->coupled) return go(harm_hw_kernel<D, true>, reinterpret_cast<const HwConsts<D, true>*>(h->hw_consts.data()));
+    return go(harm_hw_kernel<D, false>, reinterpret_cast<const HwConsts<D, false>*>(h->hw_consts.data()));
 }
 
-// Shape-specialised instances exist for the BASELINE configurations' 4-bus networks
-// (config 3: net3, 13 harmonics; config 2: net2 with two nonlinear buses, 10 harmonics);
-// every other network runs the runtime-dimension instance.
 static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const HarmTileArgs& ha,
                        bool persistent, cudaStream_t st) {
     if (h->struct_state >= 2) {
@@ -1804,12 +1820,14 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
         const int gthreads = sn.nx <= 256 ? 256 : HPF_THREADS_GMEM;
         const size_t smem = gst ? (lubd + 80) * sizeof(double)
                                 : harm_cta_smem_bytes(net.n, net.H, net.m, net.c, net.q, net.N);
-        int occ = 0;
         // global-state variant: every phase waits on L2 / HBM, so it runs with twice the warps
-        const bool big = gst && lub_needs_big(sn.nx, lubd);
-        int rc = !gst ? prep_kernel(h, harm_cta_kernel<HPF_THREADS, false>, smem, "hpf_solve", &occ)
-                      : big ? prep_kernel(h, harm_cta_kernel<HPF_THREADS_GMEM, true>, smem, "hpf_solve", &occ, gthreads)
-                            : prep_kernel(h, harm_cta_kernel<HPF_THREADS_GMEM, false>, smem, "hpf_solve", &occ, gthreads);
+        const int kind = !gst ? 0 : lub_needs_big(sn.nx, lubd) ? 2 : 1;
+        const auto kernel = with_lu_kind(kind, [](auto k) {
+            return harm_cta_kernel<decltype(k)::value ? HPF_THREADS_GMEM : HPF_THREADS, decltype(k)::value == 2>;
+        });
+        const int threads = gst ? gthreads : HPF_THREADS;
+        int occ = 0;
+        int rc = prep_kernel(h, kernel, smem, "hpf_solve", &occ, threads);
         if (rc) return rc;
         long long grid = ha.B;
         if ((persistent || gst) && grid > (long long)occ * h->sm_count) grid = (long long)occ * h->sm_count;
@@ -1826,25 +1844,17 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
             }
             ha2.gstate = h->d_gstate; ha2.gstate_stride = stride;
         }
-        if (!gst) harm_cta_kernel<HPF_THREADS, false><<<(unsigned)grid, HPF_THREADS, smem, st>>>(net, sn, ha2);
-        else if (big) harm_cta_kernel<HPF_THREADS_GMEM, true><<<(unsigned)grid, gthreads, smem, st>>>(net, sn, ha2);
-        else harm_cta_kernel<HPF_THREADS_GMEM, false><<<(unsigned)grid, gthreads, smem, st>>>(net, sn, ha2);
+        kernel<<<(unsigned)grid, threads, smem, st>>>(net, sn, ha2);
         h->launches++;
         CK(cudaGetLastError());
         return HPF_OK;
     }
-    if (h->hw_shape && !h->harm_tile_only && !ha.step_only && persistent) {
-        if (h->hw_shape == 1) return launch_harm_hw<Dims<4, 3, 2, 13, 1>>(h, ha, st);
-        return launch_harm_hw<Dims<4, 2, 1, 10, 2>>(h, ha, st);
-    }
+    if (h->shape && !h->hw_consts.empty() && !h->harm_tile_only && !ha.step_only && persistent)
+        return with_shape(h->shape, [&](auto d) { return launch_harm_hw<decltype(d)>(h, ha, st); });
+    if (h->shape)
+        return with_shape(h->shape, [&](auto d) { return launch_harm_t<8, 2, decltype(d)>(h, net, sn, ha, persistent, st); });
     const bool two = 2 * harm_tile_smem_bytes(net.n, net.H, net.m, net.c, net.q, 8, sn.yn_elems) + 2048 <=
                      (size_t)h->smem_optin + 1024;
-    if (!h->no_specialise) {
-        if (net.n == 4 && net.m == 3 && net.c == 2 && net.H == 13 && net.q == 1)
-            return launch_harm_t<8, 2, Dims<4, 3, 2, 13, 1>>(h, net, sn, ha, persistent, st);
-        if (net.n == 4 && net.m == 2 && net.c == 1 && net.H == 10 && net.q == 2)
-            return launch_harm_t<8, 2, Dims<4, 2, 1, 10, 2>>(h, net, sn, ha, persistent, st);
-    }
     if (two) return launch_harm_t<8, 2, DynDims>(h, net, sn, ha, persistent, st);
     return launch_harm_t<8, 1, DynDims>(h, net, sn, ha, persistent, st);
 }
@@ -1887,10 +1897,25 @@ struct LsTimer {
 static LsTimer g_ls_timer;
 
 // ---- lock-step batched harmonic stage (hpf_lockstep.cuh) ---------------------------------
-static bool use_lockstep(const hpf_t* h, const StructNet& sn, int B) {
-    if (h->struct_state != 3 || h->lockstep == 0) return false;
-    if (sn.nx < 1 || sn.nx > 2048) return false;             // panel kernel: at most 4 rows per thread of 512
+// Whether a batch of B systems of the given order goes through the lock-step LU ($HPF_LOCKSTEP)
+static bool use_lockstep(const hpf_t* h, int order, int B) {
+    if (h->lockstep == 0 || order < 1 || order > HPF_LS_MAX_ORDER) return false;
     return h->lockstep == 1 || B >= HPF_LS_AUTO_MIN_B;
+}
+
+// Doubles per lock-step slot for its matrix [lub_ld(N) x (N+1)], padded to a multiple of 16
+static size_t ls_mat_stride(int N) { return ((size_t)lub_ld(N) * (N + 1) + 15) / 16 * 16; }
+
+// Integer block of the lock-step work area, behind the slots' floating-point arrays
+static void ls_carve_ints(LsArgs& la, char* p, int S) {
+    int* ip = reinterpret_cast<int*>(p);
+    la.act = ip;  ip += 2 * (size_t)S;
+    la.flag = ip; ip += S;
+    la.itc = ip;  ip += S;
+    la.stat = ip; ip += S;
+    la.info = ip; ip += S;
+    la.nact = ip; ip += 2;
+    la.perm = ip;
 }
 
 template <class K>
@@ -2030,25 +2055,17 @@ static int ensure_ls(hpf_t* h, size_t per_slot, int B, int* slots) {
 // hpf_lu_solve for systems beyond shared memory through the batched LU (all matrices panel by panel)
 static int lu_solve_batched(hpf_t* h, int N, int B, const double* J, size_t stride, const double* f, double* dx,
                             int* info, cudaStream_t st) {
-    const int ldb = lub_ld(N);
-    const size_t mat_stride = ((size_t)ldb * (N + 1) + 15) / 16 * 16;
+    const size_t mat_stride = ls_mat_stride(N);
     const size_t per_slot = mat_stride * sizeof(double) + (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     int S = 0;
     int rc = ensure_ls(h, per_slot, B, &S);
     if (rc) return rc;
     LsArgs la;
     memset(&la, 0, sizeof(la));
-    la.B = B; la.S = S; la.ldb = ldb; la.mat_stride = mat_stride;
+    la.B = B; la.S = S; la.ldb = lub_ld(N); la.mat_stride = mat_stride;
     char* p = reinterpret_cast<char*>(h->d_ls);
     la.M = reinterpret_cast<double*>(p); p += mat_stride * sizeof(double) * (size_t)S;
-    int* ip = reinterpret_cast<int*>(p);
-    la.act = ip;  ip += 2 * (size_t)S;
-    la.flag = ip; ip += S;
-    la.itc = ip;  ip += S;
-    la.stat = ip; ip += S;
-    la.info = ip; ip += S;
-    la.nact = ip; ip += 2;
-    la.perm = ip;
+    ls_carve_ints(la, p, S);
     const long long nt = (N + 31) / 32;
     for (int b0 = 0; b0 < B; b0 += S) {
         la.b0 = b0;
@@ -2066,32 +2083,13 @@ static int lu_solve_batched(hpf_t* h, int N, int B, const double* J, size_t stri
     return HPF_OK;
 }
 
-static void ls_carve_ints(LsArgs& la, char* p, int S) {
-    int* ip = reinterpret_cast<int*>(p);
-    la.act = ip;  ip += 2 * (size_t)S;
-    la.flag = ip; ip += S;
-    la.itc = ip;  ip += S;
-    la.stat = ip; ip += S;
-    la.info = ip; ip += S;
-    la.nact = ip; ip += 2;
-    la.perm = ip;
-}
-
 // fundamental stage of the large networks in lock step (dense Jacobians of order Nf through the batched LU)
-static bool use_lockstep_fund(const hpf_t* h, int B) {
-    if (h->struct_state != 3 || h->lockstep == 0) return false;
-    const int Nf = 2 * h->n - 1 - h->c;
-    if (Nf < 1 || Nf > 2048) return false;
-    return h->lockstep == 1 || B >= HPF_LS_AUTO_MIN_B;
-}
-
 static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* Q, double thresh_f, int max_f,
                                 double* V_m, double* V_a, int* n_iter_f, int* status, double* hist_f, cudaStream_t st) {
     DevNet nf = devnet(h);
     const int H_full = nf.H, Nf = nf.Nf;
     nf.N = Nf; nf.H = 1; nf.nH = nf.n;
-    const int ldb = lub_ld(Nf);
-    const size_t mat_stride = ((size_t)ldb * (Nf + 1) + 15) / 16 * 16;
+    const size_t mat_stride = ls_mat_stride(Nf);
     const size_t state_stride = (scn_smem_doubles_aligned(nf.n, 1, nf.q, Nf) + 15) / 16 * 16;
     const size_t per_slot = (mat_stride + state_stride) * sizeof(double) + (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     int S = 0;
@@ -2101,7 +2099,7 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
     memset(&la, 0, sizeof(la));
     la.B = B; la.S = S; la.P = P; la.Q = Q; la.thresh_h = thresh_f; la.max_h = max_f; la.V_m = V_m; la.V_a = V_a;
     la.n_iter_h = n_iter_f; la.status = status; la.hist_h = hist_f;
-    la.ldb = ldb; la.mat_stride = mat_stride; la.state_stride = state_stride;
+    la.ldb = lub_ld(Nf); la.mat_stride = mat_stride; la.state_stride = state_stride;
     {
         char* p = reinterpret_cast<char*>(h->d_ls);
         la.M = reinterpret_cast<double*>(p);      p += mat_stride * sizeof(double) * (size_t)S;
@@ -2135,12 +2133,7 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
             if (rc) return rc;
         }
     }
-    if (H_full > 1) {
-        const size_t cnt = (size_t)(H_full - 1) * nf.n * B;
-        flat_start_fill_kernel<<<(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st>>>(
-            V_m + (size_t)nf.n * B, V_a + (size_t)nf.n * B, cnt);
-        h->launches++;
-    }
+    if (H_full > 1) flat_start_harmonics(h, nf.n, H_full, B, V_m, V_a, st);
     g_ls_timer.report("fundamental stage");
     g_ls_timer.on = false;
     CK(cudaGetLastError());
@@ -2149,8 +2142,7 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
 
 static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, const HarmTileArgs& ha, cudaStream_t st) {
     const int nx = sn.nx, nZ = sn.nZ, m = net.m, q = net.q;
-    const int ldb = lub_ld(nx);
-    const size_t mat_stride = ((size_t)ldb * (nx + 1) + 15) / 16 * 16;
+    const size_t mat_stride = ls_mat_stride(nx);
     const size_t state_stride = (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + 15) / 16 * 16;
     const size_t per_slot = (mat_stride + state_stride) * sizeof(double) + ((size_t)m + nZ + q) * sizeof(double2) +
                             (size_t)(LS_PERM_INTS + 8) * sizeof(int);
@@ -2171,16 +2163,9 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
         la.X = reinterpret_cast<double2*>(p);     p += (size_t)m * S * sizeof(double2);
         la.GX = reinterpret_cast<double2*>(p);    p += (size_t)nZ * S * sizeof(double2);
         la.U0 = reinterpret_cast<double2*>(p);    p += (size_t)q * S * sizeof(double2);
-        int* ip = reinterpret_cast<int*>(p);
-        la.act = ip;  ip += 2 * (size_t)S;
-        la.flag = ip; ip += S;
-        la.itc = ip;  ip += S;
-        la.stat = ip; ip += S;
-        la.info = ip; ip += S;
-        la.nact = ip; ip += 2;
-        la.perm = ip;
+        ls_carve_ints(la, p, S);
     }
-    la.mat_stride = mat_stride; la.state_stride = state_stride; la.ldb = ldb;
+    la.mat_stride = mat_stride; la.state_stride = state_stride; la.ldb = lub_ld(nx);
     int g_mis = 0, g_bor = 0, rc;
     rc = ls_grid(h, ls_mismatch_kernel, 256, 0, S, &g_mis);
     if (rc) return rc;
@@ -2241,7 +2226,7 @@ static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, c
     if (h->profiling) { CK(cudaEventRecord(h->ev[0], st)); }
     // fundamental stage: one lane per scenario (variant 1) or the per-CTA kernel (variant 2)
     if (h->struct_state >= 2) {
-        int rc = use_lockstep_fund(h, B)
+        int rc = h->struct_state == 3 && use_lockstep(h, net.Nf, B)
                      ? launch_lockstep_fund(h, B, P, Q, thresh_f, max_f, V_m, V_a, n_iter_f, status, hist_f, st)
                      : solve_common(h, 1, B, P, Q, nullptr, thresh_f, max_f, 0.0, 0, 0, V_m, V_a, nullptr, n_iter_f,
                                     nullptr, nullptr, nullptr, status, hist_f, nullptr, st);
@@ -2266,10 +2251,7 @@ static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, c
             kernel<<<(unsigned)grid, warps * 32, smem, st>>>(net, fa);
             return HPF_OK;
         };
-        int rcf;
-        if (!h->no_specialise && net.n == 4 && net.c == 2) rcf = launch(fund_tile_kernel<Dims<4, 3, 2, 13, 1>>);
-        else if (!h->no_specialise && net.n == 4 && net.c == 1) rcf = launch(fund_tile_kernel<Dims<4, 2, 1, 10, 2>>);
-        else rcf = launch(fund_tile_kernel<DynDims>);
+        const int rcf = with_dims(h->fund_shape, [&](auto d) { return launch(fund_tile_kernel<decltype(d)>); });
         if (rcf) return rcf;
         h->launches++;
         CK(cudaGetLastError());
@@ -2285,7 +2267,7 @@ static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, c
         ha.thresh_h = thresh_h; ha.max_h = max_h; ha.V_m = V_m; ha.V_a = V_a; ha.I_inj = (double2*)I_inj;
         ha.n_iter_h = n_iter_h; ha.status = status; ha.err_h = err_h; ha.work_counter = h->d_counter + h->cur_slot;
         ha.dx_out = nullptr; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0; ha.hist_h = hist_h; ha.epoch = HPF_HW_SERVICE_EPOCH;
-        const bool ls = use_lockstep(h, sn, B);
+        const bool ls = h->struct_state == 3 && use_lockstep(h, sn.nx, B);
         rc = ls ? launch_lockstep(h, net, sn, ha, st) : launch_harm(h, net, sn, ha, true, st);
         if (rc) return rc;
         h->last_path = ls ? 4 : (h->struct_state >= 2 ? h->struct_state : 1);
@@ -2370,7 +2352,6 @@ int hpf_create(hpf_t** out, int device) {
     if (const char* ev = getenv("HPF_SETUP")) h->setup_gj = (strcmp(ev, "gj") == 0) ? 1 : 0;
     if (const char* ev = getenv("HPF_WN_KERNEL")) h->wn_kernel = (strcmp(ev, "dmma") == 0) ? 2 : (strcmp(ev, "fma") == 0) ? 1 : 0;
     if (const char* ev = getenv("HPF_HARM_KERNEL")) h->harm_tile_only = (strcmp(ev, "tile") == 0) ? 1 : 0;
-    if (const char* ev = getenv("HPF_HW_MINB")) h->hw_minb = (atoi(ev) == 1) ? 1 : 2;
     if (const char* ev = getenv("HPF_MAX_CTAS")) h->max_ctas = atoi(ev) > 0 ? atoi(ev) : 0;
     h->sm_count = prop.multiProcessorCount;
     h->smem_optin = (int)prop.sharedMemPerBlockOptin;
@@ -2416,6 +2397,14 @@ int hpf_set_network(hpf_t* h, int n, int m, int c, int H, const int* harmonics, 
             return fail(h, HPF_E_INVALID, "hpf_set_network: line endpoint outside 1..n");
     ENTER_DEVICE(h);
     h->n = n; h->m = m; h->c = c; h->H = H; h->q = n - m; h->L = L;
+    h->shape = h->fund_shape = 0;
+    for (int s = 1; s <= HPF_SHAPES && !h->no_specialise; ++s)
+        with_shape(s, [&](auto d) {
+            using D = decltype(d);
+            if (n == D::n && m == D::m && c == D::c && H == D::H && n - m == D::q) h->shape = s;
+            if (n == D::n && c == D::c && !h->fund_shape) h->fund_shape = s;
+            return 0;
+        });
     CK(upload(&h->d_harm, harmonics, (size_t)H));
     CK(upload(&h->d_from, from_id, (size_t)L));
     CK(upload(&h->d_to, to_id, (size_t)L));
@@ -2980,12 +2969,8 @@ static int mismatch_impl(hpf_t* h, int B, const double* V_m, const double* V_a, 
     const int yn_elems = h->n_dev * (h->coupled ? h->H * h->H : h->H);
     size_t smem = tile_smem_bytes(net.n, net.H, net.q, net.m, yn_elems);
     int occ = 0;
-    const bool lane_ok = !h->no_specialise && !h->mismatch_tile;
-    if (lane_ok && net.n == 4 && net.m == 3 && net.c == 2 && net.H == 13 && net.q == 1) {
-        rc = launch_mismatch_lane<Dims<4, 3, 2, 13, 1>>(h, a, (cudaStream_t)stream);
-        if (rc) return rc;
-    } else if (lane_ok && net.n == 4 && net.m == 2 && net.c == 1 && net.H == 10 && net.q == 2) {
-        rc = launch_mismatch_lane<Dims<4, 2, 1, 10, 2>>(h, a, (cudaStream_t)stream);
+    if (h->shape && !h->mismatch_tile) {
+        rc = with_shape(h->shape, [&](auto d) { return launch_mismatch_lane<decltype(d)>(h, a, (cudaStream_t)stream); });
         if (rc) return rc;
     } else if (smem <= (size_t)h->smem_optin) {
         const long long tiles = ((long long)B + HPF_TILE - 1) / HPF_TILE;
@@ -2999,12 +2984,7 @@ static int mismatch_impl(hpf_t* h, int B, const double* V_m, const double* V_a, 
             kernel<<<(unsigned)grid, HPF_THREADS, smem, (cudaStream_t)stream>>>(net, a, yn_elems);
             return HPF_OK;
         };
-        if (!h->no_specialise && net.n == 4 && net.m == 3 && net.c == 2 && net.H == 13 && net.q == 1)
-            rc = launch(mismatch_tile_kernel<Dims<4, 3, 2, 13, 1>>);
-        else if (!h->no_specialise && net.n == 4 && net.m == 2 && net.c == 1 && net.H == 10 && net.q == 2)
-            rc = launch(mismatch_tile_kernel<Dims<4, 2, 1, 10, 2>>);
-        else
-            rc = launch(mismatch_tile_kernel<DynDims>);
+        rc = with_dims(h->shape, [&](auto d) { return launch(mismatch_tile_kernel<decltype(d)>); });
         if (rc) return rc;
     } else {
         smem = scn_smem_bytes(net.n, net.H, net.q, net.N, false);
@@ -3069,32 +3049,25 @@ static int lu_solve_impl(hpf_t* h, int B, const double* J, const double* f, doub
     const DevNet net = devnet(h);
     LuArgs a;
     a.B = B; a.J = J; a.f = f; a.dx = dx; a.info = info; a.stride = hpf_jacobian_stride(h);
-    const bool gm = !fits_smem_lu(h, net);
-    const size_t lubd = gm ? gmem_kernel_lub_doubles(net.n, net.H, net.q, net.N, (size_t)h->smem_optin) : 0;
-    const size_t smem = gm ? (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + lubd) * sizeof(double) + 16
-                           : scn_smem_bytes(net.n, net.H, net.q, net.N, true);
-    a.lub_doubles = (int)lubd;
+    const LuPlan lu = lu_plan(h, net);
+    a.lub_doubles = (int)lu.lubd;
     a.lu_classic = h->lu_classic;
+    const auto kernel = with_lu_kind(lu.kind, [](auto k) { return lu_solve_kernel<decltype(k)::value>; });
+    const int threads = lu.kind ? HPF_THREADS_GMEM : HPF_THREADS;
     int occ = 0;
-    const bool big = gm && lub_needs_big(net.N, lubd);
-    rc = !gm ? prep_kernel(h, lu_solve_kernel<0>, smem, "hpf_lu_solve", &occ)
-             : big ? prep_kernel(h, lu_solve_kernel<2>, smem, "hpf_lu_solve", &occ, HPF_THREADS_GMEM)
-                   : prep_kernel(h, lu_solve_kernel<1>, smem, "hpf_lu_solve", &occ, HPF_THREADS_GMEM);
+    rc = prep_kernel(h, kernel, lu.smem, "hpf_lu_solve", &occ, threads);
     if (rc) return rc;
-    if (gm && net.N <= 2048 && (h->lockstep == 1 || (h->lockstep != 0 && B >= HPF_LS_AUTO_MIN_B)))
+    if (lu.kind && use_lockstep(h, net.N, B))
         return lu_solve_batched(h, net.N, B, J, a.stride, f, dx, info, (cudaStream_t)stream);
     long long grid = (long long)occ * h->sm_count;
     if (grid > B) grid = B;
     a.workspace = nullptr;
-    if (gm) {
+    if (lu.kind) {
         rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
         if (rc) return rc;
         a.workspace = h->d_work;
-        if (big) lu_solve_kernel<2><<<(unsigned)grid, HPF_THREADS_GMEM, smem, (cudaStream_t)stream>>>(net, a);
-        else lu_solve_kernel<1><<<(unsigned)grid, HPF_THREADS_GMEM, smem, (cudaStream_t)stream>>>(net, a);
-    } else {
-        lu_solve_kernel<0><<<(unsigned)grid, HPF_THREADS, smem, (cudaStream_t)stream>>>(net, a);
     }
+    kernel<<<(unsigned)grid, threads, lu.smem, (cudaStream_t)stream>>>(net, a);
     h->launches++;
     CK(cudaGetLastError());
     return HPF_OK;
