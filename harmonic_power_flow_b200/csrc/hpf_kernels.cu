@@ -1063,10 +1063,6 @@ struct hpf_handle {
     double* d_io = nullptr;       // staging buffers of hpf_solve_host (grow-only)
     size_t io_doubles = 0;
     cudaStream_t st_io[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // copy-in, compute, copy-out, compute 2..4
-    // hpf_solve_host runs consecutive chunks on two compute streams (the tail of chunk k overlaps
-    // the start of chunk k+1); each in-flight chunk has its own work counter and w_N scratch
-    int cur_slot = 0;             // work-counter slot of the chunk being issued (0 outside hpf_solve_host)
-    size_t wN_off = 0;            // offset of that chunk's w_N scratch inside d_wN
     cudaEvent_t ev_io[2 * HPF_HOST_MAX_CHUNKS] = {};
     // structured strategy: 0 = not set up yet, 1 = ready, -1 = not available for this network
     int struct_state = 0;
@@ -1280,20 +1276,74 @@ static void flat_start_harmonics(hpf_t* h, int n, int H, int B, double* V_m, dou
     h->launches++;
 }
 
-static int solve_common(hpf_t* h, int mode, int B, const double* P, const double* Q, const double* I_N,
-                        double thresh_f, int max_f, double thresh_h, int max_h, int flags, double* V_m,
-                        double* V_a, double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h,
-                        double* err_f, int* status, double* hist_f, double* hist_h, void* stream) {
-    const char* who = mode ? "hpf_fund_solve" : "hpf_solve";
+// ---- solve requests -------------------------------------------------------------------
+// Outputs of a batch solve ([rows, B] layout): the device buffers of hpf_solve, the host arrays of
+// hpf_solve_host, or the device copies that hpf_solve_host_keep leaves behind.
+struct BatchOut {
+    double *V_m = nullptr, *V_a = nullptr;
+    double2* I_inj = nullptr;
+    int *n_iter_f = nullptr, *n_iter_h = nullptr, *status = nullptr;
+    double* err_h = nullptr;
+};
+
+// One solve request as it travels through the host solve path: built once by the entry point,
+// then read by every stage and kernel argument block.
+struct SolveReq {
+    int B = 0, flags = 0;
+    const double *P = nullptr, *Q = nullptr;
+    const double2* I_N = nullptr;
+    double thresh_f = 0.0, thresh_h = 0.0;
+    int max_f = 0, max_h = 0;
+    BatchOut out;
+    double *err_f = nullptr, *hist_f = nullptr, *hist_h = nullptr;
+    // hpf_solve_host runs consecutive chunks on several compute streams (the tail of chunk k overlaps
+    // the start of chunk k+1), so each chunk in flight has its own work counter and w_N scratch
+    int slot = 0;                 // work-counter slot: the chunk index of a dual-stream hpf_solve_host, else 0
+    size_t wN_off = 0;            // offset of this solve's w_N scratch inside h->d_wN
+};
+
+// Argument checks of a solve request at entry point `who`, in this order: handle ready, B < 0, NULL
+// buffers.  I_N is needed only with nonlinear buses; the fundamental-only solve (mode 1) needs no
+// device tables and has no harmonic outputs.  A request with B == 0 passes: it has nothing to do.
+static int check_request(hpf_t* h, const SolveReq& r, int mode, const char* who) {
     int rc = ready(h, who, mode == 0);
     if (rc) return rc;
-    if (B < 0) return fail(h, HPF_E_INVALID, std::string(who) + ": B < 0");
-    if (B == 0) return HPF_OK;
-    if (!P || !Q || !V_m || !V_a || !n_iter_f ||
-        (mode == 0 && (!n_iter_h || !err_h || !status || (h->q > 0 && !I_N))))
+    if (r.B < 0) return fail(h, HPF_E_INVALID, std::string(who) + ": B < 0");
+    if (r.B == 0) return HPF_OK;
+    const BatchOut& o = r.out;
+    if (!r.P || !r.Q || !o.V_m || !o.V_a || !o.n_iter_f ||
+        (mode == 0 && (!o.n_iter_h || !o.err_h || !o.status || (h->q > 0 && !r.I_N))))
         return fail(h, HPF_E_INVALID, std::string(who) + ": NULL buffer");
-    ENTER_DEVICE(h);
-    cudaStream_t st = (cudaStream_t)stream;
+    return HPF_OK;
+}
+
+// The fundamental stage of a request on its own: the harmonic stage's inputs, limits and outputs
+// cleared, as hpf_fund_solve passes them.
+static SolveReq fund_stage(SolveReq r) {
+    r.flags = 0; r.I_N = nullptr; r.thresh_h = 0.0; r.max_h = 0; r.hist_h = nullptr;
+    r.out.I_inj = nullptr; r.out.n_iter_h = nullptr; r.out.err_h = nullptr;
+    return r;
+}
+
+static SolveArgs solve_args(const hpf_t* h, const SolveReq& r, int mode, const LuPlan& lu, double* workspace) {
+    SolveArgs a;
+    a.B = r.B; a.mode = mode; a.flags = r.flags; a.P = r.P; a.Q = r.Q; a.I_N = r.I_N;
+    a.hist_f = r.hist_f; a.hist_h = r.hist_h;
+    a.thresh_f = r.thresh_f; a.thresh_h = r.thresh_h; a.max_f = r.max_f; a.max_h = r.max_h;
+    a.V_m = r.out.V_m; a.V_a = r.out.V_a; a.I_inj = r.out.I_inj;
+    a.n_iter_f = r.out.n_iter_f; a.n_iter_h = r.out.n_iter_h; a.status = r.out.status; a.err_h = r.out.err_h;
+    a.err_f = r.err_f;
+    a.work_counter = h->d_counter + r.slot;
+    a.workspace = workspace;
+    a.lub_doubles = (int)lu.lubd;
+    a.lu_classic = h->lu_classic;
+    return a;
+}
+
+// Per-scenario solve kernel over a checked request with B > 0: mode 0 the whole solve (dense path),
+// mode 1 the fundamental stage only.
+static int solve_common(hpf_t* h, int mode, const SolveReq& r, cudaStream_t st) {
+    const char* who = mode ? "hpf_fund_solve" : "hpf_solve";
     DevNet net = devnet(h);
     if (mode == 1) net.N = net.Nf;      // fundamental only: size the matrix for Nf
     const int H_full = net.H;
@@ -1307,30 +1357,21 @@ static int solve_common(hpf_t* h, int mode, int B, const double* P, const double
     const auto kernel = with_lu_kind(lu.kind, [](auto k) { return solve_kernel<decltype(k)::value>; });
     const int threads = lu.kind ? HPF_THREADS_GMEM : HPF_THREADS;
     int occ = 0;
-    rc = prep_kernel(h, kernel, lu.smem, who, &occ, threads);
+    int rc = prep_kernel(h, kernel, lu.smem, who, &occ, threads);
     if (rc) return rc;
-    SolveArgs a;
-    a.B = B; a.mode = mode; a.flags = flags; a.P = P; a.Q = Q; a.I_N = (const double2*)I_N;
-    a.hist_f = hist_f; a.hist_h = hist_h;
-    a.thresh_f = thresh_f; a.thresh_h = thresh_h; a.max_f = max_f; a.max_h = max_h;
-    a.V_m = V_m; a.V_a = V_a; a.I_inj = (double2*)I_inj;
-    a.n_iter_f = n_iter_f; a.n_iter_h = n_iter_h; a.status = status; a.err_h = err_h; a.err_f = err_f;
-    a.work_counter = h->d_counter + h->cur_slot;
-    a.lub_doubles = (int)lu.lubd;
-    a.lu_classic = h->lu_classic;
-    CK(cudaMemsetAsync(h->d_counter + h->cur_slot, 0, sizeof(int), st));
+    CK(cudaMemsetAsync(h->d_counter + r.slot, 0, sizeof(int), st));
     long long grid = (long long)occ * h->sm_count;
-    if (grid > B) grid = B;
+    if (grid > r.B) grid = r.B;
     if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
-    a.workspace = nullptr;
+    double* workspace = nullptr;
     if (lu.kind) {
         rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
         if (rc) return rc;
-        a.workspace = h->d_work;
+        workspace = h->d_work;
     }
     if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
-    kernel<<<(unsigned)grid, threads, lu.smem, st>>>(net, a);
-    if (net.H != H_full) flat_start_harmonics(h, net.n, H_full, B, V_m, V_a, st);
+    kernel<<<(unsigned)grid, threads, lu.smem, st>>>(net, solve_args(h, r, mode, lu, workspace));
+    if (net.H != H_full) flat_start_harmonics(h, net.n, H_full, r.B, r.out.V_m, r.out.V_a, st);
     if (h->profiling) { CK(cudaEventRecord(h->ev[2], st)); h->ev_valid = 2; }
     h->launches++;
     CK(cudaGetLastError());
@@ -1721,19 +1762,25 @@ static bool wn_use_dmma(const hpf_t* h, int nZ, int qH, int B) {
     return B >= ZG_BN && nZ >= ZG_BM && qH >= 64;
 }
 
-static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, const double* I_N,
-                     cudaStream_t st) {
-    const size_t off = h->wN_off;
-    const size_t need = off + (size_t)sn.nZ * B;
-    if (need > h->wN_elems) {
-        if (h->d_wN) { CK(cudaDeviceSynchronize()); cudaFree(h->d_wN); h->d_wN = nullptr; h->wN_elems = 0; }
-        CK(cudaMalloc((void**)&h->d_wN, need * sizeof(double2)));
-        h->wN_elems = need;
-    }
-    const int qH = net.q * net.H;
-    if (qH == 0) { CK(cudaMemsetAsync(h->d_wN + off, 0, (need - off) * sizeof(double2), st)); return HPF_OK; }
+// Grow-only w_N scratch of at least `elems` entries
+static int ensure_wn(hpf_t* h, size_t elems) {
+    if (elems <= h->wN_elems) return HPF_OK;
+    if (h->d_wN) { CK(cudaDeviceSynchronize()); cudaFree(h->d_wN); h->d_wN = nullptr; h->wN_elems = 0; }
+    CK(cudaMalloc((void**)&h->d_wN, elems * sizeof(double2)));
+    h->wN_elems = elems;
+    return HPF_OK;
+}
+
+// w_N of a batch into the scratch at offset `off` of h->d_wN; *wN <- where it was written
+static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, const double2* I_N, size_t off,
+                     const double2** wN, cudaStream_t st) {
+    int rc = ensure_wn(h, off + (size_t)sn.nZ * B);
+    if (rc) return rc;
     WnArgs wa;
-    wa.B = B; wa.I_N = (const double2*)I_N; wa.wN = h->d_wN + off;
+    wa.B = B; wa.I_N = I_N; wa.wN = h->d_wN + off;
+    *wN = wa.wN;
+    const int qH = net.q * net.H;
+    if (qH == 0) { CK(cudaMemsetAsync(wa.wN, 0, (size_t)sn.nZ * B * sizeof(double2), st)); return HPF_OK; }
     if (h->shape && h->struct_state == 1 && !h->hWNL.empty()) {
         with_shape(h->shape, [&](auto d) {
             using D = decltype(d);
@@ -1747,13 +1794,11 @@ static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, co
         CK(cudaGetLastError());
         return HPF_OK;
     }
-    if (wn_use_dmma(h, sn.nZ, qH, B)) {
-        int rcz = launch_zgemm(h, sn.nZ, B, qH, sn.WNL, (size_t)qH, (const double2*)I_N, (size_t)B, wa.wN, (size_t)B, st);
-        return rcz;
-    }
+    if (wn_use_dmma(h, sn.nZ, qH, B))
+        return launch_zgemm(h, sn.nZ, B, qH, sn.WNL, (size_t)qH, I_N, (size_t)B, wa.wN, (size_t)B, st);
     const size_t smem = (size_t)(qH < HPF_WN_UCH ? qH : HPF_WN_UCH) * HPF_T * sizeof(double2) + 16;
     int occ = 0;
-    int rc = prep_kernel(h, wn_tile_kernel, smem, "hpf_solve", &occ, 256);
+    rc = prep_kernel(h, wn_tile_kernel, smem, "hpf_solve", &occ, 256);
     if (rc) return rc;
     const long long tiles = ((long long)B + HPF_T - 1) / HPF_T;
     long long grid = (long long)occ * h->sm_count;
@@ -2083,9 +2128,26 @@ static int lu_solve_batched(hpf_t* h, int N, int B, const double* J, size_t stri
     return HPF_OK;
 }
 
+// LsArgs of a request's harmonic stage (wN: its w_N), or of its fundamental stage (fund); the
+// caller carves the work area and sets the wave.
+static LsArgs ls_args(const SolveReq& r, bool fund, const double2* wN) {
+    LsArgs la;
+    memset(&la, 0, sizeof(la));
+    la.B = r.B; la.P = r.P; la.Q = r.Q; la.V_m = r.out.V_m; la.V_a = r.out.V_a; la.status = r.out.status;
+    if (fund) {
+        // the lock-step rounds read the limits of the stage they run and write its iteration counts and
+        // error history through the _h fields: the fundamental stage puts its _f values there
+        la.thresh_h = r.thresh_f; la.max_h = r.max_f; la.n_iter_h = r.out.n_iter_f; la.hist_h = r.hist_f;
+    } else {
+        la.flags = r.flags; la.I_N = r.I_N; la.wN = wN; la.thresh_h = r.thresh_h; la.max_h = r.max_h;
+        la.I_inj = r.out.I_inj; la.n_iter_h = r.out.n_iter_h; la.err_h = r.out.err_h; la.hist_h = r.hist_h;
+    }
+    return la;
+}
+
 // fundamental stage of the large networks in lock step (dense Jacobians of order Nf through the batched LU)
-static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* Q, double thresh_f, int max_f,
-                                double* V_m, double* V_a, int* n_iter_f, int* status, double* hist_f, cudaStream_t st) {
+static int launch_lockstep_fund(hpf_t* h, const SolveReq& r, cudaStream_t st) {
+    const int B = r.B, max_f = r.max_f;
     DevNet nf = devnet(h);
     const int H_full = nf.H, Nf = nf.Nf;
     nf.N = Nf; nf.H = 1; nf.nH = nf.n;
@@ -2095,11 +2157,8 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
     int S = 0;
     int rc = ensure_ls(h, per_slot, B, &S);
     if (rc) return rc;
-    LsArgs la;
-    memset(&la, 0, sizeof(la));
-    la.B = B; la.S = S; la.P = P; la.Q = Q; la.thresh_h = thresh_f; la.max_h = max_f; la.V_m = V_m; la.V_a = V_a;
-    la.n_iter_h = n_iter_f; la.status = status; la.hist_h = hist_f;
-    la.ldb = lub_ld(Nf); la.mat_stride = mat_stride; la.state_stride = state_stride;
+    LsArgs la = ls_args(r, true, nullptr);
+    la.S = S; la.ldb = lub_ld(Nf); la.mat_stride = mat_stride; la.state_stride = state_stride;
     {
         char* p = reinterpret_cast<char*>(h->d_ls);
         la.M = reinterpret_cast<double*>(p);      p += mat_stride * sizeof(double) * (size_t)S;
@@ -2119,13 +2178,13 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
         ls_init_kernel<<<(S + 255) / 256, 256, 0, st>>>(la);
         h->launches++;
         g_ls_timer.mark(0);
-        for (int r = 0; r <= max_f; ++r) {
-            const int cur = r & 1, nxt = cur ^ 1;
-            ls_fund_mismatch_kernel<<<g_mis, 256, 0, st>>>(nf, la, cur, r == 0);
+        for (int it = 0; it <= max_f; ++it) {
+            const int cur = it & 1, nxt = cur ^ 1;
+            ls_fund_mismatch_kernel<<<g_mis, 256, 0, st>>>(nf, la, cur, it == 0);
             ls_compact_kernel<<<1, 1024, 0, st>>>(la, cur);
             h->launches += 2;
             g_ls_timer.mark(1);
-            if (r == max_f) break;
+            if (it == max_f) break;
             ls_fund_jac_kernel<<<g_jac, 256, 0, st>>>(nf, la, nxt);
             h->launches++;
             g_ls_timer.mark(3);
@@ -2133,14 +2192,15 @@ static int launch_lockstep_fund(hpf_t* h, int B, const double* P, const double* 
             if (rc) return rc;
         }
     }
-    if (H_full > 1) flat_start_harmonics(h, nf.n, H_full, B, V_m, V_a, st);
+    if (H_full > 1) flat_start_harmonics(h, nf.n, H_full, B, r.out.V_m, r.out.V_a, st);
     g_ls_timer.report("fundamental stage");
     g_ls_timer.on = false;
     CK(cudaGetLastError());
     return HPF_OK;
 }
 
-static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, const HarmTileArgs& ha, cudaStream_t st) {
+static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, const SolveReq& r, const double2* wN,
+                           cudaStream_t st) {
     const int nx = sn.nx, nZ = sn.nZ, m = net.m, q = net.q;
     const size_t mat_stride = ls_mat_stride(nx);
     const size_t state_stride = (scn_smem_doubles_aligned(net.n, net.H, net.q, net.N) + 15) / 16 * 16;
@@ -2148,14 +2208,12 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
                             (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     // slots: the whole batch when it fits the memory budget, else waves
     {
-        int rcs = ensure_ls(h, per_slot, ha.B, &h->ls_slots);
+        int rcs = ensure_ls(h, per_slot, r.B, &h->ls_slots);
         if (rcs) return rcs;
     }
     const int S = h->ls_slots;
-    LsArgs la;
-    la.B = ha.B; la.S = S; la.flags = ha.flags; la.P = ha.P; la.Q = ha.Q; la.I_N = ha.I_N; la.wN = ha.wN;
-    la.thresh_h = ha.thresh_h; la.max_h = ha.max_h; la.V_m = ha.V_m; la.V_a = ha.V_a; la.I_inj = ha.I_inj;
-    la.n_iter_h = ha.n_iter_h; la.status = ha.status; la.err_h = ha.err_h; la.hist_h = ha.hist_h;
+    LsArgs la = ls_args(r, false, wN);
+    la.S = S;
     {
         char* p = reinterpret_cast<char*>(h->d_ls);
         la.M = reinterpret_cast<double*>(p);      p += mat_stride * sizeof(double) * (size_t)S;
@@ -2175,19 +2233,19 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
     const int g_el = (int)std::min<long long>(((long long)S * m + 255) / 256, (long long)h->sm_count * 8);
     g_ls_timer.on = getenv("HPF_LS_TIMING") != nullptr && !stream_capturing(st);
     g_ls_timer.st = st;
-    for (int b0 = 0; b0 < ha.B; b0 += S) {
+    for (int b0 = 0; b0 < r.B; b0 += S) {
         la.b0 = b0;
-        la.nwave = (ha.B - b0 < S) ? ha.B - b0 : S;
+        la.nwave = (r.B - b0 < S) ? r.B - b0 : S;
         ls_init_kernel<<<(S + 255) / 256, 256, 0, st>>>(la);
         h->launches++;
         g_ls_timer.mark(0);
-        for (int r = 0; r <= ha.max_h; ++r) {
-            const int cur = r & 1, nxt = cur ^ 1;
-            ls_mismatch_kernel<<<g_mis, 256, 0, st>>>(net, sn, la, cur, r == 0);
+        for (int it = 0; it <= r.max_h; ++it) {
+            const int cur = it & 1, nxt = cur ^ 1;
+            ls_mismatch_kernel<<<g_mis, 256, 0, st>>>(net, sn, la, cur, it == 0);
             ls_compact_kernel<<<1, 1024, 0, st>>>(la, cur);
             h->launches += 2;
             g_ls_timer.mark(1);
-            if (r == ha.max_h) break;
+            if (it == r.max_h) break;
             ls_pack_vf_kernel<<<g_el, 256, 0, st>>>(net, la, nxt);
             h->launches++;
             if (q > 0) {
@@ -2213,33 +2271,50 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
     return HPF_OK;
 }
 
-static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, const double* I_N,
-                            double thresh_f, int max_f, double thresh_h, int max_h, int flags,
-                            double* V_m, double* V_a, double* I_inj, int* n_iter_f, int* n_iter_h,
-                            double* err_h, int* status, double* hist_f, double* hist_h, cudaStream_t st) {
+static FundTileArgs fund_tile_args(const SolveReq& r) {
+    FundTileArgs fa;
+    fa.B = r.B; fa.P = r.P; fa.Q = r.Q; fa.thresh_f = r.thresh_f; fa.max_f = r.max_f;
+    fa.V_m = r.out.V_m; fa.V_a = r.out.V_a; fa.n_iter_f = r.out.n_iter_f; fa.status = r.out.status; fa.hist_f = r.hist_f;
+    return fa;
+}
+
+// HarmTileArgs of a request's harmonic stage (wN: its w_N).  With dx_out, one Newton step of the
+// iterate in r.out instead (hpf_newton_step): the update goes to dx_out, and there is no work queue
+// and no lane servicing.
+static HarmTileArgs harm_args(const hpf_t* h, const SolveReq& r, const double2* wN, double* dx_out = nullptr) {
+    const bool step = dx_out != nullptr;
+    HarmTileArgs ha;
+    ha.B = r.B; ha.flags = r.flags; ha.step_only = step ? 1 : 0; ha.P = r.P; ha.Q = r.Q; ha.I_N = r.I_N; ha.wN = wN;
+    ha.thresh_h = r.thresh_h; ha.max_h = r.max_h; ha.V_m = r.out.V_m; ha.V_a = r.out.V_a; ha.I_inj = r.out.I_inj;
+    ha.n_iter_h = r.out.n_iter_h; ha.status = r.out.status; ha.err_h = r.out.err_h; ha.hist_h = r.hist_h;
+    ha.work_counter = step ? nullptr : h->d_counter + r.slot;
+    ha.dx_out = dx_out; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0;
+    ha.epoch = step ? 1 : HPF_HW_SERVICE_EPOCH;
+    return ha;
+}
+
+static int solve_structured(hpf_t* h, const SolveReq& r, cudaStream_t st) {
     const DevNet net = devnet(h);
     const StructNet sn = structnet(h);
+    const int B = r.B;
+    int* const counter = h->d_counter + r.slot;
     // error histories: the unused tail is NaN (all-ones bytes are a quiet NaN)
-    if (hist_f) CK(cudaMemsetAsync(hist_f, 0xff, (size_t)(max_f + 1) * B * sizeof(double), st));
-    if (hist_h) CK(cudaMemsetAsync(hist_h, 0xff, (size_t)(max_h + 1) * B * sizeof(double), st));
-    CK(cudaMemsetAsync(h->d_counter + h->cur_slot, 0, sizeof(int), st));
+    if (r.hist_f) CK(cudaMemsetAsync(r.hist_f, 0xff, (size_t)(r.max_f + 1) * B * sizeof(double), st));
+    if (r.hist_h) CK(cudaMemsetAsync(r.hist_h, 0xff, (size_t)(r.max_h + 1) * B * sizeof(double), st));
+    CK(cudaMemsetAsync(counter, 0, sizeof(int), st));
     if (h->profiling) { CK(cudaEventRecord(h->ev[0], st)); }
     // fundamental stage: one lane per scenario (variant 1) or the per-CTA kernel (variant 2)
     if (h->struct_state >= 2) {
-        int rc = h->struct_state == 3 && use_lockstep(h, net.Nf, B)
-                     ? launch_lockstep_fund(h, B, P, Q, thresh_f, max_f, V_m, V_a, n_iter_f, status, hist_f, st)
-                     : solve_common(h, 1, B, P, Q, nullptr, thresh_f, max_f, 0.0, 0, 0, V_m, V_a, nullptr, n_iter_f,
-                                    nullptr, nullptr, nullptr, status, hist_f, nullptr, st);
+        int rc = h->struct_state == 3 && use_lockstep(h, net.Nf, B) ? launch_lockstep_fund(h, r, st)
+                                                                     : solve_common(h, 1, fund_stage(r), st);
         if (rc) return rc;
-        CK(cudaMemsetAsync(h->d_counter + h->cur_slot, 0, sizeof(int), st));     // solve_common used the counter
+        CK(cudaMemsetAsync(counter, 0, sizeof(int), st));     // solve_common used the counter
     } else {
         const size_t per_warp = fund_tile_doubles_per_warp(net.n, net.Nf) * sizeof(double);
         int warps = 4;
         while (warps > 1 && per_warp * warps > (size_t)h->smem_optin / 2) warps >>= 1;
         const size_t smem = per_warp * warps;
-        FundTileArgs fa;
-        fa.B = B; fa.P = P; fa.Q = Q; fa.thresh_f = thresh_f; fa.max_f = max_f;
-        fa.V_m = V_m; fa.V_a = V_a; fa.n_iter_f = n_iter_f; fa.status = status; fa.hist_f = hist_f;
+        const FundTileArgs fa = fund_tile_args(r);
         const long long tiles = ((long long)B + HPF_T - 1) / HPF_T;
         auto launch = [&](auto kernel) -> int {
             CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -2259,16 +2334,11 @@ static int solve_structured(hpf_t* h, int B, const double* P, const double* Q, c
     if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
     // per-scenario constant w_N = A_ZZ^-1 I_N,Z, then the harmonic stage
     {
-        int rc = launch_wn(h, net, sn, B, I_N, st);
+        const double2* wN = nullptr;
+        int rc = launch_wn(h, net, sn, B, r.I_N, r.wN_off, &wN, st);
         if (rc) return rc;
-        HarmTileArgs ha;
-        ha.B = B; ha.flags = flags; ha.step_only = 0; ha.P = P; ha.Q = Q; ha.I_N = (const double2*)I_N;
-        ha.wN = h->d_wN + h->wN_off;
-        ha.thresh_h = thresh_h; ha.max_h = max_h; ha.V_m = V_m; ha.V_a = V_a; ha.I_inj = (double2*)I_inj;
-        ha.n_iter_h = n_iter_h; ha.status = status; ha.err_h = err_h; ha.work_counter = h->d_counter + h->cur_slot;
-        ha.dx_out = nullptr; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0; ha.hist_h = hist_h; ha.epoch = HPF_HW_SERVICE_EPOCH;
         const bool ls = h->struct_state == 3 && use_lockstep(h, sn.nx, B);
-        rc = ls ? launch_lockstep(h, net, sn, ha, st) : launch_harm(h, net, sn, ha, true, st);
+        rc = ls ? launch_lockstep(h, net, sn, r, wN, st) : launch_harm(h, net, sn, harm_args(h, r, wN), true, st);
         if (rc) return rc;
         h->last_path = ls ? 4 : (h->struct_state >= 2 ? h->struct_state : 1);
     }
@@ -2575,30 +2645,19 @@ long long hpf_jacobian_stride(const hpf_t* h) {
 
 } // extern "C"
 
-// hpf_solve proper; hpf_solve_host calls it per chunk with its own scratch slot selected.
-static int solve_dispatch(hpf_t* h, int B, const double* P, const double* Q, const double* I_N, double thresh_f,
-                          int max_iter_f, double thresh_h, int max_iter_h, int flags, double* V_m, double* V_a,
-                          double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h, int* status,
-                          double* err_hist_f, double* err_hist_h, void* stream) {
+// hpf_solve proper, for a checked request with B > 0 on the handle's device; hpf_solve_host calls it
+// per chunk with the chunk's scratch slot.
+static int solve_dispatch(hpf_t* h, const SolveReq& r, cudaStream_t st) {
     // default strategy: structured Newton step; dense LU when forced or when the network does
     // not admit the structured set-up
-    if (h && !(flags & HPF_SOLVE_DENSE) && B > 0) {
-        int rc = ready(h, "hpf_solve", true);
+    if (!(r.flags & HPF_SOLVE_DENSE)) {
+        int rc = ensure_struct(h, st);
         if (rc) return rc;
-        if (!P || !Q || !V_m || !V_a || !n_iter_f || !n_iter_h || !err_h || !status || (h->q > 0 && !I_N))
-            return fail(h, HPF_E_INVALID, "hpf_solve: NULL buffer");
-        ENTER_DEVICE(h);
-        rc = ensure_struct(h, (cudaStream_t)stream);
-        if (rc) return rc;
-        if (h->struct_state >= 1)
-            return solve_structured(h, B, P, Q, I_N, thresh_f, max_iter_f, thresh_h, max_iter_h, flags,
-                                    V_m, V_a, I_inj, n_iter_f, n_iter_h, err_h, status, err_hist_f, err_hist_h,
-                                    (cudaStream_t)stream);
+        if (h->struct_state >= 1) return solve_structured(h, r, st);
     }
-    const int rcd = solve_common(h, 0, B, P, Q, I_N, thresh_f, max_iter_f, thresh_h, max_iter_h, flags, V_m, V_a,
-                                 I_inj, n_iter_f, n_iter_h, err_h, nullptr, status, err_hist_f, err_hist_h, stream);
-    if (h && rcd == HPF_OK && B > 0) h->last_path = 5;
-    return rcd;
+    const int rc = solve_common(h, 0, r, st);
+    if (rc == HPF_OK) h->last_path = 5;
+    return rc;
 }
 
 extern "C" {
@@ -2607,10 +2666,16 @@ int hpf_solve(hpf_t* h, int B, const double* P, const double* Q, const double* I
               int max_iter_f, double thresh_h, int max_iter_h, int flags, double* V_m, double* V_a,
               double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h, int* status,
               double* err_hist_f, double* err_hist_h, void* stream) {
-    if (h) { h->cur_slot = 0; h->wN_off = 0; }      // (a failed hpf_solve_host may have left them set)
+    SolveReq r;
+    r.B = B; r.flags = flags; r.P = P; r.Q = Q; r.I_N = (const double2*)I_N;
+    r.thresh_f = thresh_f; r.max_f = max_iter_f; r.thresh_h = thresh_h; r.max_h = max_iter_h;
+    r.out.V_m = V_m; r.out.V_a = V_a; r.out.I_inj = (double2*)I_inj;
+    r.out.n_iter_f = n_iter_f; r.out.n_iter_h = n_iter_h; r.out.err_h = err_h; r.out.status = status;
+    r.hist_f = err_hist_f; r.hist_h = err_hist_h;
     return ordered(h, stream, [&] {
-        return solve_dispatch(h, B, P, Q, I_N, thresh_f, max_iter_f, thresh_h, max_iter_h, flags, V_m, V_a, I_inj,
-                              n_iter_f, n_iter_h, err_h, status, err_hist_f, err_hist_h, stream);
+        const int rc = check_request(h, r, 0, "hpf_solve");
+        if (rc || B == 0) return rc;
+        return solve_dispatch(h, r, (cudaStream_t)stream);
     });
 }
 
@@ -2632,9 +2697,12 @@ int hpf_prepare(hpf_t* h, int B_max, void* stream) {
     double *P = buf, *Q = P + n * B, *IN = Q + n * B, *Vm = IN + 2 * q * H * B, *Va = Vm + n * H * B,
            *Inj = Va + n * H * B, *err = Inj + 2 * q * H * B;
     int* iw = reinterpret_cast<int*>(err + B);
-    if (e == cudaSuccess)
-        rc = hpf_solve(h, B_max, P, Q, q ? IN : nullptr, 1e300, 1, 1e300, 1, 0, Vm, Va, q ? Inj : nullptr, iw, iw + B, err,
-                       iw + 2 * B, nullptr, nullptr, stream);
+    SolveReq r;
+    r.B = B_max; r.P = P; r.Q = Q; r.I_N = q ? (const double2*)IN : nullptr;
+    r.thresh_f = 1e300; r.max_f = 1; r.thresh_h = 1e300; r.max_h = 1;
+    r.out.V_m = Vm; r.out.V_a = Va; r.out.I_inj = q ? (double2*)Inj : nullptr;
+    r.out.n_iter_f = iw; r.out.n_iter_h = iw + B; r.out.err_h = err; r.out.status = iw + 2 * B;
+    if (e == cudaSuccess) rc = ordered(h, stream, [&] { return solve_dispatch(h, r, st); });
     const cudaError_t e2 = cudaStreamSynchronize(st);
     cudaFree(buf);
     if (rc) return rc;
@@ -2670,15 +2738,13 @@ static int newton_step_impl(hpf_t* h, int B, const double* V_m, const double* V_
         return fail(h, HPF_E_UNSUPPORTED, "hpf_newton_step: structured strategy not available for this network");
     const DevNet net = devnet(h);
     const StructNet sn = structnet(h);
-    rc = launch_wn(h, net, sn, B, I_N, (cudaStream_t)stream);
+    SolveReq r;
+    r.B = B; r.P = P; r.Q = Q; r.I_N = (const double2*)I_N; r.max_h = 1;
+    r.out.V_m = const_cast<double*>(V_m); r.out.V_a = const_cast<double*>(V_a);
+    const double2* wN = nullptr;
+    rc = launch_wn(h, net, sn, B, r.I_N, 0, &wN, (cudaStream_t)stream);
     if (rc) return rc;
-    HarmTileArgs ha;
-    ha.B = B; ha.flags = 0; ha.step_only = 1; ha.P = P; ha.Q = Q; ha.I_N = (const double2*)I_N;
-    ha.wN = h->d_wN;
-    ha.thresh_h = 0.0; ha.max_h = 1; ha.V_m = const_cast<double*>(V_m); ha.V_a = const_cast<double*>(V_a);
-    ha.I_inj = nullptr; ha.n_iter_h = nullptr; ha.status = nullptr; ha.err_h = nullptr;
-    ha.work_counter = nullptr; ha.dx_out = dx; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0; ha.hist_h = nullptr; ha.epoch = 1;
-    return launch_harm(h, net, sn, ha, false, (cudaStream_t)stream);
+    return launch_harm(h, net, sn, harm_args(h, r, wN, dx), false, (cudaStream_t)stream);
 }
 
 int hpf_newton_step(hpf_t* h, int B, const double* V_m, const double* V_a, const double* P,
@@ -2699,10 +2765,10 @@ int hpf_norton_wn(hpf_t* h, int B, const double* I_N, double* wN, void* stream) 
             return fail(h, HPF_E_UNSUPPORTED, "hpf_norton_wn: structured strategy not available for this network");
         const DevNet net = devnet(h);
         const StructNet sn = structnet(h);
-        h->cur_slot = 0; h->wN_off = 0;
-        rc = launch_wn(h, net, sn, B, I_N, (cudaStream_t)stream);
+        const double2* w = nullptr;
+        rc = launch_wn(h, net, sn, B, (const double2*)I_N, 0, &w, (cudaStream_t)stream);
         if (rc) return rc;
-        CK(cudaMemcpyAsync(wN, h->d_wN, (size_t)sn.nZ * B * sizeof(double2), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+        CK(cudaMemcpyAsync(wN, w, (size_t)sn.nZ * B * sizeof(double2), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
         return HPF_OK;
     });
 }
@@ -2736,9 +2802,13 @@ int hpf_ne_extract(hpf_t* h, int D, int N, const double* Vf, const double* Vh, c
 int hpf_fund_solve(hpf_t* h, int B, const double* P, const double* Q, double thresh_f, int max_iter_f,
                    double* V_m, double* V_a, int* n_iter_f, double* err_f, double* err_hist_f,
                    void* stream) {
+    SolveReq r;
+    r.B = B; r.P = P; r.Q = Q; r.thresh_f = thresh_f; r.max_f = max_iter_f;
+    r.out.V_m = V_m; r.out.V_a = V_a; r.out.n_iter_f = n_iter_f; r.err_f = err_f; r.hist_f = err_hist_f;
     return ordered(h, stream, [&] {
-        return solve_common(h, 1, B, P, Q, nullptr, thresh_f, max_iter_f, 0.0, 0, 0, V_m, V_a, nullptr,
-                            n_iter_f, nullptr, nullptr, err_f, nullptr, err_hist_f, nullptr, stream);
+        const int rc = check_request(h, r, 1, "hpf_fund_solve");
+        if (rc || B == 0) return rc;
+        return solve_common(h, 1, r, (cudaStream_t)stream);
     });
 }
 
@@ -2781,21 +2851,10 @@ static int host_chunk_plan(size_t Bs, size_t* cb, int* streams) {
     return k;
 }
 
-// Device copies of the results that hpf_solve_host_keep leaves behind ([rows, B] layout).
-struct HostKeep {
-    double *V_m = nullptr, *V_a = nullptr, *I_inj = nullptr, *err_h = nullptr;
-    int *n_iter_f = nullptr, *n_iter_h = nullptr, *status = nullptr;
-};
-
-static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, const double* I_N, double thresh_f,
-                           int max_iter_f, double thresh_h, int max_iter_h, double* V_m, double* V_a,
-                           double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h, int* status,
-                           const HostKeep* keep) {
-    int rc = ready(h, "hpf_solve_host", true);
-    if (rc) return rc;
-    if (B <= 0) return B == 0 ? HPF_OK : fail(h, HPF_E_INVALID, "hpf_solve_host: B < 0");
-    if (!P || !Q || !V_m || !V_a || !n_iter_f || !n_iter_h || !err_h || !status || (h->q > 0 && !I_N))
-        return fail(h, HPF_E_INVALID, "hpf_solve_host: NULL buffer");
+// hpf_solve_host: `hr` holds host arrays; keep, when given, receives device copies of the results.
+static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
+    int rc = check_request(h, hr, 0, "hpf_solve_host");
+    if (rc || hr.B == 0) return rc;
     ENTER_DEVICE(h);
     // Pipelined in chunks of scenarios: while chunk k is being solved, chunk k+1 is copied in and
     // the results of chunk k-1 are copied out (PCIe is full duplex); consecutive chunks rotate over
@@ -2807,7 +2866,7 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
     // busy: fewer, larger copies and solves later on (host_chunk_plan).
     // The host arrays are batch-innermost [rows, B]; a chunk is a column block, moved with 2-D
     // copies into compact [rows, Bc] device arrays (pinned host memory makes them asynchronous).
-    const size_t n = h->n, H = h->H, q = h->q, Bs = (size_t)B;
+    const size_t n = h->n, H = h->H, q = h->q, Bs = (size_t)hr.B;
     size_t cb[HPF_HOST_MAX_CHUNKS + 1];
     int ncs = 2;
     const int nchunk = host_chunk_plan(Bs, cb, &ncs);
@@ -2840,11 +2899,8 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
     const size_t wN_rows = (size_t)(h->n * h->H - h->m);
     if (dual) {
         // reserve the w_N scratch of all chunks up front (no reallocation while chunks are in flight)
-        if (wN_rows * Bs > h->wN_elems) {
-            if (h->d_wN) { CK(cudaDeviceSynchronize()); cudaFree(h->d_wN); h->d_wN = nullptr; h->wN_elems = 0; }
-            CK(cudaMalloc((void**)&h->d_wN, wN_rows * Bs * sizeof(double2)));
-            h->wN_elems = wN_rows * Bs;
-        }
+        rc = ensure_wn(h, wN_rows * Bs);
+        if (rc) return rc;
     }
     auto cp2d = [&](void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t rows,
                     cudaMemcpyKind kind, cudaStream_t st) {
@@ -2861,6 +2917,7 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
         for (auto& ev : tle) cudaEventCreate(&ev);
         cudaEventRecord(tle[3 * HPF_HOST_MAX_CHUNKS], s_in);
     }
+    const BatchOut& ho = hr.out;
     for (int k = 0; k < nchunk && !rc; ++k) {
         const size_t b0 = cb[k], Bc = cb[k + 1] - cb[k];
         double* d = h->d_io + per_scn * b0;
@@ -2869,32 +2926,35 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
         int *di_f = di_all + b0, *di_h = di_all + Bp + b0, *di_s = di_all + 2 * Bp + b0;
         const size_t w8 = Bc * sizeof(double), w16 = Bc * 2 * sizeof(double);
         const size_t p8 = Bs * sizeof(double), p16 = Bs * 2 * sizeof(double);
-        e = cp2d(dP, w8, P + b0, p8, w8, n, cudaMemcpyHostToDevice, s_in);
-        if (e == cudaSuccess) e = cp2d(dQ, w8, Q + b0, p8, w8, n, cudaMemcpyHostToDevice, s_in);
+        e = cp2d(dP, w8, hr.P + b0, p8, w8, n, cudaMemcpyHostToDevice, s_in);
+        if (e == cudaSuccess) e = cp2d(dQ, w8, hr.Q + b0, p8, w8, n, cudaMemcpyHostToDevice, s_in);
         if (e == cudaSuccess && q)
-            e = cp2d(dI, w16, I_N + 2 * b0, p16, w16, q * H, cudaMemcpyHostToDevice, s_in);
+            e = cp2d(dI, w16, hr.I_N + b0, p16, w16, q * H, cudaMemcpyHostToDevice, s_in);
         cudaStream_t s_cmp = h->st_io[dual ? cmp_stream[k % ncs] : 1];
-        h->cur_slot = dual ? k : 0;
-        h->wN_off = dual ? wN_rows * b0 : 0;
         if (e == cudaSuccess) e = cudaEventRecord(h->ev_io[k], s_in);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(s_cmp, h->ev_io[k], 0);
         if (e != cudaSuccess) break;
         if (tl) cudaEventRecord(tle[3 * k], s_in);
-        rc = solve_dispatch(h, (int)Bc, dP, dQ, dI, thresh_f, max_iter_f, thresh_h, max_iter_h, 0, dVm, dVa,
-                       I_inj ? dInj : nullptr, di_f, di_h, dErr, di_s, nullptr, nullptr, s_cmp);
+        SolveReq c = hr;          // the same thresholds and limits on the chunk's device buffers
+        c.B = (int)Bc; c.P = dP; c.Q = dQ; c.I_N = (const double2*)dI;
+        c.out.V_m = dVm; c.out.V_a = dVa; c.out.I_inj = ho.I_inj ? (double2*)dInj : nullptr;
+        c.out.n_iter_f = di_f; c.out.n_iter_h = di_h; c.out.err_h = dErr; c.out.status = di_s;
+        c.slot = dual ? k : 0;
+        c.wN_off = dual ? wN_rows * b0 : 0;
+        rc = solve_dispatch(h, c, s_cmp);
         if (rc) break;
         e = cudaEventRecord(h->ev_io[HPF_HOST_MAX_CHUNKS + k], s_cmp);
         if (tl) cudaEventRecord(tle[3 * k + 1], s_cmp);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(s_out, h->ev_io[HPF_HOST_MAX_CHUNKS + k], 0);
-        if (e == cudaSuccess) e = cp2d(V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
-        if (e == cudaSuccess) e = cp2d(V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
-        if (e == cudaSuccess && I_inj && q)
-            e = cp2d(I_inj + 2 * b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToHost, s_out);
+        if (e == cudaSuccess) e = cp2d(ho.V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
+        if (e == cudaSuccess) e = cp2d(ho.V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
+        if (e == cudaSuccess && ho.I_inj && q)
+            e = cp2d(ho.I_inj + b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToHost, s_out);
         if (e == cudaSuccess && k == nchunk - 1) {       // s_out has waited for every chunk by now
-            e = cudaMemcpyAsync(err_h, dErr_all, Bs * sizeof(double), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(n_iter_f, di_all, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(n_iter_h, di_all + Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(status, di_all + 2 * Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            e = cudaMemcpyAsync(ho.err_h, dErr_all, Bs * sizeof(double), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.n_iter_f, di_all, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.n_iter_h, di_all + Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.status, di_all + 2 * Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
         }
         if (tl) cudaEventRecord(tle[3 * k + 2], s_out);
         if (e == cudaSuccess && keep) {
@@ -2902,8 +2962,8 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
             // 2-D copies on the compute stream, ~20 us for the whole batch)
             e = cp2d(keep->V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToDevice, s_cmp);
             if (e == cudaSuccess) e = cp2d(keep->V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess && keep->I_inj && I_inj && q)
-                e = cp2d(keep->I_inj + 2 * b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->I_inj && ho.I_inj && q)
+                e = cp2d(keep->I_inj + b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToDevice, s_cmp);
             if (e == cudaSuccess) e = cudaMemcpyAsync(keep->err_h + b0, dErr, Bc * sizeof(double), cudaMemcpyDeviceToDevice, s_cmp);
             if (e == cudaSuccess) e = cudaMemcpyAsync(keep->n_iter_f + b0, di_f, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
             if (e == cudaSuccess) e = cudaMemcpyAsync(keep->n_iter_h + b0, di_h, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
@@ -2911,8 +2971,6 @@ static int solve_host_impl(hpf_t* h, int B, const double* P, const double* Q, co
         }
         if (e != cudaSuccess) break;
     }
-    h->cur_slot = 0;
-    h->wN_off = 0;
     if (!rc && e != cudaSuccess) rc = fail(h, HPF_E_CUDA, std::string("hpf_solve_host: ") + cudaGetErrorString(e));
     for (int i = 0; i < 6; ++i) {
         const cudaError_t e2 = cudaStreamSynchronize(h->st_io[i]);
@@ -2936,8 +2994,12 @@ extern "C" {
 int hpf_solve_host(hpf_t* h, int B, const double* P, const double* Q, const double* I_N, double thresh_f,
                    int max_iter_f, double thresh_h, int max_iter_h, double* V_m, double* V_a,
                    double* I_inj, int* n_iter_f, int* n_iter_h, double* err_h, int* status) {
-    return solve_host_impl(h, B, P, Q, I_N, thresh_f, max_iter_f, thresh_h, max_iter_h, V_m, V_a, I_inj,
-                           n_iter_f, n_iter_h, err_h, status, nullptr);
+    SolveReq r;
+    r.B = B; r.P = P; r.Q = Q; r.I_N = (const double2*)I_N;
+    r.thresh_f = thresh_f; r.max_f = max_iter_f; r.thresh_h = thresh_h; r.max_h = max_iter_h;
+    r.out.V_m = V_m; r.out.V_a = V_a; r.out.I_inj = (double2*)I_inj;
+    r.out.n_iter_f = n_iter_f; r.out.n_iter_h = n_iter_h; r.out.err_h = err_h; r.out.status = status;
+    return solve_host_impl(h, r, nullptr);
 }
 
 int hpf_solve_host_keep(hpf_t* h, int B, const double* P, const double* Q, const double* I_N, double thresh_f,
@@ -2947,11 +3009,15 @@ int hpf_solve_host_keep(hpf_t* h, int B, const double* P, const double* Q, const
                         double* derr_h, int* dstatus) {
     if (!dV_m || !dV_a || !dn_iter_f || !dn_iter_h || !derr_h || !dstatus)
         return fail(h, HPF_E_INVALID, "hpf_solve_host_keep: NULL device buffer");
-    HostKeep k;
-    k.V_m = dV_m; k.V_a = dV_a; k.I_inj = dI_inj; k.err_h = derr_h;
+    SolveReq r;
+    r.B = B; r.P = P; r.Q = Q; r.I_N = (const double2*)I_N;
+    r.thresh_f = thresh_f; r.max_f = max_iter_f; r.thresh_h = thresh_h; r.max_h = max_iter_h;
+    r.out.V_m = V_m; r.out.V_a = V_a; r.out.I_inj = (double2*)I_inj;
+    r.out.n_iter_f = n_iter_f; r.out.n_iter_h = n_iter_h; r.out.err_h = err_h; r.out.status = status;
+    BatchOut k;
+    k.V_m = dV_m; k.V_a = dV_a; k.I_inj = (double2*)dI_inj; k.err_h = derr_h;
     k.n_iter_f = dn_iter_f; k.n_iter_h = dn_iter_h; k.status = dstatus;
-    return solve_host_impl(h, B, P, Q, I_N, thresh_f, max_iter_f, thresh_h, max_iter_h, V_m, V_a, I_inj,
-                           n_iter_f, n_iter_h, err_h, status, &k);
+    return solve_host_impl(h, r, &k);
 }
 
 static int mismatch_impl(hpf_t* h, int B, const double* V_m, const double* V_a, const double* P, const double* Q,

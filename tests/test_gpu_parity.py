@@ -368,11 +368,13 @@ def test_host_entry_point_chunked_pipeline(solvers, tmp_path):
 def test_host_entry_point_chunk_plans(solvers, monkeypatch, plan, streams, B):
     """$HPF_HOST_PLAN / $HPF_HOST_STREAMS (growing chunks of hpf_solve_host over 1..4 compute streams,
     more sizes than chunk slots, a last chunk of odd length, a plan larger than the batch): host results
-    and the device copy of hpf_solve_host_keep carry the bits of the device-resident call."""
+    and the device copy of hpf_solve_host_keep carry the bits of the device-resident call, and the
+    per-chunk w_N scratch of the call leaves hpf_norton_wn unchanged."""
     from harmonic_power_flow_b200 import scenarios
     sol, net, _ = solvers("net3_c_h25")
     P, Q, I_N = scenarios.make_batch(net, B, "tight")
     a = sol.solve(P, Q, I_N).to_host()
+    wn = sol.norton_wn(I_N).cpu().numpy()
     monkeypatch.setenv("HPF_HOST_PLAN", plan)
     monkeypatch.setenv("HPF_HOST_STREAMS", str(streams))
     b = sol.solve_host(P, Q, I_N, keep=True)
@@ -381,6 +383,7 @@ def test_host_entry_point_chunk_plans(solvers, monkeypatch, plan, streams, B):
         assert np.array_equal(a[k], b[k]), k
         assert np.array_equal(a[k], dev[k]), k
     assert (b["status"] == 0).all()
+    assert np.array_equal(sol.norton_wn(I_N).cpu().numpy(), wn)
 
 
 def test_fused_solve_equals_stepwise_kernels(solvers, tmp_path, monkeypatch):
@@ -590,14 +593,22 @@ def test_invalid_arguments_are_refused_loudly(solvers):
     sol, net, d = solvers("net3_c_h25")
     with pytest.raises(ValueError):
         sol.solve(net.P[:, None], net.Q[:, None], net.I_N[:, :1, None])       # wrong I_N shape
-    with pytest.raises(_lib.HpfError) as e:
-        _lib.check(sol._h, sol.lib.hpf_solve(sol._h, 1, None, None, None, 1e-6, 30, 1e-4, 50, 0, None, None,
-                                             None, None, None, None, None, None, None, None))
-    assert e.value.code == _lib.HPF_E_INVALID and "NULL" in str(e.value)
-    with pytest.raises(_lib.HpfError) as e:
-        _lib.check(sol._h, sol.lib.hpf_solve(sol._h, -1, None, None, None, 1e-6, 30, 1e-4, 50, 0, None, None,
-                                             None, None, None, None, None, None, None, None))
-    assert e.value.code == _lib.HPF_E_INVALID
+    lib, h = sol.lib, sol._h
+
+    def refused(rc, msg):
+        with pytest.raises(_lib.HpfError) as e:
+            _lib.check(h, rc)
+        assert e.value.code == _lib.HPF_E_INVALID and msg in str(e.value), str(e.value)
+
+    # every solve entry point, with each of its paths, checks its request before it runs
+    for flags in (0, _lib.SOLVE_DENSE):
+        refused(lib.hpf_solve(h, 1, None, None, None, 1e-6, 30, 1e-4, 50, flags, *[None] * 10),
+                "hpf_solve: NULL buffer")
+    refused(lib.hpf_solve(h, -1, None, None, None, 1e-6, 30, 1e-4, 50, 0, *[None] * 10), "hpf_solve: B < 0")
+    refused(lib.hpf_fund_solve(h, 1, None, None, 1e-6, 30, *[None] * 6), "hpf_fund_solve: NULL buffer")
+    refused(lib.hpf_solve_host(h, 1, None, None, None, 1e-6, 30, 1e-4, 50, *[None] * 7),
+            "hpf_solve_host: NULL buffer")
+    refused(lib.hpf_solve_host(h, -1, None, None, None, 1e-6, 30, 1e-4, 50, *[None] * 7), "hpf_solve_host: B < 0")
 
 
 # ---------------------------------------------------------------- drop-in API
