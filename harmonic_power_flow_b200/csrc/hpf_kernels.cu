@@ -13,6 +13,7 @@
 #include <cstdlib>
 #include <chrono>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
 #include <vector>
@@ -1046,33 +1047,55 @@ __global__ void bus_currents_kernel(const DevNet net, int B, const double* __res
 #define HPF_LS_AUTO_MIN_B 128           // large networks: batches of at least this many scenarios take the lock-step path
 #define HPF_LS_MAX_ORDER 2048           // largest system of the lock-step LU (panel kernel: at most 4 rows per thread of 512)
 #define HPF_HW_SERVICE_EPOCH 3          // service interval of finished lanes in the one-warp-per-harmonic kernel (profiles/r2_small_batch_ab.txt)
+
+// Owners of CUDA resources: device memory, streams and events are released when they are reset or
+// replaced, and when the handle is deleted.  AsyncPtr frees in stream order, on the stream it holds.
+struct CudaFree { void operator()(void* p) const { cudaFree(p); } };
+struct AsyncFree { cudaStream_t st = nullptr; void operator()(void* p) const { cudaFreeAsync(p, st); } };
+struct StreamDestroy { void operator()(cudaStream_t s) const { cudaStreamDestroy(s); } };
+struct EventDestroy { void operator()(cudaEvent_t e) const { cudaEventDestroy(e); } };
+template <class T> using DevPtr = std::unique_ptr<T, CudaFree>;
+template <class T> using AsyncPtr = std::unique_ptr<T, AsyncFree>;
+using Stream = std::unique_ptr<CUstream_st, StreamDestroy>;
+using Event = std::unique_ptr<CUevent_st, EventDestroy>;
+
+// A grow-only scratch buffer and its size in bytes (see grow)
+template <class T>
+struct Scratch {
+    DevPtr<T> p;
+    size_t bytes = 0;
+    T* get() const { return p.get(); }
+};
+
+// Operators of the structured strategy (ensure_struct): built, and dropped, together
+struct StructBufs {
+    DevPtr<double2> Ainv, Gz, GzT, WNL;
+    DevPtr<int> nbr_ptr, nbr_idx;
+};
+
 struct hpf_handle {
     int device = 0;
     int sm_count = 0;
     int smem_optin = 0;
     int n = 0, m = 0, c = 0, H = 0, q = 0, L = 0, n_dev = 0, coupled = 0;
     bool have_net = false, have_dev = false, have_Y = false;
-    int *d_harm = nullptr, *d_from = nullptr, *d_to = nullptr, *d_devof = nullptr;
-    double *d_R = nullptr, *d_X = nullptr, *d_G = nullptr, *d_B = nullptr, *d_Xsh = nullptr;
-    double *d_tau = nullptr, *d_phase = nullptr;             // optional transformer data (hpf_set_transformers)
+    DevPtr<int> d_harm, d_from, d_to, d_devof;
+    DevPtr<double> d_R, d_X, d_G, d_B, d_Xsh;
+    DevPtr<double> d_tau, d_phase;                           // optional transformer data (hpf_set_transformers)
     int y_flags = 0;                                         // HPF_Y_* (hpf_set_y_options)
-    double2 *d_Y = nullptr, *d_YN = nullptr;
-    int* d_counter = nullptr;
-    double* d_work = nullptr;
-    size_t work_doubles = 0;
-    double* d_io = nullptr;       // staging buffers of hpf_solve_host (grow-only)
-    size_t io_doubles = 0;
-    cudaStream_t st_io[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // copy-in, compute, copy-out, compute 2..4
-    cudaEvent_t ev_io[2 * HPF_HOST_MAX_CHUNKS] = {};
+    DevPtr<double2> d_Y, d_YN;
+    DevPtr<int> d_counter;
+    Scratch<double> d_work;
+    Scratch<double> d_io;         // staging buffers of hpf_solve_host
+    Stream st_io[6];              // copy-in, compute, copy-out, compute 2..4
+    Event ev_io[2 * HPF_HOST_MAX_CHUNKS];
     // structured strategy: 0 = not set up yet, 1 = ready, -1 = not available for this network
     int struct_state = 0;
-    double2 *d_Ainv = nullptr, *d_Gz = nullptr, *d_GzT = nullptr, *d_WNL = nullptr, *d_wN = nullptr;
-    int *d_nbr_ptr = nullptr, *d_nbr_idx = nullptr;
-    int* d_ell_col = nullptr;     // sparsity pattern of Y(h) for the larger networks (see DevNet)
+    StructBufs d_struct;
+    Scratch<double2> d_wN;
+    DevPtr<int> d_ell_col;        // sparsity pattern of Y(h) for the larger networks (see DevNet)
     int ell_w = 0;
-    double* d_gstate = nullptr;   // variant 3: per-CTA scenario state slabs
-    size_t gstate_doubles = 0;
-    size_t wN_elems = 0;
+    Scratch<double> d_gstate;     // variant 3: per-CTA scenario state slabs
     int no_specialise = 0;        // $HPF_NO_SPECIALISE=1: always use the runtime-dimension kernels
     int shape = 0;                // shape-specialised instances of the network (see with_shape), 0 = none
     int fund_shape = 0;           // the same for fund_tile_kernel, matched on (n, c) only: it reads no other dimension
@@ -1086,9 +1109,7 @@ struct hpf_handle {
     // lock-step batched harmonic stage of the large networks (hpf_lockstep.cuh)
     int lockstep = -1;            // $HPF_LOCKSTEP=0|1: never / always; default (-1): batches of at least HPF_LS_AUTO_MIN_B scenarios
     size_t ls_budget = 0;         // $HPF_LOCKSTEP_GB: device memory the lock-step work areas may take (0 = 40 % of the free memory, at most 64 GB)
-    void* d_ls = nullptr;         // one allocation: state slabs | border systems | X | GX | U0 | ints
-    size_t ls_bytes = 0;
-    int ls_slots = 0;
+    Scratch<char> d_ls;           // one allocation: state slabs | border systems | X | GX | U0 | ints
     int last_path = 0;            // hpf_last_solve_path
     // host mirror of the network constants for kernels that take them as parameters
     // (constant bank): fetched lazily from the device tables, see host_consts()
@@ -1100,10 +1121,10 @@ struct hpf_handle {
     bool host_consts_valid = false;
     double pivot_min = 0.0, pivot_max = 0.0;
     int profiling = 0;
-    cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};
+    Event ev[3];
     int ev_valid = 0;             // 0 none, 1 structured (3 events), 2 dense (ev[1], ev[2])
     long long launches = 0;
-    cudaEvent_t ev_last = nullptr;     // recorded after the last kernel sequence of this handle
+    Event ev_last;                // recorded after the last kernel sequence of this handle
     cudaStream_t last_stream = nullptr;
     bool last_valid = false;
     std::string err;
@@ -1149,12 +1170,12 @@ static bool stream_capturing(cudaStream_t st) {
     return cs != cudaStreamCaptureStatusNone;
 }
 static int order_after_previous(hpf_t* h, cudaStream_t st) {
-    if (h->last_valid && st != h->last_stream && !stream_capturing(st)) CK(cudaStreamWaitEvent(st, h->ev_last, 0));
+    if (h->last_valid && st != h->last_stream && !stream_capturing(st)) CK(cudaStreamWaitEvent(st, h->ev_last.get(), 0));
     return HPF_OK;
 }
 static int mark_last(hpf_t* h, cudaStream_t st) {
     if (stream_capturing(st)) return HPF_OK;
-    CK(cudaEventRecord(h->ev_last, st));
+    CK(cudaEventRecord(h->ev_last.get(), st));
     h->last_stream = st;
     h->last_valid = true;
     return HPF_OK;
@@ -1180,17 +1201,63 @@ static DevNet devnet(const hpf_t* h) {
     d.N = 2 * d.nH - 1 - h->c;
     d.Nf = 2 * h->n - 1 - h->c;
     d.coupled = h->coupled;
-    d.Y = h->d_Y; d.YN = h->d_YN; d.dev_of_nl = h->d_devof;
-    d.ell_col = h->d_ell_col; d.ell_w = h->ell_w;
+    d.Y = h->d_Y.get(); d.YN = h->d_YN.get(); d.dev_of_nl = h->d_devof.get();
+    d.ell_col = h->d_ell_col.get(); d.ell_w = h->ell_w;
     return d;
 }
 
+// Reports a failed allocation of `bytes` for `who` (entry point and buffer).  A failed allocation
+// leaves its error as the runtime's last error, which is consumed here: the next launch check
+// would otherwise report it as its own.
+static int alloc_failed(hpf_t* h, cudaError_t e, const char* who, size_t bytes) {
+    cudaGetLastError();
+    return fail(h, e == cudaErrorMemoryAllocation ? HPF_E_NOMEM : HPF_E_CUDA,
+                std::string(who) + ": allocation of " + std::to_string(bytes) + " B: " + cudaGetErrorString(e));
+}
+
+// Frees what p holds, then allocates `bytes` into it
 template <class T>
-static cudaError_t upload(T** dst, const T* src, size_t count) {
-    if (*dst) { cudaFree(*dst); *dst = nullptr; }
-    cudaError_t e = cudaMalloc((void**)dst, (count ? count : 1) * sizeof(T));
-    if (e != cudaSuccess) return e;
-    if (src && count) e = cudaMemcpy(*dst, src, count * sizeof(T), cudaMemcpyHostToDevice);
+static int dev_alloc(hpf_t* h, DevPtr<T>& p, size_t bytes, const char* who) {
+    p.reset();
+    void* raw = nullptr;
+    const cudaError_t e = cudaMalloc(&raw, bytes);
+    if (e != cudaSuccess) return alloc_failed(h, e, who, bytes);
+    p.reset(static_cast<T*>(raw));
+    return HPF_OK;
+}
+
+template <class T>
+static int upload(hpf_t* h, DevPtr<T>& dst, const T* src, size_t count, const char* who) {
+    const int rc = dev_alloc(h, dst, (count ? count : 1) * sizeof(T), who);
+    if (rc) return rc;
+    if (src && count) CK(cudaMemcpy(dst.get(), src, count * sizeof(T), cudaMemcpyHostToDevice));
+    return HPF_OK;
+}
+
+// Grow-only scratch: reallocated only for a request larger than any before it.  Work in flight may
+// still read the old buffer, so the device is synchronised before it is freed; after
+// hpf_prepare(B_max), solves of up to B_max scenarios return at the first line.
+template <class T>
+static int grow(hpf_t* h, Scratch<T>& buf, size_t bytes, const char* who) {
+    if (bytes <= buf.bytes) return HPF_OK;
+    if (buf.p) CK(cudaDeviceSynchronize());
+    const int rc = dev_alloc(h, buf.p, bytes, who);
+    buf.bytes = rc ? 0 : bytes;
+    return rc;
+}
+
+// Y(h) or the device tables changed: the structured operators and the host mirrors are rebuilt
+// when next needed.  `pattern`: Y(h) itself changed, so its sparsity pattern goes as well.
+static void invalidate_derived(hpf_t* h, bool pattern) {
+    h->struct_state = 0;
+    h->host_consts_valid = false;
+    if (pattern) { h->d_ell_col.reset(); h->ell_w = 0; }
+}
+
+static cudaError_t create_event(Event& ev, unsigned flags) {
+    cudaEvent_t raw = nullptr;
+    const cudaError_t e = cudaEventCreateWithFlags(&raw, flags);
+    if (e == cudaSuccess) ev.reset(raw);
     return e;
 }
 
@@ -1207,14 +1274,6 @@ static int ready(hpf_t* h, const char* who, bool need_dev) {
 static bool fits_smem_lu(const hpf_t* h, const DevNet& net) {
     return net.N <= 32 * HPF_LU_MAXCHUNK &&
            scn_smem_bytes(net.n, net.H, net.q, net.N, true) <= (size_t)h->smem_optin;
-}
-
-static int ensure_workspace(hpf_t* h, size_t doubles) {
-    if (doubles <= h->work_doubles) return HPF_OK;
-    if (h->d_work) { CK(cudaDeviceSynchronize()); cudaFree(h->d_work); h->d_work = nullptr; h->work_doubles = 0; }
-    CK(cudaMalloc((void**)&h->d_work, doubles * sizeof(double)));
-    h->work_doubles = doubles;
-    return HPF_OK;
 }
 
 template <class K>
@@ -1333,7 +1392,7 @@ static SolveArgs solve_args(const hpf_t* h, const SolveReq& r, int mode, const L
     a.V_m = r.out.V_m; a.V_a = r.out.V_a; a.I_inj = r.out.I_inj;
     a.n_iter_f = r.out.n_iter_f; a.n_iter_h = r.out.n_iter_h; a.status = r.out.status; a.err_h = r.out.err_h;
     a.err_f = r.err_f;
-    a.work_counter = h->d_counter + r.slot;
+    a.work_counter = h->d_counter.get() + r.slot;
     a.workspace = workspace;
     a.lub_doubles = (int)lu.lubd;
     a.lu_classic = h->lu_classic;
@@ -1359,20 +1418,21 @@ static int solve_common(hpf_t* h, int mode, const SolveReq& r, cudaStream_t st) 
     int occ = 0;
     int rc = prep_kernel(h, kernel, lu.smem, who, &occ, threads);
     if (rc) return rc;
-    CK(cudaMemsetAsync(h->d_counter + r.slot, 0, sizeof(int), st));
+    CK(cudaMemsetAsync(h->d_counter.get() + r.slot, 0, sizeof(int), st));
     long long grid = (long long)occ * h->sm_count;
     if (grid > r.B) grid = r.B;
     if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
     double* workspace = nullptr;
     if (lu.kind) {
-        rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
+        rc = grow(h, h->d_work, (size_t)grid * lub_ld(net.N) * (net.N + 1) * sizeof(double),
+                  mode ? "hpf_fund_solve: LU workspace" : "hpf_solve: LU workspace");
         if (rc) return rc;
-        workspace = h->d_work;
+        workspace = h->d_work.get();
     }
-    if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
+    if (h->profiling) { CK(cudaEventRecord(h->ev[1].get(), st)); }
     kernel<<<(unsigned)grid, threads, lu.smem, st>>>(net, solve_args(h, r, mode, lu, workspace));
     if (net.H != H_full) flat_start_harmonics(h, net.n, H_full, r.B, r.out.V_m, r.out.V_a, st);
-    if (h->profiling) { CK(cudaEventRecord(h->ev[2], st)); h->ev_valid = 2; }
+    if (h->profiling) { CK(cudaEventRecord(h->ev[2].get(), st)); h->ev_valid = 2; }
     h->launches++;
     CK(cudaGetLastError());
     return HPF_OK;
@@ -1383,12 +1443,12 @@ static StructNet structnet(const hpf_t* h) {
     StructNet s;
     s.nZ = h->n * h->H - h->m;
     s.nx = (h->m - 1) + (h->m - h->c);
-    s.Ainv = h->d_Ainv;
-    s.G = h->d_Gz;
-    s.GT = h->d_GzT;
-    s.nbr_ptr = h->d_nbr_ptr;
-    s.nbr_idx = h->d_nbr_idx;
-    s.WNL = h->d_WNL;
+    s.Ainv = h->d_struct.Ainv.get();
+    s.G = h->d_struct.Gz.get();
+    s.GT = h->d_struct.GzT.get();
+    s.nbr_ptr = h->d_struct.nbr_ptr.get();
+    s.nbr_idx = h->d_struct.nbr_idx.get();
+    s.WNL = h->d_struct.WNL.get();
     s.yn_elems = h->n_dev * (h->coupled ? h->H * h->H : h->H);
     return s;
 }
@@ -1444,29 +1504,23 @@ static int gj_invert(hpf_t* h, double2* A, int nn, int* ipiv, int* info, double*
     return HPF_OK;
 }
 
+template <class T>
+static int alloc_async(hpf_t* h, AsyncPtr<T>& p, size_t count, cudaStream_t st, const char* who) {
+    void* raw = nullptr;
+    const cudaError_t e = cudaMallocAsync(&raw, count * sizeof(T), st);
+    if (e != cudaSuccess) return alloc_failed(h, e, who, count * sizeof(T));
+    p = AsyncPtr<T>(static_cast<T*>(raw), AsyncFree{st});
+    return HPF_OK;
+}
+
 // Structured set-up of the large networks through the block structure of A_ZZ (Woodbury identity,
-// see hpf_structured.cuh): fills d_WNL, d_Gz, d_GzT; *info_out = 0 or a zero-pivot indicator,
+// see hpf_structured.cuh): fills the operators W_NL, G, G^T; *info_out = 0 or a zero-pivot indicator,
 // prh = min / max pivot modulus over all inversions.
 static int setup_woodbury(hpf_t* h, const DevNet& net, cudaStream_t st, int* info_out, double* prh) {
     const int n = net.n, m = net.m, q = net.q, H = net.H, qH = q * H, nZ = net.nH - m;
     const size_t nblk = (size_t)q * q + (size_t)(H - 1) * n * n;
     const int nmax = n > qH ? n : qH;
-    double2 *Dinv = nullptr, *Mx = nullptr, *T = nullptr, *U = nullptr, *tmp = nullptr, *FR = nullptr;
-    int *ipiv = nullptr, *info = nullptr;
-    double* pr = nullptr;
-    // (stream-ordered allocations: a plain cudaFree of these ~1.7 GB of temporaries costs 160 ms)
-    auto cleanup = [&] {
-        cudaFreeAsync(Dinv, st); cudaFreeAsync(Mx, st); cudaFreeAsync(T, st); cudaFreeAsync(U, st); cudaFreeAsync(tmp, st);
-        cudaFreeAsync(FR, st); cudaFreeAsync(ipiv, st); cudaFreeAsync(info, st); cudaFreeAsync(pr, st);
-    };
-#define WB(call)                                                                                  \
-    do {                                                                                          \
-        cudaError_t e_ = (call);                                                                  \
-        if (e_ != cudaSuccess) {                                                                  \
-            cleanup();                                                                            \
-            return fail(h, HPF_E_CUDA, std::string("structured setup: " #call ": ") + cudaGetErrorString(e_)); \
-        }                                                                                         \
-    } while (0)
+    double2 *const WNL = h->d_struct.WNL.get(), *const Gz = h->d_struct.Gz.get(), *const GzT = h->d_struct.GzT.get();
     const bool timing = getenv("HPF_SETUP_TIMING") != nullptr;       // phase times on stderr (synchronises)
     auto now = [] { return std::chrono::steady_clock::now(); };
     auto tprev = now();
@@ -1477,60 +1531,63 @@ static int setup_woodbury(hpf_t* h, const DevNet& net, cudaStream_t st, int* inf
         fprintf(stderr, "[hpf setup] %-34s %8.1f ms\n", what, std::chrono::duration<double, std::milli>(t - tprev).count());
         tprev = t;
     };
-    WB(cudaMallocAsync((void**)&Dinv, (nblk + 1) * sizeof(double2), st));
-    WB(cudaMallocAsync((void**)&Mx, ((size_t)qH * qH + 1) * sizeof(double2), st));
-    WB(cudaMallocAsync((void**)&T, ((size_t)q * m + 1) * sizeof(double2), st));
-    WB(cudaMallocAsync((void**)&U, ((size_t)qH * m + 1) * sizeof(double2), st));
-    WB(cudaMallocAsync((void**)&tmp, ((size_t)2 * nmax + 1) * sizeof(double2), st));
-    WB(cudaMallocAsync((void**)&FR, ((size_t)2 * nmax * GJB_NB + GJB_NB + 1) * sizeof(double2), st));      // F, R, 1 / pivots
-    WB(cudaMallocAsync((void**)&ipiv, (size_t)(nmax + 2) * sizeof(int), st));
-    WB(cudaMallocAsync((void**)&info, (size_t)(H + 1) * sizeof(int), st));
-    WB(cudaMallocAsync((void**)&pr, (size_t)2 * (H + 1) * sizeof(double), st));
+    // stream-ordered temporaries: a plain cudaFree of these ~1.7 GB costs 160 ms
+    AsyncPtr<double2> Dinv, Mx, T, U, tmp, FR;
+    AsyncPtr<int> ipiv, info;
+    AsyncPtr<double> pr;
+    const char* who = "structured set-up: Woodbury temporaries";
+    int rc = alloc_async(h, Dinv, nblk + 1, st, who);
+    if (!rc) rc = alloc_async(h, Mx, (size_t)qH * qH + 1, st, who);
+    if (!rc) rc = alloc_async(h, T, (size_t)q * m + 1, st, who);
+    if (!rc) rc = alloc_async(h, U, (size_t)qH * m + 1, st, who);
+    if (!rc) rc = alloc_async(h, tmp, (size_t)2 * nmax + 1, st, who);
+    if (!rc) rc = alloc_async(h, FR, (size_t)2 * nmax * GJB_NB + GJB_NB + 1, st, who);      // F, R, 1 / pivots
+    if (!rc) rc = alloc_async(h, ipiv, (size_t)nmax + 2, st, who);
+    if (!rc) rc = alloc_async(h, info, (size_t)H + 1, st, who);
+    if (!rc) rc = alloc_async(h, pr, (size_t)2 * (H + 1), st, who);
+    if (rc) return rc;
     tick("allocations");
-    wb_blocks_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv);
+    wb_blocks_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv.get());
     h->launches++;
-    int rc = HPF_OK;
     for (int hh = 0; hh < H && !rc; ++hh) {
-        double2* blk = hh == 0 ? Dinv : Dinv + (size_t)q * q + (size_t)(hh - 1) * n * n;
-        rc = gj_invert(h, blk, hh == 0 ? q : n, ipiv, info + hh, pr + 2 * hh, tmp, st, FR);
+        double2* blk = hh == 0 ? Dinv.get() : Dinv.get() + (size_t)q * q + (size_t)(hh - 1) * n * n;
+        rc = gj_invert(h, blk, hh == 0 ? q : n, ipiv.get(), info.get() + hh, pr.get() + 2 * hh, tmp.get(), st, FR.get());
     }
     tick("block inversions D_h");
     if (!rc) {
-        wb_capacitance_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv, Mx);
+        wb_capacitance_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv.get(), Mx.get());
         h->launches++;
-        rc = gj_invert(h, Mx, qH, ipiv, info + H, pr + 2 * H, tmp, st, FR);
+        rc = gj_invert(h, Mx.get(), qH, ipiv.get(), info.get() + H, pr.get() + 2 * H, tmp.get(), st, FR.get());
     }
     tick("capacitance matrix M: build + invert");
     // W_NL = (D^-1 E) M^-1, one GEMM per harmonic block: rows of block h x the rows (k, h) of M^-1
     for (int hh = 0; hh < H && !rc; ++hh) {
-        const double2* blk = hh == 0 ? Dinv : Dinv + (size_t)q * q + (size_t)(hh - 1) * n * n;
+        const double2* blk = hh == 0 ? Dinv.get() : Dinv.get() + (size_t)q * q + (size_t)(hh - 1) * n * n;
         const int rows = hh == 0 ? q : n;
         const double2* Ablk = hh == 0 ? blk : blk + m;               // columns of the nonlinear buses
         const size_t z0 = hh == 0 ? 0 : (size_t)hh * n - m;
-        rc = launch_zgemm(h, rows, qH, q, Ablk, (size_t)rows, Mx + (size_t)hh * qH, (size_t)H * qH,
-                          h->d_WNL + z0 * qH, (size_t)qH, st);
+        rc = launch_zgemm(h, rows, qH, q, Ablk, (size_t)rows, Mx.get() + (size_t)hh * qH, (size_t)H * qH,
+                          WNL + z0 * qH, (size_t)qH, st);
     }
     // T = D_0^-1 Y_0[nl, lin];  U = YN E^T D^-1 A_ZF;  G = W_NL U + [T; 0]
-    if (!rc) rc = launch_zgemm(h, q, m, q, Dinv, (size_t)q, net.Y + (size_t)m * n, (size_t)n, T, (size_t)m, st);
+    if (!rc) rc = launch_zgemm(h, q, m, q, Dinv.get(), (size_t)q, net.Y + (size_t)m * n, (size_t)n, T.get(), (size_t)m, st);
     if (!rc) {
-        wb_coupling_rhs_kernel<<<h->sm_count * 4, 256, 0, st>>>(net, T, U);
+        wb_coupling_rhs_kernel<<<h->sm_count * 4, 256, 0, st>>>(net, T.get(), U.get());
         h->launches++;
-        rc = launch_zgemm(h, nZ, m, qH, h->d_WNL, (size_t)qH, U, (size_t)m, h->d_Gz, (size_t)m, st);
+        rc = launch_zgemm(h, nZ, m, qH, WNL, (size_t)qH, U.get(), (size_t)m, Gz, (size_t)m, st);
     }
     if (!rc) {
-        wb_finish_G_kernel<<<h->sm_count * 8, 256, 0, st>>>(nZ, m, q, T, h->d_Gz, h->d_GzT);
+        wb_finish_G_kernel<<<h->sm_count * 8, 256, 0, st>>>(nZ, m, q, T.get(), Gz, GzT);
         h->launches++;
     }
     tick("W_NL, G (tensor-core GEMMs)");
-    if (rc) { cleanup(); return rc; }
+    if (rc) return rc;
     std::vector<int> hinfo((size_t)H + 1);
     std::vector<double> hpr((size_t)2 * (H + 1));
-    WB(cudaMemcpyAsync(hinfo.data(), info, hinfo.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
-    WB(cudaMemcpyAsync(hpr.data(), pr, hpr.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
-    WB(cudaStreamSynchronize(st));
-#undef WB
-    cleanup();
-    tick("read-back + frees");
+    CK(cudaMemcpyAsync(hinfo.data(), info.get(), hinfo.size() * sizeof(int), cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(hpr.data(), pr.get(), hpr.size() * sizeof(double), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    tick("read-back");
     *info_out = 0;
     prh[0] = 1.0e308; prh[1] = 0.0;
     for (int t = 0; t <= H; ++t) {
@@ -1578,34 +1635,20 @@ static void build_hw_consts(hpf_t* h) {
 //   2  one scenario per CTA, state in shared memory (net1: 20 buses x 26 harmonics)
 //   3  one scenario per CTA, state in a global-memory slab, blocked tensor-core LU for the
 //      border system (200- / 1000-bus configurations)
-// frees the temporaries of a set-up on every exit path
-struct TmpFree {
-    std::vector<void*> p;
-    ~TmpFree() { for (void* x : p) cudaFree(x); }
-};
-
-static void free_struct_buffers(hpf_t* h) {
-    cudaFree(h->d_Ainv); cudaFree(h->d_Gz); cudaFree(h->d_GzT); cudaFree(h->d_WNL);
-    h->d_Ainv = nullptr; h->d_Gz = nullptr; h->d_GzT = nullptr; h->d_WNL = nullptr;
-}
-
 static int ensure_struct(hpf_t* h, cudaStream_t st) {
     if (h->struct_state != 0) return HPF_OK;
     h->struct_state = -1;
-    TmpFree guard;
     // allocation inside the set-up: out of device memory is not an error of the solve - the structured
     // buffers are released, the reason is left in hpf_last_error() and hpf_solve uses the dense strategy
-#define SK(ptr, bytes, temp)                                                                          \
+#define SK(ptr, bytes)                                                                                \
     do {                                                                                              \
-        cudaError_t e_ = cudaMalloc((void**)&(ptr), (bytes));                                         \
-        if (e_ == cudaErrorMemoryAllocation) {                                                        \
-            cudaGetLastError();                                                                       \
-            free_struct_buffers(h);                                                                   \
+        const int rc_ = dev_alloc(h, ptr, (bytes), "structured set-up: " #ptr);                        \
+        if (rc_ == HPF_E_NOMEM) {                                                                     \
+            h->d_struct = {};                                                                         \
             h->err = "structured set-up skipped (out of device memory for " #ptr "): dense strategy"; \
             return HPF_OK;                                                                            \
         }                                                                                             \
-        if (e_ != cudaSuccess) return fail(h, HPF_E_CUDA, std::string("structured setup: cudaMalloc " #ptr ": ") + cudaGetErrorString(e_)); \
-        if (temp) guard.p.push_back((void*)(ptr));                                                    \
+        if (rc_) return rc_;                                                                          \
     } while (0)
     const DevNet net = devnet(h);
     const int nZ = net.nH - net.m;
@@ -1629,13 +1672,8 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
         if (!fits_smem_lu(h, nf) && gmem_kernel_smem_bytes(nf.n, 1, nf.q, nf.N) > (size_t)h->smem_optin)
             return HPF_OK;                              // (n beyond ~2000 buses)
     }
-    double2* AZF = nullptr;
-    double2* tmp = nullptr;
-    int* ipiv = nullptr;
-    double* pr = nullptr;
-    free_struct_buffers(h);
-    cudaFree(h->d_nbr_ptr); cudaFree(h->d_nbr_idx);
-    h->d_nbr_ptr = nullptr; h->d_nbr_idx = nullptr;
+    StructBufs& sb = h->d_struct;
+    sb = {};
     const int qH = net.q * net.H;
     // nonlinear neighbours of the linear buses (structure of Y1), from the host mirror of Y
     {
@@ -1649,10 +1687,11 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
             }
             ptr[(size_t)i + 1] = (int)idx.size();
         }
-        CK(upload(&h->d_nbr_ptr, ptr.data(), ptr.size()));
-        CK(upload(&h->d_nbr_idx, idx.data(), idx.size()));
+        rc = upload(h, sb.nbr_ptr, ptr.data(), ptr.size(), "structured set-up: neighbour lists");
+        if (!rc) rc = upload(h, sb.nbr_idx, idx.data(), idx.size(), "structured set-up: neighbour lists");
+        if (rc) return rc;
         // sparsity pattern of Y(h), union over the harmonics (diagonal always listed)
-        cudaFree(h->d_ell_col); h->d_ell_col = nullptr; h->ell_w = 0;
+        h->d_ell_col.reset(); h->ell_w = 0;
         if (net.n >= 16) {
             const int n = net.n;
             std::vector<std::vector<int>> cols((size_t)n);
@@ -1672,14 +1711,15 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
                 std::vector<int> ell((size_t)n * w, -1);
                 for (int i = 0; i < n; ++i)
                     for (size_t e = 0; e < cols[(size_t)i].size(); ++e) ell[(size_t)i * w + e] = cols[(size_t)i][e];
-                CK(upload(&h->d_ell_col, ell.data(), ell.size()));
+                rc = upload(h, h->d_ell_col, ell.data(), ell.size(), "structured set-up: sparsity pattern of Y(h)");
+                if (rc) return rc;
                 h->ell_w = w;
             }
         }
     }
-    SK(h->d_WNL, ((size_t)nZ * qH + 1) * sizeof(double2), false);
-    SK(h->d_Gz, (size_t)nZ * net.m * sizeof(double2), false);
-    SK(h->d_GzT, (size_t)nZ * net.m * sizeof(double2), false);
+    SK(sb.WNL, ((size_t)nZ * qH + 1) * sizeof(double2));
+    SK(sb.Gz, (size_t)nZ * net.m * sizeof(double2));
+    SK(sb.GzT, (size_t)nZ * net.m * sizeof(double2));
     if (variant == 3 && qH > 0 && !h->setup_gj) {
         // large networks: the operator inverse through its block structure (Woodbury) - no nZ x nZ inverse
         int winfo = -1;
@@ -1691,42 +1731,45 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
         if (winfo == 0 && wpr[0] > 0.0 && wpr[1] / wpr[0] < 1e12) h->struct_state = variant;
         return HPF_OK;
     }
-    SK(h->d_Ainv, (size_t)nZ * nZ * sizeof(double2), false);
-    SK(AZF, (size_t)nZ * net.m * sizeof(double2), true);
-    SK(ipiv, (size_t)(nZ + 2) * sizeof(int), true);
-    SK(pr, 2 * sizeof(double), true);
-    struct_assemble_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, h->d_Ainv, AZF);
+    DevPtr<double2> AZF, tmp;         // temporaries of the set-up
+    DevPtr<int> ipiv;
+    DevPtr<double> pr;
+    SK(sb.Ainv, (size_t)nZ * nZ * sizeof(double2));
+    SK(AZF, (size_t)nZ * net.m * sizeof(double2));
+    SK(ipiv, (size_t)(nZ + 2) * sizeof(int));
+    SK(pr, 2 * sizeof(double));
+    struct_assemble_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, sb.Ainv.get(), AZF.get());
     h->launches++;
-    if (nZ > h->gj_single_max) SK(tmp, ((size_t)2 * nZ + 1) * sizeof(double2), true);
-    const int rcg = gj_invert(h, h->d_Ainv, nZ, ipiv, ipiv + nZ, pr, tmp, st);
+    if (nZ > h->gj_single_max) SK(tmp, ((size_t)2 * nZ + 1) * sizeof(double2));
+    const int rcg = gj_invert(h, sb.Ainv.get(), nZ, ipiv.get(), ipiv.get() + nZ, pr.get(), tmp.get(), st);
     if (rcg) return rcg;
     {
         const size_t tot = (size_t)nZ * net.m;
         struct_G_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(nZ, net.m, net.q < nZ ? net.q : nZ,
-                                                                       h->d_Ainv, AZF, h->d_Gz, h->d_GzT);
+                                                                       sb.Ainv.get(), AZF.get(), sb.Gz.get(), sb.GzT.get());
         h->launches++;
     }
     if (qH > 0) {
         const size_t tot = (size_t)nZ * qH;
-        struct_WNL_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(net, nZ, h->d_Ainv, h->d_WNL);
+        struct_WNL_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(net, nZ, sb.Ainv.get(), sb.WNL.get());
         h->launches++;
     }
     int info = -1;
     double prh[2] = {0.0, 0.0};
-    cudaError_t e = cudaMemcpyAsync(&info, ipiv + nZ, sizeof(int), cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(prh, pr, sizeof(prh), cudaMemcpyDeviceToHost, st);
+    cudaError_t e = cudaMemcpyAsync(&info, ipiv.get() + nZ, sizeof(int), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(prh, pr.get(), sizeof(prh), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
     h->hWNL.clear();
     h->hG.clear();
     h->hw_consts.clear();
     if (variant == 1 && e == cudaSuccess && qH > 0 && (size_t)nZ * qH <= 1024) {   // small operators: host mirror
         h->hWNL.resize((size_t)nZ * qH);
-        e = cudaMemcpy(h->hWNL.data(), h->d_WNL, h->hWNL.size() * sizeof(double2), cudaMemcpyDeviceToHost);
+        e = cudaMemcpy(h->hWNL.data(), sb.WNL.get(), h->hWNL.size() * sizeof(double2), cudaMemcpyDeviceToHost);
         h->hG.resize((size_t)nZ * net.m);
         if (e == cudaSuccess)
-            e = cudaMemcpy(h->hG.data(), h->d_Gz, h->hG.size() * sizeof(double2), cudaMemcpyDeviceToHost);
+            e = cudaMemcpy(h->hG.data(), sb.Gz.get(), h->hG.size() * sizeof(double2), cudaMemcpyDeviceToHost);
     }
-    if (variant == 3) { cudaFree(h->d_Ainv); h->d_Ainv = nullptr; }    // (GBs for the 1000-bus network)
+    if (variant == 3) sb.Ainv.reset();                                   // (GBs for the 1000-bus network)
     if (e != cudaSuccess) return fail(h, HPF_E_CUDA, std::string("structured setup: ") + cudaGetErrorString(e));
     h->pivot_min = prh[0]; h->pivot_max = prh[1];
     // usable when the inversion met no zero pivot and the pivots span < 1e12 (well conditioned)
@@ -1762,22 +1805,13 @@ static bool wn_use_dmma(const hpf_t* h, int nZ, int qH, int B) {
     return B >= ZG_BN && nZ >= ZG_BM && qH >= 64;
 }
 
-// Grow-only w_N scratch of at least `elems` entries
-static int ensure_wn(hpf_t* h, size_t elems) {
-    if (elems <= h->wN_elems) return HPF_OK;
-    if (h->d_wN) { CK(cudaDeviceSynchronize()); cudaFree(h->d_wN); h->d_wN = nullptr; h->wN_elems = 0; }
-    CK(cudaMalloc((void**)&h->d_wN, elems * sizeof(double2)));
-    h->wN_elems = elems;
-    return HPF_OK;
-}
-
 // w_N of a batch into the scratch at offset `off` of h->d_wN; *wN <- where it was written
 static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, const double2* I_N, size_t off,
                      const double2** wN, cudaStream_t st) {
-    int rc = ensure_wn(h, off + (size_t)sn.nZ * B);
+    int rc = grow(h, h->d_wN, (off + (size_t)sn.nZ * B) * sizeof(double2), "hpf_solve: w_N scratch");
     if (rc) return rc;
     WnArgs wa;
-    wa.B = B; wa.I_N = I_N; wa.wN = h->d_wN + off;
+    wa.B = B; wa.I_N = I_N; wa.wN = h->d_wN.get() + off;
     *wN = wa.wN;
     const int qH = net.q * net.H;
     if (qH == 0) { CK(cudaMemsetAsync(wa.wN, 0, (size_t)sn.nZ * B * sizeof(double2), st)); return HPF_OK; }
@@ -1882,12 +1916,9 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
         if (gst) {
             const size_t stride = (harm_cta_state_doubles(net.n, net.H, net.m, net.c, net.q, net.N, true) + 15) / 8 * 8;
             const size_t need = stride * (size_t)grid;
-            if (need > h->gstate_doubles) {
-                if (h->d_gstate) { CK(cudaDeviceSynchronize()); cudaFree(h->d_gstate); h->d_gstate = nullptr; h->gstate_doubles = 0; }
-                CK(cudaMalloc((void**)&h->d_gstate, need * sizeof(double)));
-                h->gstate_doubles = need;
-            }
-            ha2.gstate = h->d_gstate; ha2.gstate_stride = stride;
+            rc = grow(h, h->d_gstate, need * sizeof(double), "hpf_solve: scenario state slabs");
+            if (rc) return rc;
+            ha2.gstate = h->d_gstate.get(); ha2.gstate_stride = stride;
         }
         kernel<<<(unsigned)grid, threads, smem, st>>>(net, sn, ha2);
         h->launches++;
@@ -2067,29 +2098,22 @@ static int launch_ls_lu(hpf_t* h, const LsArgs& la, int cur, int N, int nwave, c
 }
 
 // Grow-only work area of the lock-step kernels: room for min(B, budget / per_slot) slots; -> slots
-static int ensure_ls(hpf_t* h, size_t per_slot, int B, int* slots) {
-    size_t have = h->ls_bytes > 4096 ? (h->ls_bytes - 4096) / per_slot : 0;
+static int ensure_ls(hpf_t* h, size_t per_slot, int B, int* slots, const char* who) {
+    size_t have = h->d_ls.bytes > 4096 ? (h->d_ls.bytes - 4096) / per_slot : 0;
     if (have < (size_t)B) {
         size_t budget = h->ls_budget;
         if (!budget) {
             size_t fr = 0, tot = 0;
             CK(cudaMemGetInfo(&fr, &tot));
-            budget = (size_t)(0.4 * (double)(fr + h->ls_bytes));
+            budget = (size_t)(0.4 * (double)(fr + h->d_ls.bytes));
             if (budget > ((size_t)64 << 30)) budget = (size_t)64 << 30;
         }
         size_t want = budget / per_slot;
         if (want > (size_t)B) want = (size_t)B;
         if (want < 1) want = 1;
         if (want > have) {
-            if (h->d_ls) { CK(cudaDeviceSynchronize()); cudaFree(h->d_ls); h->d_ls = nullptr; h->ls_bytes = 0; }
-            const size_t bytes = per_slot * want + 4096;
-            cudaError_t e = cudaMalloc(&h->d_ls, bytes);
-            if (e != cudaSuccess) {
-                cudaGetLastError();
-                return fail(h, e == cudaErrorMemoryAllocation ? HPF_E_NOMEM : HPF_E_CUDA,
-                            std::string("lock-step work areas: ") + cudaGetErrorString(e));
-            }
-            h->ls_bytes = bytes;
+            const int rc = grow(h, h->d_ls, per_slot * want + 4096, who);
+            if (rc) return rc;
             have = want;
         }
     }
@@ -2103,12 +2127,12 @@ static int lu_solve_batched(hpf_t* h, int N, int B, const double* J, size_t stri
     const size_t mat_stride = ls_mat_stride(N);
     const size_t per_slot = mat_stride * sizeof(double) + (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     int S = 0;
-    int rc = ensure_ls(h, per_slot, B, &S);
+    int rc = ensure_ls(h, per_slot, B, &S, "hpf_lu_solve: lock-step work areas");
     if (rc) return rc;
     LsArgs la;
     memset(&la, 0, sizeof(la));
     la.B = B; la.S = S; la.ldb = lub_ld(N); la.mat_stride = mat_stride;
-    char* p = reinterpret_cast<char*>(h->d_ls);
+    char* p = h->d_ls.get();
     la.M = reinterpret_cast<double*>(p); p += mat_stride * sizeof(double) * (size_t)S;
     ls_carve_ints(la, p, S);
     const long long nt = (N + 31) / 32;
@@ -2155,12 +2179,12 @@ static int launch_lockstep_fund(hpf_t* h, const SolveReq& r, cudaStream_t st) {
     const size_t state_stride = (scn_smem_doubles_aligned(nf.n, 1, nf.q, Nf) + 15) / 16 * 16;
     const size_t per_slot = (mat_stride + state_stride) * sizeof(double) + (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     int S = 0;
-    int rc = ensure_ls(h, per_slot, B, &S);
+    int rc = ensure_ls(h, per_slot, B, &S, "hpf_solve: lock-step work areas");
     if (rc) return rc;
     LsArgs la = ls_args(r, true, nullptr);
     la.S = S; la.ldb = lub_ld(Nf); la.mat_stride = mat_stride; la.state_stride = state_stride;
     {
-        char* p = reinterpret_cast<char*>(h->d_ls);
+        char* p = h->d_ls.get();
         la.M = reinterpret_cast<double*>(p);      p += mat_stride * sizeof(double) * (size_t)S;
         la.state = reinterpret_cast<double*>(p);  p += state_stride * sizeof(double) * (size_t)S;
         ls_carve_ints(la, p, S);
@@ -2207,15 +2231,13 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
     const size_t per_slot = (mat_stride + state_stride) * sizeof(double) + ((size_t)m + nZ + q) * sizeof(double2) +
                             (size_t)(LS_PERM_INTS + 8) * sizeof(int);
     // slots: the whole batch when it fits the memory budget, else waves
-    {
-        int rcs = ensure_ls(h, per_slot, r.B, &h->ls_slots);
-        if (rcs) return rcs;
-    }
-    const int S = h->ls_slots;
+    int S = 0;
+    int rc = ensure_ls(h, per_slot, r.B, &S, "hpf_solve: lock-step work areas");
+    if (rc) return rc;
     LsArgs la = ls_args(r, false, wN);
     la.S = S;
     {
-        char* p = reinterpret_cast<char*>(h->d_ls);
+        char* p = h->d_ls.get();
         la.M = reinterpret_cast<double*>(p);      p += mat_stride * sizeof(double) * (size_t)S;
         la.state = reinterpret_cast<double*>(p);  p += state_stride * sizeof(double) * (size_t)S;
         la.X = reinterpret_cast<double2*>(p);     p += (size_t)m * S * sizeof(double2);
@@ -2224,7 +2246,7 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
         ls_carve_ints(la, p, S);
     }
     la.mat_stride = mat_stride; la.state_stride = state_stride; la.ldb = lub_ld(nx);
-    int g_mis = 0, g_bor = 0, rc;
+    int g_mis = 0, g_bor = 0;
     rc = ls_grid(h, ls_mismatch_kernel, 256, 0, S, &g_mis);
     if (rc) return rc;
     const long long btiles = (long long)((m - 1 + 31) / 32) * ((nx + 1 + 31) / 32);
@@ -2287,7 +2309,7 @@ static HarmTileArgs harm_args(const hpf_t* h, const SolveReq& r, const double2* 
     ha.B = r.B; ha.flags = r.flags; ha.step_only = step ? 1 : 0; ha.P = r.P; ha.Q = r.Q; ha.I_N = r.I_N; ha.wN = wN;
     ha.thresh_h = r.thresh_h; ha.max_h = r.max_h; ha.V_m = r.out.V_m; ha.V_a = r.out.V_a; ha.I_inj = r.out.I_inj;
     ha.n_iter_h = r.out.n_iter_h; ha.status = r.out.status; ha.err_h = r.out.err_h; ha.hist_h = r.hist_h;
-    ha.work_counter = step ? nullptr : h->d_counter + r.slot;
+    ha.work_counter = step ? nullptr : h->d_counter.get() + r.slot;
     ha.dx_out = dx_out; ha.gstate = nullptr; ha.gstate_stride = 0; ha.lub_doubles = 0;
     ha.epoch = step ? 1 : HPF_HW_SERVICE_EPOCH;
     return ha;
@@ -2297,12 +2319,12 @@ static int solve_structured(hpf_t* h, const SolveReq& r, cudaStream_t st) {
     const DevNet net = devnet(h);
     const StructNet sn = structnet(h);
     const int B = r.B;
-    int* const counter = h->d_counter + r.slot;
+    int* const counter = h->d_counter.get() + r.slot;
     // error histories: the unused tail is NaN (all-ones bytes are a quiet NaN)
     if (r.hist_f) CK(cudaMemsetAsync(r.hist_f, 0xff, (size_t)(r.max_f + 1) * B * sizeof(double), st));
     if (r.hist_h) CK(cudaMemsetAsync(r.hist_h, 0xff, (size_t)(r.max_h + 1) * B * sizeof(double), st));
     CK(cudaMemsetAsync(counter, 0, sizeof(int), st));
-    if (h->profiling) { CK(cudaEventRecord(h->ev[0], st)); }
+    if (h->profiling) { CK(cudaEventRecord(h->ev[0].get(), st)); }
     // fundamental stage: one lane per scenario (variant 1) or the per-CTA kernel (variant 2)
     if (h->struct_state >= 2) {
         int rc = h->struct_state == 3 && use_lockstep(h, net.Nf, B) ? launch_lockstep_fund(h, r, st)
@@ -2331,7 +2353,7 @@ static int solve_structured(hpf_t* h, const SolveReq& r, cudaStream_t st) {
         h->launches++;
         CK(cudaGetLastError());
     }
-    if (h->profiling) { CK(cudaEventRecord(h->ev[1], st)); }
+    if (h->profiling) { CK(cudaEventRecord(h->ev[1].get(), st)); }
     // per-scenario constant w_N = A_ZZ^-1 I_N,Z, then the harmonic stage
     {
         const double2* wN = nullptr;
@@ -2342,7 +2364,7 @@ static int solve_structured(hpf_t* h, const SolveReq& r, cudaStream_t st) {
         if (rc) return rc;
         h->last_path = ls ? 4 : (h->struct_state >= 2 ? h->struct_state : 1);
     }
-    if (h->profiling) { CK(cudaEventRecord(h->ev[2], st)); h->ev_valid = 1; }
+    if (h->profiling) { CK(cudaEventRecord(h->ev[2].get(), st)); h->ev_valid = 1; }
     return HPF_OK;
 }
 
@@ -2356,9 +2378,9 @@ static int host_consts(hpf_t* h) {
     h->hY.resize(ny);
     h->hYN.resize(nyn);
     h->hdev.resize((size_t)h->q);
-    CK(cudaMemcpy(h->hY.data(), h->d_Y, ny * sizeof(double2), cudaMemcpyDeviceToHost));
-    if (nyn && h->have_dev) CK(cudaMemcpy(h->hYN.data(), h->d_YN, nyn * sizeof(double2), cudaMemcpyDeviceToHost));
-    if (h->q && h->have_dev) CK(cudaMemcpy(h->hdev.data(), h->d_devof, (size_t)h->q * sizeof(int), cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(h->hY.data(), h->d_Y.get(), ny * sizeof(double2), cudaMemcpyDeviceToHost));
+    if (nyn && h->have_dev) CK(cudaMemcpy(h->hYN.data(), h->d_YN.get(), nyn * sizeof(double2), cudaMemcpyDeviceToHost));
+    if (h->q && h->have_dev) CK(cudaMemcpy(h->hdev.data(), h->d_devof.get(), (size_t)h->q * sizeof(int), cudaMemcpyDeviceToHost));
     h->host_consts_valid = true;
     return HPF_OK;
 }
@@ -2425,12 +2447,12 @@ int hpf_create(hpf_t** out, int device) {
     if (const char* ev = getenv("HPF_MAX_CTAS")) h->max_ctas = atoi(ev) > 0 ? atoi(ev) : 0;
     h->sm_count = prop.multiProcessorCount;
     h->smem_optin = (int)prop.sharedMemPerBlockOptin;
-    e = cudaMalloc((void**)&h->d_counter, HPF_HOST_MAX_CHUNKS * sizeof(int));
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&h->ev_last, cudaEventDisableTiming);
-    if (e != cudaSuccess) {
-        cudaFree(h->d_counter);
+    int rc = dev_alloc(nullptr, h->d_counter, HPF_HOST_MAX_CHUNKS * sizeof(int), "hpf_create: work counters");
+    if (!rc && (e = create_event(h->ev_last, cudaEventDisableTiming)) != cudaSuccess)
+        rc = fail(nullptr, HPF_E_CUDA, std::string("hpf_create: ") + cudaGetErrorString(e));
+    if (rc) {
         delete h;
-        return fail(nullptr, HPF_E_CUDA, std::string("hpf_create: ") + cudaGetErrorString(e));
+        return rc;
     }
     *out = h;
     return HPF_OK;
@@ -2440,16 +2462,7 @@ int hpf_destroy(hpf_t* h) {
     if (!h) return HPF_OK;
     DeviceGuard dg_(h->device);
     cudaDeviceSynchronize();
-    if (h->ev_last) cudaEventDestroy(h->ev_last);
-    cudaFree(h->d_harm); cudaFree(h->d_from); cudaFree(h->d_to); cudaFree(h->d_devof);
-    cudaFree(h->d_R); cudaFree(h->d_X); cudaFree(h->d_G); cudaFree(h->d_B); cudaFree(h->d_Xsh);
-    cudaFree(h->d_Y); cudaFree(h->d_YN); cudaFree(h->d_counter); cudaFree(h->d_work); cudaFree(h->d_io); cudaFree(h->d_Ainv); cudaFree(h->d_Gz);
-    cudaFree(h->d_WNL); cudaFree(h->d_wN); cudaFree(h->d_GzT); cudaFree(h->d_nbr_ptr); cudaFree(h->d_nbr_idx);
-    cudaFree(h->d_gstate); cudaFree(h->d_ls); cudaFree(h->d_ell_col); cudaFree(h->d_tau); cudaFree(h->d_phase);
-    for (int i = 0; i < 3; ++i) if (h->ev[i]) cudaEventDestroy(h->ev[i]);
-    for (int i = 0; i < 6; ++i) if (h->st_io[i]) cudaStreamDestroy(h->st_io[i]);
-    for (int i = 0; i < 2 * HPF_HOST_MAX_CHUNKS; ++i) if (h->ev_io[i]) cudaEventDestroy(h->ev_io[i]);
-    delete h;
+    delete h;                     // the members release their memory, streams and events on the handle's device
     return HPF_OK;
 }
 
@@ -2466,6 +2479,20 @@ int hpf_set_network(hpf_t* h, int n, int m, int c, int H, const int* harmonics, 
         if (from_id[l] < 1 || from_id[l] > n || to_id[l] < 1 || to_id[l] > n)
             return fail(h, HPF_E_INVALID, "hpf_set_network: line endpoint outside 1..n");
     ENTER_DEVICE(h);
+    // the previous network goes first: after a failed upload the handle has no network
+    h->have_net = h->have_Y = h->have_dev = false;
+    invalidate_derived(h, true);
+    h->d_tau.reset(); h->d_phase.reset();
+    int rc = upload(h, h->d_harm, harmonics, (size_t)H, "hpf_set_network: harmonics");
+    if (!rc) rc = upload(h, h->d_from, from_id, (size_t)L, "hpf_set_network: from_id");
+    if (!rc) rc = upload(h, h->d_to, to_id, (size_t)L, "hpf_set_network: to_id");
+    if (!rc) rc = upload(h, h->d_R, R, (size_t)L, "hpf_set_network: R");
+    if (!rc) rc = upload(h, h->d_X, X, (size_t)L, "hpf_set_network: X");
+    if (!rc) rc = upload(h, h->d_G, G, (size_t)L, "hpf_set_network: G");
+    if (!rc) rc = upload(h, h->d_B, B, (size_t)L, "hpf_set_network: B");
+    if (!rc) rc = upload(h, h->d_Xsh, X_sh, (size_t)n, "hpf_set_network: X_sh");
+    if (!rc) rc = upload(h, h->d_Y, (const double2*)nullptr, (size_t)H * n * n, "hpf_set_network: Y(h)");
+    if (rc) return rc;
     h->n = n; h->m = m; h->c = c; h->H = H; h->q = n - m; h->L = L;
     h->shape = h->fund_shape = 0;
     for (int s = 1; s <= HPF_SHAPES && !h->no_specialise; ++s)
@@ -2475,22 +2502,7 @@ int hpf_set_network(hpf_t* h, int n, int m, int c, int H, const int* harmonics, 
             if (n == D::n && c == D::c && !h->fund_shape) h->fund_shape = s;
             return 0;
         });
-    CK(upload(&h->d_harm, harmonics, (size_t)H));
-    CK(upload(&h->d_from, from_id, (size_t)L));
-    CK(upload(&h->d_to, to_id, (size_t)L));
-    CK(upload(&h->d_R, R, (size_t)L));
-    CK(upload(&h->d_X, X, (size_t)L));
-    CK(upload(&h->d_G, G, (size_t)L));
-    CK(upload(&h->d_B, B, (size_t)L));
-    CK(upload(&h->d_Xsh, X_sh, (size_t)n));
-    cudaFree(h->d_tau); cudaFree(h->d_phase); h->d_tau = nullptr; h->d_phase = nullptr;
-    CK(upload(&h->d_Y, (const double2*)nullptr, (size_t)H * n * n));
     h->have_net = true;
-    h->have_Y = false;
-    h->have_dev = false;
-    h->struct_state = 0;
-    h->host_consts_valid = false;
-    cudaFree(h->d_ell_col); h->d_ell_col = nullptr; h->ell_w = 0;
     return HPF_OK;
 }
 
@@ -2503,14 +2515,15 @@ int hpf_set_devices(hpf_t* h, int n_dev, int coupled, const double* Y_N, const i
         if (dev_of_nl_bus[k] < 0 || dev_of_nl_bus[k] >= n_dev)
             return fail(h, HPF_E_INVALID, "hpf_set_devices: dev_of_nl_bus entry outside 0..n_dev-1");
     ENTER_DEVICE(h);
+    h->have_dev = false;                                     // after a failed upload: no devices
+    invalidate_derived(h, false);
+    const size_t per = coupled ? (size_t)h->H * h->H : (size_t)h->H;
+    int rc = upload(h, h->d_YN, (const double2*)Y_N, per * (size_t)(n_dev > 0 ? n_dev : 0), "hpf_set_devices: Y_N");
+    if (!rc) rc = upload(h, h->d_devof, dev_of_nl_bus, (size_t)h->q, "hpf_set_devices: dev_of_nl_bus");
+    if (rc) return rc;
     h->n_dev = n_dev;
     h->coupled = coupled ? 1 : 0;
-    const size_t per = coupled ? (size_t)h->H * h->H : (size_t)h->H;
-    CK(upload(&h->d_YN, (const double2*)Y_N, per * (size_t)(n_dev > 0 ? n_dev : 0)));
-    CK(upload(&h->d_devof, dev_of_nl_bus, (size_t)h->q));
     h->have_dev = true;
-    h->struct_state = 0;
-    h->host_consts_valid = false;
     return HPF_OK;
 }
 
@@ -2519,17 +2532,17 @@ int hpf_set_transformers(hpf_t* h, const double* tau, const double* phase_shift_
     if (!h->have_net) return fail(h, HPF_E_INVALID, "hpf_set_transformers: call hpf_set_network first");
     if ((tau == nullptr) != (phase_shift_deg == nullptr))
         return fail(h, HPF_E_INVALID, "hpf_set_transformers: give both arrays or neither");
+    for (int l = 0; tau && l < h->L; ++l)
+        if (!(tau[l] != 0.0)) return fail(h, HPF_E_INVALID, "hpf_set_transformers: tau must be non-zero");
     ENTER_DEVICE(h);
-    cudaFree(h->d_tau); cudaFree(h->d_phase); h->d_tau = nullptr; h->d_phase = nullptr;
-    if (tau) {
-        for (int l = 0; l < h->L; ++l)
-            if (!(tau[l] != 0.0)) return fail(h, HPF_E_INVALID, "hpf_set_transformers: tau must be non-zero");
-        CK(upload(&h->d_tau, tau, (size_t)h->L));
-        CK(upload(&h->d_phase, phase_shift_deg, (size_t)h->L));
-    }
     h->have_Y = false;                                       // Y(h) must be rebuilt
-    h->struct_state = 0;
-    h->host_consts_valid = false;
+    invalidate_derived(h, false);
+    h->d_tau.reset(); h->d_phase.reset();
+    if (tau) {
+        int rc = upload(h, h->d_tau, tau, (size_t)h->L, "hpf_set_transformers: tau");
+        if (!rc) rc = upload(h, h->d_phase, phase_shift_deg, (size_t)h->L, "hpf_set_transformers: phase_shift_deg");
+        if (rc) { h->d_tau.reset(); return rc; }             // Y(h) reads both or neither
+    }
     return HPF_OK;
 }
 
@@ -2539,8 +2552,7 @@ int hpf_set_y_options(hpf_t* h, int flags) {
         return fail(h, HPF_E_INVALID, "hpf_set_y_options: unknown flag");
     h->y_flags = flags;
     h->have_Y = false;                                       // Y(h) must be rebuilt
-    h->struct_state = 0;
-    h->host_consts_valid = false;
+    invalidate_derived(h, false);
     return HPF_OK;
 }
 
@@ -2550,17 +2562,16 @@ static int build_Y_impl(hpf_t* h, double* Y_out, void* stream) {
     ENTER_DEVICE(h);
     cudaStream_t st = (cudaStream_t)stream;
     const int total = h->n * h->H;
-    ybus_kernel<<<(total + 127) / 128, 128, 0, st>>>(h->n, h->H, h->L, h->d_harm, h->d_from, h->d_to,
-                                                      h->d_R, h->d_X, h->d_G, h->d_B, h->d_Xsh, h->d_tau, h->d_phase, h->y_flags, h->d_Y);
+    ybus_kernel<<<(total + 127) / 128, 128, 0, st>>>(h->n, h->H, h->L, h->d_harm.get(), h->d_from.get(), h->d_to.get(),
+                                                      h->d_R.get(), h->d_X.get(), h->d_G.get(), h->d_B.get(), h->d_Xsh.get(),
+                                                      h->d_tau.get(), h->d_phase.get(), h->y_flags, h->d_Y.get());
     h->launches++;
     CK(cudaGetLastError());
     if (Y_out)
-        CK(cudaMemcpyAsync(Y_out, h->d_Y, (size_t)h->H * h->n * h->n * sizeof(double2),
+        CK(cudaMemcpyAsync(Y_out, h->d_Y.get(), (size_t)h->H * h->n * h->n * sizeof(double2),
                            cudaMemcpyDeviceToDevice, st));
     h->have_Y = true;
-    h->struct_state = 0;
-    h->host_consts_valid = false;
-    cudaFree(h->d_ell_col); h->d_ell_col = nullptr; h->ell_w = 0;
+    invalidate_derived(h, true);
     return HPF_OK;
 }
 
@@ -2573,11 +2584,9 @@ int hpf_set_Y(hpf_t* h, const double* Y) {
     if (!h->have_net) return fail(h, HPF_E_INVALID, "hpf_set_Y: call hpf_set_network first");
     if (!Y) return fail(h, HPF_E_INVALID, "hpf_set_Y: Y is NULL");
     ENTER_DEVICE(h);
-    CK(cudaMemcpy(h->d_Y, Y, (size_t)h->H * h->n * h->n * sizeof(double2), cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(h->d_Y.get(), Y, (size_t)h->H * h->n * h->n * sizeof(double2), cudaMemcpyHostToDevice));
     h->have_Y = true;
-    h->struct_state = 0;
-    h->host_consts_valid = false;
-    cudaFree(h->d_ell_col); h->d_ell_col = nullptr; h->ell_w = 0;
+    invalidate_derived(h, true);
     return HPF_OK;
 }
 
@@ -2588,7 +2597,7 @@ int hpf_thd(hpf_t* h, int B, const double* V_m, double* thd, void* stream) {
     if (!V_m || !thd) return fail(h, HPF_E_INVALID, "hpf_thd: NULL buffer");
     ENTER_DEVICE(h);
     const size_t total = (size_t)h->n * B;
-    thd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->n, h->H, h->d_harm, B,
+    thd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->n, h->H, h->d_harm.get(), B,
                                                                                     V_m, thd);
     h->launches++;
     CK(cudaGetLastError());
@@ -2615,7 +2624,7 @@ int hpf_set_profiling(hpf_t* h, int enabled) {
     ENTER_DEVICE(h);
     if (enabled)
         for (int i = 0; i < 3; ++i)
-            if (!h->ev[i]) CK(cudaEventCreate(&h->ev[i]));
+            if (!h->ev[i]) CK(create_event(h->ev[i], cudaEventDefault));
     h->profiling = enabled ? 1 : 0;
     h->ev_valid = 0;
     return HPF_OK;
@@ -2624,10 +2633,10 @@ int hpf_set_profiling(hpf_t* h, int enabled) {
 int hpf_last_kernel_ms(hpf_t* h, double* ms) {
     if (!h || !ms) return HPF_E_INVALID;
     if (!h->profiling || !h->ev_valid) return fail(h, HPF_E_INVALID, "hpf_last_kernel_ms: no profiled solve");
-    CK(cudaEventSynchronize(h->ev[2]));
+    CK(cudaEventSynchronize(h->ev[2].get()));
     float a = 0.f, b = 0.f;
-    if (h->ev_valid == 1) CK(cudaEventElapsedTime(&a, h->ev[0], h->ev[1]));
-    CK(cudaEventElapsedTime(&b, h->ev[1], h->ev[2]));
+    if (h->ev_valid == 1) CK(cudaEventElapsedTime(&a, h->ev[0].get(), h->ev[1].get()));
+    CK(cudaEventElapsedTime(&b, h->ev[1].get(), h->ev[2].get()));
     ms[0] = a; ms[1] = b;
     return HPF_OK;
 }
@@ -2689,12 +2698,11 @@ int hpf_prepare(hpf_t* h, int B_max, void* stream) {
     // the allocation paths of hpf_solve: structured set-up, w_N scratch, LU workspaces, state slabs
     const size_t B = (size_t)B_max, n = h->n, H = h->H, q = h->q;
     const size_t nd = 2 * n * B + 2 * q * H * B + 2 * n * H * B + 2 * q * H * B + B + 2 * B + 8;
-    double* buf = nullptr;
-    cudaError_t e = cudaMalloc((void**)&buf, nd * sizeof(double));
-    if (e != cudaSuccess) return fail(h, e == cudaErrorMemoryAllocation ? HPF_E_NOMEM : HPF_E_CUDA,
-                                      std::string("hpf_prepare: ") + cudaGetErrorString(e));
-    e = cudaMemsetAsync(buf, 0, nd * sizeof(double), st);
-    double *P = buf, *Q = P + n * B, *IN = Q + n * B, *Vm = IN + 2 * q * H * B, *Va = Vm + n * H * B,
+    DevPtr<double> buf;
+    rc = dev_alloc(h, buf, nd * sizeof(double), "hpf_prepare: scenario buffers");
+    if (rc) return rc;
+    const cudaError_t e = cudaMemsetAsync(buf.get(), 0, nd * sizeof(double), st);
+    double *P = buf.get(), *Q = P + n * B, *IN = Q + n * B, *Vm = IN + 2 * q * H * B, *Va = Vm + n * H * B,
            *Inj = Va + n * H * B, *err = Inj + 2 * q * H * B;
     int* iw = reinterpret_cast<int*>(err + B);
     SolveReq r;
@@ -2704,7 +2712,6 @@ int hpf_prepare(hpf_t* h, int B_max, void* stream) {
     r.out.n_iter_f = iw; r.out.n_iter_h = iw + B; r.out.err_h = err; r.out.status = iw + 2 * B;
     if (e == cudaSuccess) rc = ordered(h, stream, [&] { return solve_dispatch(h, r, st); });
     const cudaError_t e2 = cudaStreamSynchronize(st);
-    cudaFree(buf);
     if (rc) return rc;
     if (e != cudaSuccess || e2 != cudaSuccess)
         return fail(h, HPF_E_CUDA, std::string("hpf_prepare: ") + cudaGetErrorString(e != cudaSuccess ? e : e2));
@@ -2877,29 +2884,35 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
     const size_t per_scn = 2 * n + 2 * q * H + 2 * n * H + 2 * q * H;
     const size_t Bp = (Bs + 3) / 4 * 4;
     const size_t nd = per_scn * Bs + Bp + 3 * (Bp / 2);
-    if (nd > h->io_doubles) {
-        if (h->d_io) { CK(cudaDeviceSynchronize()); cudaFree(h->d_io); h->d_io = nullptr; h->io_doubles = 0; }
-        CK(cudaMalloc((void**)&h->d_io, nd * sizeof(double)));
-        h->io_doubles = nd;
-    }
+    rc = grow(h, h->d_io, nd * sizeof(double), "hpf_solve_host: staging buffers");
+    if (rc) return rc;
     if (!h->st_io[0]) {
-        for (int i = 0; i < 6; ++i) CK(cudaStreamCreateWithFlags(&h->st_io[i], cudaStreamNonBlocking));
-        for (int i = 0; i < 2 * HPF_HOST_MAX_CHUNKS; ++i) CK(cudaEventCreateWithFlags(&h->ev_io[i], cudaEventDisableTiming));
+        // all or nothing: the handle takes the streams and events only when every one of them exists
+        Stream st[6];
+        Event ev[2 * HPF_HOST_MAX_CHUNKS];
+        for (auto& s : st) {
+            cudaStream_t raw = nullptr;
+            CK(cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking));
+            s.reset(raw);
+        }
+        for (auto& e : ev) CK(create_event(e, cudaEventDisableTiming));
+        for (int i = 0; i < 6; ++i) h->st_io[i] = std::move(st[i]);
+        for (int i = 0; i < 2 * HPF_HOST_MAX_CHUNKS; ++i) h->ev_io[i] = std::move(ev[i]);
     }
-    cudaStream_t s_in = h->st_io[0], s_out = h->st_io[2];
+    cudaStream_t s_in = h->st_io[0].get(), s_out = h->st_io[2].get();
     const int cmp_stream[4] = {1, 3, 4, 5};
     // ordered after the handle's previous kernel sequence like every other entry point (the copy-in
     // overwrites the staging buffers, the solves share the handle's scratch)
     if (h->last_valid)
-        for (int i = 0; i < 6; ++i) CK(cudaStreamWaitEvent(h->st_io[i], h->ev_last, 0));
+        for (auto& s : h->st_io) CK(cudaStreamWaitEvent(s.get(), h->ev_last.get(), 0));
     // several compute streams only where concurrent solves share no scratch (tile variant)
-    rc = ensure_struct(h, h->st_io[1]);
+    rc = ensure_struct(h, h->st_io[1].get());
     if (rc) return rc;
     const bool dual = (h->struct_state == 1) && nchunk > 1 && ncs > 1;
     const size_t wN_rows = (size_t)(h->n * h->H - h->m);
     if (dual) {
         // reserve the w_N scratch of all chunks up front (no reallocation while chunks are in flight)
-        rc = ensure_wn(h, wN_rows * Bs);
+        rc = grow(h, h->d_wN, wN_rows * Bs * sizeof(double2), "hpf_solve_host: w_N scratch");
         if (rc) return rc;
     }
     auto cp2d = [&](void* dst, size_t dpitch, const void* src, size_t spitch, size_t width, size_t rows,
@@ -2908,19 +2921,19 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
     };
     rc = HPF_OK;
     cudaError_t e = cudaSuccess;
-    double* const dErr_all = h->d_io + per_scn * Bs;
+    double* const dErr_all = h->d_io.get() + per_scn * Bs;
     int* const di_all = reinterpret_cast<int*>(dErr_all + Bp);
     // $HPF_HOST_TIMELINE: per-chunk completion times of copy-in, solve and copy-out on stderr
     const bool tl = getenv("HPF_HOST_TIMELINE") != nullptr;
-    cudaEvent_t tle[3 * HPF_HOST_MAX_CHUNKS + 1] = {};
+    Event tle[3 * HPF_HOST_MAX_CHUNKS + 1];
     if (tl) {
-        for (auto& ev : tle) cudaEventCreate(&ev);
-        cudaEventRecord(tle[3 * HPF_HOST_MAX_CHUNKS], s_in);
+        for (auto& ev : tle) create_event(ev, cudaEventDefault);
+        cudaEventRecord(tle[3 * HPF_HOST_MAX_CHUNKS].get(), s_in);
     }
     const BatchOut& ho = hr.out;
     for (int k = 0; k < nchunk && !rc; ++k) {
         const size_t b0 = cb[k], Bc = cb[k + 1] - cb[k];
-        double* d = h->d_io + per_scn * b0;
+        double* d = h->d_io.get() + per_scn * b0;
         double *dP = d, *dQ = dP + n * Bc, *dI = dQ + n * Bc, *dVm = dI + 2 * q * H * Bc, *dVa = dVm + n * H * Bc,
                *dInj = dVa + n * H * Bc, *dErr = dErr_all + b0;
         int *di_f = di_all + b0, *di_h = di_all + Bp + b0, *di_s = di_all + 2 * Bp + b0;
@@ -2930,11 +2943,11 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
         if (e == cudaSuccess) e = cp2d(dQ, w8, hr.Q + b0, p8, w8, n, cudaMemcpyHostToDevice, s_in);
         if (e == cudaSuccess && q)
             e = cp2d(dI, w16, hr.I_N + b0, p16, w16, q * H, cudaMemcpyHostToDevice, s_in);
-        cudaStream_t s_cmp = h->st_io[dual ? cmp_stream[k % ncs] : 1];
-        if (e == cudaSuccess) e = cudaEventRecord(h->ev_io[k], s_in);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(s_cmp, h->ev_io[k], 0);
+        cudaStream_t s_cmp = h->st_io[dual ? cmp_stream[k % ncs] : 1].get();
+        if (e == cudaSuccess) e = cudaEventRecord(h->ev_io[k].get(), s_in);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(s_cmp, h->ev_io[k].get(), 0);
         if (e != cudaSuccess) break;
-        if (tl) cudaEventRecord(tle[3 * k], s_in);
+        if (tl) cudaEventRecord(tle[3 * k].get(), s_in);
         SolveReq c = hr;          // the same thresholds and limits on the chunk's device buffers
         c.B = (int)Bc; c.P = dP; c.Q = dQ; c.I_N = (const double2*)dI;
         c.out.V_m = dVm; c.out.V_a = dVa; c.out.I_inj = ho.I_inj ? (double2*)dInj : nullptr;
@@ -2943,9 +2956,9 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
         c.wN_off = dual ? wN_rows * b0 : 0;
         rc = solve_dispatch(h, c, s_cmp);
         if (rc) break;
-        e = cudaEventRecord(h->ev_io[HPF_HOST_MAX_CHUNKS + k], s_cmp);
-        if (tl) cudaEventRecord(tle[3 * k + 1], s_cmp);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(s_out, h->ev_io[HPF_HOST_MAX_CHUNKS + k], 0);
+        e = cudaEventRecord(h->ev_io[HPF_HOST_MAX_CHUNKS + k].get(), s_cmp);
+        if (tl) cudaEventRecord(tle[3 * k + 1].get(), s_cmp);
+        if (e == cudaSuccess) e = cudaStreamWaitEvent(s_out, h->ev_io[HPF_HOST_MAX_CHUNKS + k].get(), 0);
         if (e == cudaSuccess) e = cp2d(ho.V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
         if (e == cudaSuccess) e = cp2d(ho.V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
         if (e == cudaSuccess && ho.I_inj && q)
@@ -2956,7 +2969,7 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
             if (e == cudaSuccess) e = cudaMemcpyAsync(ho.n_iter_h, di_all + Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
             if (e == cudaSuccess) e = cudaMemcpyAsync(ho.status, di_all + 2 * Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
         }
-        if (tl) cudaEventRecord(tle[3 * k + 2], s_out);
+        if (tl) cudaEventRecord(tle[3 * k + 2].get(), s_out);
         if (e == cudaSuccess && keep) {
             // also leave the results on the device in the full [rows, B] layout (device-to-device
             // 2-D copies on the compute stream, ~20 us for the whole batch)
@@ -2972,18 +2985,17 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
         if (e != cudaSuccess) break;
     }
     if (!rc && e != cudaSuccess) rc = fail(h, HPF_E_CUDA, std::string("hpf_solve_host: ") + cudaGetErrorString(e));
-    for (int i = 0; i < 6; ++i) {
-        const cudaError_t e2 = cudaStreamSynchronize(h->st_io[i]);
+    for (auto& s : h->st_io) {
+        const cudaError_t e2 = cudaStreamSynchronize(s.get());
         if (!rc && e2 != cudaSuccess) rc = fail(h, HPF_E_CUDA, std::string("hpf_solve_host: ") + cudaGetErrorString(e2));
     }
     if (tl) {
         for (int k = 0; k < nchunk && !rc; ++k) {
             float t[3] = {0.f, 0.f, 0.f};
-            for (int i = 0; i < 3; ++i) cudaEventElapsedTime(&t[i], tle[3 * HPF_HOST_MAX_CHUNKS], tle[3 * k + i]);
+            for (int i = 0; i < 3; ++i) cudaEventElapsedTime(&t[i], tle[3 * HPF_HOST_MAX_CHUNKS].get(), tle[3 * k + i].get());
             fprintf(stderr, "hpf_solve_host chunk %2d [%6zu..%6zu): copy-in done %.3f ms, solve done %.3f ms, copy-out done %.3f ms\n",
                     k, cb[k], cb[k + 1], t[0], t[1], t[2]);
         }
-        for (auto& ev : tle) cudaEventDestroy(ev);
     }
     if (!rc) h->last_valid = false;        // everything this handle issued has completed
     return rc;
@@ -3129,9 +3141,9 @@ static int lu_solve_impl(hpf_t* h, int B, const double* J, const double* f, doub
     if (grid > B) grid = B;
     a.workspace = nullptr;
     if (lu.kind) {
-        rc = ensure_workspace(h, (size_t)grid * lub_ld(net.N) * (net.N + 1));
+        rc = grow(h, h->d_work, (size_t)grid * lub_ld(net.N) * (net.N + 1) * sizeof(double), "hpf_lu_solve: LU workspace");
         if (rc) return rc;
-        a.workspace = h->d_work;
+        a.workspace = h->d_work.get();
     }
     kernel<<<(unsigned)grid, threads, lu.smem, (cudaStream_t)stream>>>(net, a);
     h->launches++;

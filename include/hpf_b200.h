@@ -58,7 +58,7 @@ typedef struct hpf_handle hpf_t;
 #define HPF_E_INVALID      -1   /* bad argument / call order                      */
 #define HPF_E_CUDA         -2   /* CUDA runtime error (text in hpf_last_error)    */
 #define HPF_E_UNSUPPORTED  -3   /* dimensions exceed what the kernels support     */
-#define HPF_E_NOMEM        -4
+#define HPF_E_NOMEM        -4   /* out of device memory: the text names the call and the buffer; other CUDA errors stay HPF_E_CUDA */
 
 /* per-scenario status word (status[B]) */
 #define HPF_ST_CONVERGED    0

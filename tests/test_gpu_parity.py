@@ -611,6 +611,54 @@ def test_invalid_arguments_are_refused_loudly(solvers):
     refused(lib.hpf_solve_host(h, -1, None, None, None, 1e-6, 30, 1e-4, 50, *[None] * 7), "hpf_solve_host: B < 0")
 
 
+def test_failed_allocation_leaves_handle_usable(tmp_path):
+    """A device allocation that cudaMalloc refuses is reported as HPF_E_NOMEM by the call that made
+    it and by no later call; a network that could not be uploaded leaves the handle with no network,
+    not with a mix of the old and the new one.  Own handle: this test leaves it in error states."""
+    from harmonic_power_flow_b200 import BatchSolver, _lib
+    from harmonic_power_flow_b200.solver import _np_d, _np_i
+    d = helpers.load_case("net3_c_h25")
+    net, _, _ = helpers.packed_from_files(str(d["net"]), int(d["h_max"]), bool(d["coupled"]), tmp_path)
+    sol = BatchSolver(net)
+    lib, h = sol.lib, sol._h
+
+    def solve_nominal():
+        r = sol.solve(net.P[:, None], net.Q[:, None], net.I_N[:, :, None])
+        assert int(r.n_iter_f.item()) == int(d["n_iter_f"])
+        assert int(r.n_iter_h.item()) == int(d["n_iter_h"])
+        assert int(r.status.item()) == 0
+        V = helpers.phasor(r.V_m[:, :, 0].cpu().numpy(), r.V_a[:, :, 0].cpu().numpy())
+        Vg = helpers.phasor(d["V_m"], d["V_a"])
+        tol = 1e-9 if float(d["err_h"]) < 1e-6 else 1e-7
+        assert (np.abs(V - Vg) / np.abs(Vg)).max() < tol
+
+    try:
+        # 1. a failed hpf_prepare (terabytes of scenario buffers), then a solve
+        with pytest.raises(_lib.HpfError) as e:
+            sol.prepare_batch(2 ** 31 - 1)
+        assert e.value.code == _lib.HPF_E_NOMEM and "hpf_prepare" in str(e.value), str(e.value)
+        solve_nominal()
+        # 2. a failed hpf_set_network (Y(h) of 200,000 buses: 640 GB), then a clean set-up
+        n = 200000
+        rc = lib.hpf_set_network(h, n, n, 1, 1, _np_i(np.ones(1, np.int32)), 0, None, None, None, None, None, None,
+                                 _np_d(np.zeros(n)))
+        assert rc == _lib.HPF_E_NOMEM, lib.hpf_last_error(h)
+        assert lib.hpf_dim_N(h) == 0
+        with pytest.raises(_lib.HpfError) as e:
+            _lib.check(h, lib.hpf_solve(h, 1, None, None, None, 1e-6, 30, 1e-4, 50, 0, *[None] * 10))
+        assert e.value.code == _lib.HPF_E_INVALID and "hpf_set_network" in str(e.value), str(e.value)
+        _lib.check(h, lib.hpf_set_network(h, net.n, net.m, net.c, net.H, _np_i(net.harmonics), len(net.R),
+                                          _np_i(net.from_id), _np_i(net.to_id), _np_d(net.R), _np_d(net.X),
+                                          _np_d(net.G), _np_d(net.B), _np_d(net.X_sh)))
+        _lib.check(h, lib.hpf_set_devices(h, len(net.devices), int(net.coupled),
+                                          _np_d(np.ascontiguousarray(net.Y_N).view(np.float64)),
+                                          _np_i(net.dev_of_nl_bus)))
+        sol.build_Y()
+        solve_nominal()
+    finally:
+        sol.close()
+
+
 # ---------------------------------------------------------------- drop-in API
 def test_reference_shaped_api(tmp_path):
     from harmonic_power_flow_b200 import hcne_generalized as hg
