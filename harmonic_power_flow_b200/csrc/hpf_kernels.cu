@@ -2579,11 +2579,14 @@ int hpf_build_Y(hpf_t* h, double* Y_out, void* stream) {
     return ordered(h, stream, [&] { return build_Y_impl(h, Y_out, stream); });
 }
 
+// The copy runs on the legacy stream, which does not wait for non-blocking streams: without the
+// wait on ev_last, a solve still in flight on such a stream could read the new Y(h) partway through.
 int hpf_set_Y(hpf_t* h, const double* Y) {
     if (!h) return HPF_E_INVALID;
     if (!h->have_net) return fail(h, HPF_E_INVALID, "hpf_set_Y: call hpf_set_network first");
     if (!Y) return fail(h, HPF_E_INVALID, "hpf_set_Y: Y is NULL");
     ENTER_DEVICE(h);
+    if (h->last_valid) CK(cudaEventSynchronize(h->ev_last.get()));
     CK(cudaMemcpy(h->d_Y.get(), Y, (size_t)h->H * h->n * h->n * sizeof(double2), cudaMemcpyHostToDevice));
     h->have_Y = true;
     invalidate_derived(h, true);

@@ -127,7 +127,9 @@ int hpf_build_Y(hpf_t* h, double* Y_out, void* stream);
 
 /*
  * Use a caller-supplied admittance table instead of building it: Y complex [H, n, n]
- * (host).  This is what pf(Y, buses) of the reference takes (HG:244,255).
+ * (host).  This is what pf(Y, buses) of the reference takes (HG:244,255).  The host waits
+ * for the handle's previous kernel sequence before it copies, so a solve still in flight on
+ * any stream finishes on the table it was issued with.
  */
 int hpf_set_Y(hpf_t* h, const double* Y);
 

@@ -69,6 +69,26 @@ def oracle_net(net):
                  I_N=net.I_N, Y_N=Y_N, coupled=bool(net.coupled))
 
 
+def textbook_admittance(net):
+    """Textbook nodal admittance matrices Y(h) [H, n, n] in incidence form: every branch adds its
+    series admittance and both halves of its pi-shunt at the buses it connects, parallel branches
+    add up, and the bus shunt 1/(j X_sh h) applies above the fundamental.  This is what
+    hpf_set_y_options(FIX_SHUNT_INDEX | SUM_PARALLEL) builds."""
+    harmonics, n = np.asarray(net.harmonics), net.n
+    want = np.zeros((len(harmonics), n, n), dtype=complex)
+    for hi, h in enumerate(harmonics):
+        for l in range(len(net.R)):
+            f, t = net.from_id[l] - 1, net.to_id[l] - 1
+            y = 1 / (net.R[l] + 1j * net.X[l] * h)
+            sh = (net.G[l] + 1j * h * net.B[l]) / 2
+            want[hi, f, f] += y + sh; want[hi, t, t] += y + sh
+            want[hi, f, t] -= y; want[hi, t, f] -= y
+        for k in range(n):
+            if net.X_sh[k] != 0 and h != 1:
+                want[hi, k, k] += 1 / (1j * net.X_sh[k] * h)
+    return want
+
+
 def synthetic_packed(kind, tmpdir, h_max=25, coupled=True, **kw):
     """Synthetic network (config 4 / 5 generators) through the product's own CSV loaders."""
     from harmonic_power_flow_b200 import synthetic

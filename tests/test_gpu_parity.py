@@ -1026,17 +1026,7 @@ def test_ybus_corrected_options_match_textbook_admittance_matrix():
     sol = BatchSolver(net)
     Y_ref_behaviour = sol.Y.cpu().numpy().copy()
     Y = sol.set_y_options(fix_shunt_index=True, sum_parallel=True).cpu().numpy()
-    want = np.zeros((len(harmonics), n, n), dtype=complex)
-    for hi, h in enumerate(harmonics):
-        for l in range(L):
-            f, t = frm[l] - 1, to[l] - 1
-            y = 1 / (R[l] + 1j * X[l] * h)
-            sh = (G[l] + 1j * h * B[l]) / 2
-            want[hi, f, f] += y + sh; want[hi, t, t] += y + sh
-            want[hi, f, t] -= y; want[hi, t, f] -= y
-        for k in range(n):
-            if X_sh[k] != 0 and h != 1:
-                want[hi, k, k] += 1 / (1j * X_sh[k] * h)
+    want = helpers.textbook_admittance(net)
     assert np.abs(Y - want).max() <= 1e-13 * np.abs(want).max()
     assert np.abs(Y - Y_ref_behaviour).max() > 1e-3 * np.abs(want).max()      # the quirks do matter here
     assert np.array_equal(sol.set_y_options().cpu().numpy(), Y_ref_behaviour)
