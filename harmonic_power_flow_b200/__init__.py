@@ -10,7 +10,7 @@ all arithmetic runs in hand-written sm_100a CUDA kernels.  No CPU fallback.
 from . import netio  # noqa: F401
 from .netio import Settings, PackedNet, pack_network  # noqa: F401
 
-__all__ = ["netio", "Settings", "PackedNet", "pack_network", "BatchSolver", "BatchResult",
+__all__ = ["netio", "Settings", "PackedNet", "pack_network", "BatchSolver", "BatchResult", "BatchStats",
            "hcne_generalized", "ne_from_sim", "scenarios", "synthetic", "dist"]
 
 
@@ -18,7 +18,7 @@ def __getattr__(name):
     # torch-dependent modules are imported lazily so that the data-contract layer
     # (netio) stays importable in tools that only read/write the CSV formats
     import importlib
-    if name in ("BatchSolver", "BatchResult"):
+    if name in ("BatchSolver", "BatchResult", "BatchStats"):
         return getattr(importlib.import_module(".solver", __name__), name)
     if name in ("hcne_generalized", "ne_from_sim", "scenarios", "synthetic", "dist", "solver", "_lib", "build"):
         return importlib.import_module("." + name, __name__)

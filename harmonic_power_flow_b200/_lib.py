@@ -16,7 +16,8 @@ HPF_OK, HPF_E_INVALID, HPF_E_CUDA, HPF_E_UNSUPPORTED, HPF_E_NOMEM = 0, -1, -2, -
 ST_CONVERGED, ST_MAXITER, ST_SINGULAR, ST_NONFINITE = 0, 1, 2, 3
 SOLVE_RAW = 1
 SOLVE_DENSE = 2
-ABI_VERSION = 11
+ABI_VERSION = 12
+HPF_STATS_MAX_Q = 16
 
 _vp, _i, _d, _ll = C.c_void_p, C.c_int, C.c_double, C.c_longlong
 _ip, _dp = C.POINTER(C.c_int), C.POINTER(C.c_double)
@@ -42,10 +43,12 @@ SIGNATURES = {
     "hpf_last_kernel_ms": (_i, [_vp, _dp]),
     "hpf_thd": (_i, [_vp, _i, _vp, _vp, _vp]),
     "hpf_bus_currents": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "hpf_batch_stats": (_i, [_vp, _i, _vp, _vp, _i, _dp, _vp, _vp, _vp, _vp]),
     "hpf_solve": (_i, [_vp, _i, _vp, _vp, _vp, _d, _i, _d, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
                        _vp, _vp, _vp]),
     "hpf_solve_host": (_i, [_vp, _i, _vp, _vp, _vp, _d, _i, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hpf_solve_host_keep": (_i, [_vp, _i, _vp, _vp, _vp, _d, _i, _d, _i] + [_vp] * 14),
+    "hpf_solve_host_stats": (_i, [_vp, _i, _vp, _vp, _vp, _d, _i, _d, _i, _i, _dp, _vp] + [_vp] * 6),
     "hpf_fund_solve": (_i, [_vp, _i, _vp, _vp, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hpf_mismatch": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hpf_jacobian": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),

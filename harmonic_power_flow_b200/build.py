@@ -16,7 +16,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libhpf_b200.so")
 SOURCES = ["hpf_kernels.cu"]
-DEPS = ["hpf_device.cuh", "hpf_zgemm.cuh", "hpf_lu_panel.cuh", "hpf_structured.cuh", "hpf_lane.cuh", "hpf_harmonic_warp.cuh", "hpf_lu_blocked.cuh", "hpf_lockstep.cuh", "hpf_ne_extract.cuh", os.path.join(ROOT, "include", "hpf_b200.h")]
+DEPS = ["hpf_device.cuh", "hpf_zgemm.cuh", "hpf_lu_panel.cuh", "hpf_structured.cuh", "hpf_lane.cuh", "hpf_harmonic_warp.cuh", "hpf_lu_blocked.cuh", "hpf_lockstep.cuh", "hpf_ne_extract.cuh", "hpf_stats.cuh", os.path.join(ROOT, "include", "hpf_b200.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "--shared", "-Xcompiler", "-fPIC", "-Xptxas", "-v"]

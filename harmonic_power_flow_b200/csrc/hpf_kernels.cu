@@ -5,6 +5,7 @@
 //   kernel 3  jacobian_kernel        dense FP64 Jacobian -> HBM (TMA)   HG:401-473
 //   kernel 4  lu_solve_kernel        batched smem LU + solves           HG:476-479
 //   fused     solve_kernel           pf() + hpf() Newton loops          HG:244-275,511-560
+//   after     stats_kernel           batch statistics (hpf_stats.cuh)
 //
 // HG = "Harmonic Power Flow/hcne_generalized.py" of the reference.  No reference code is
 // used; the arithmetic is restated from the formulas (see hpf_device.cuh).
@@ -13,6 +14,7 @@
 #include <cstdlib>
 #include <chrono>
 #include <cstring>
+#include <limits>
 #include <memory>
 #include <new>
 #include <string>
@@ -1038,6 +1040,8 @@ __global__ void bus_currents_kernel(const DevNet net, int B, const double* __res
     I_bus[idx] = acc;
 }
 
+#include "hpf_stats.cuh"
+
 // =======================================================================================
 // Host side: handle + C ABI
 #define HPF_HOST_MAX_CHUNKS 16          // chunks of one hpf_solve_host call (work-counter slots, event pairs)
@@ -1088,7 +1092,8 @@ struct hpf_handle {
     Scratch<double> d_work;
     Scratch<double> d_io;         // staging buffers of hpf_solve_host
     Stream st_io[6];              // copy-in, compute, copy-out, compute 2..4
-    Event ev_io[2 * HPF_HOST_MAX_CHUNKS];
+    Event ev_io[3 * HPF_HOST_MAX_CHUNKS];   // per chunk: inputs copied, solved, V_m kept (hpf_solve_host_stats)
+    Scratch<double> d_stats;      // hpf_batch_stats: THD rows; hpf_solve_host_stats: whole-batch V_m, THD rows, limits, results
     // structured strategy: 0 = not set up yet, 1 = ready, -1 = not available for this network
     int struct_state = 0;
     StructBufs d_struct;
@@ -1364,14 +1369,15 @@ struct SolveReq {
 // Argument checks of a solve request at entry point `who`, in this order: handle ready, B < 0, NULL
 // buffers.  I_N is needed only with nonlinear buses; the fundamental-only solve (mode 1) needs no
 // device tables and has no harmonic outputs.  A request with B == 0 passes: it has nothing to do.
+// Mode 2 is the statistics host solve: a whole solve whose per-scenario outputs are all optional.
 static int check_request(hpf_t* h, const SolveReq& r, int mode, const char* who) {
-    int rc = ready(h, who, mode == 0);
+    int rc = ready(h, who, mode != 1);
     if (rc) return rc;
     if (r.B < 0) return fail(h, HPF_E_INVALID, std::string(who) + ": B < 0");
     if (r.B == 0) return HPF_OK;
     const BatchOut& o = r.out;
-    if (!r.P || !r.Q || !o.V_m || !o.V_a || !o.n_iter_f ||
-        (mode == 0 && (!o.n_iter_h || !o.err_h || !o.status || (h->q > 0 && !r.I_N))))
+    const bool outs = mode == 2 || (o.V_m && o.V_a && o.n_iter_f && (mode == 1 || (o.n_iter_h && o.err_h && o.status)));
+    if (!r.P || !r.Q || !outs || (mode != 1 && h->q > 0 && !r.I_N))
         return fail(h, HPF_E_INVALID, std::string(who) + ": NULL buffer");
     return HPF_OK;
 }
@@ -2824,6 +2830,80 @@ int hpf_fund_solve(hpf_t* h, int B, const double* P, const double* Q, double thr
 
 } // extern "C"
 
+// ---- batch statistics -------------------------------------------------------------------
+// Argument checks shared by hpf_batch_stats and hpf_solve_host_stats (h != NULL).
+static int check_stats_args(hpf_t* h, int B, int K, const double* quantiles, const int* counts,
+                            const double* stats, const char* who) {
+    const std::string w(who);
+    if (!h->have_net) return fail(h, HPF_E_INVALID, w + ": call hpf_set_network first");
+    if (B < 0) return fail(h, HPF_E_INVALID, w + ": B < 0");
+    if (K < 0 || K > HPF_STATS_MAX_Q)
+        return fail(h, HPF_E_INVALID, w + ": K = " + std::to_string(K) + " outside [0, HPF_STATS_MAX_Q]");
+    if ((K > 0 && !quantiles) || !counts || !stats) return fail(h, HPF_E_INVALID, w + ": NULL buffer");
+    for (int k = 0; k < K; ++k)
+        if (!(quantiles[k] >= 0.0 && quantiles[k] <= 1.0))
+            return fail(h, HPF_E_INVALID, w + ": quantile " + std::to_string(k) + " is NaN or outside [0, 1]");
+    return HPF_OK;
+}
+
+// CTAs per row (the cluster size of stats_kernel): about four CTAs per SM over all rows, at most 8 (the
+// portable cluster size), at least 2,048 scenarios per CTA.  The reduction order follows from it, so it
+// depends on (R, B) and the device only.
+static int stats_cluster(const hpf_t* h, int R, int B) {
+    int cs = (4 * h->sm_count + R - 1) / R;
+    if (cs > 8) cs = 8;
+    const int by_b = (B + 2047) / 2048;
+    if (cs > by_b) cs = by_b;
+    return cs < 1 ? 1 : cs;
+}
+
+// THD rows of V_m into `thd` ([2, n, B] scratch, thd_kernel as in hpf_thd), then one cluster of
+// stats_kernel per row.  Checked arguments; all pointers device memory except `quantiles`.
+static int launch_batch_stats(hpf_t* h, int B, const double* V_m, const int* status, int K, const double* quantiles,
+                              const double* limits, int* counts, double* stats, double* thd, cudaStream_t st) {
+    const int n = h->n, nH = n * h->H, R = nH + 2 * n;
+    if (B > 0) {
+        const size_t total = (size_t)n * B;
+        thd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n, h->H, h->d_harm.get(), B, V_m, thd);
+        h->launches++;
+        CK(cudaGetLastError());
+    }
+    StatsArgs a;
+    a.B = B; a.R = R; a.nH = nH; a.K = K;
+    a.V_m = V_m; a.thd = thd; a.status = status; a.limits = limits; a.counts = counts; a.stats = stats;
+    for (int k = 0; k < HPF_STATS_MAX_Q; ++k) a.q[k] = k < K ? quantiles[k] : 0.0;
+    const int cs = stats_cluster(h, R, B);
+    const size_t smem = stats_smem_bytes(K);
+    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(cs * R)); cfg.blockDim = dim3(HPF_STATS_THREADS);
+    cfg.dynamicSmemBytes = smem; cfg.stream = st; cfg.attrs = attr; cfg.numAttrs = 1;
+    CK(cudaLaunchKernelEx(&cfg, stats_kernel, a));
+    h->launches++;
+    return HPF_OK;
+}
+
+extern "C" {
+
+int hpf_batch_stats(hpf_t* h, int B, const double* V_m, const int* status, int K, const double* quantiles,
+                    const double* limits, int* status_counts, double* stats, void* stream) {
+    if (!h) return HPF_E_INVALID;
+    int rc = check_stats_args(h, B, K, quantiles, status_counts, stats, "hpf_batch_stats");
+    if (rc) return rc;
+    if (B > 0 && !V_m) return fail(h, HPF_E_INVALID, "hpf_batch_stats: NULL V_m");
+    return ordered(h, stream, [&] {
+        const int r = grow(h, h->d_stats, (size_t)2 * h->n * B * sizeof(double), "hpf_batch_stats: THD rows");
+        if (r) return r;
+        return launch_batch_stats(h, B, V_m, status, K, quantiles, limits, status_counts, stats, h->d_stats.get(),
+                                  (cudaStream_t)stream);
+    });
+}
+
+} // extern "C"
+
 // Chunk plan of hpf_solve_host: boundaries cb[0..nchunk] (multiples of 32 scenarios except the end) and
 // the number of compute streams the chunks rotate over.  $HPF_HOST_PLAN = comma-separated chunk sizes
 // (the last size repeats until the batch is covered; at most HPF_HOST_MAX_CHUNKS chunks, the last one
@@ -2861,9 +2941,20 @@ static int host_chunk_plan(size_t Bs, size_t* cb, int* streams) {
     return k;
 }
 
+// What hpf_solve_host_stats asks of the host solve path: statistics instead of phasors (host buffers).
+struct StatsOut {
+    int K = 0;
+    const double *quantiles = nullptr, *limits = nullptr;
+    int* counts = nullptr;
+    double* stats = nullptr;
+};
+
 // hpf_solve_host: `hr` holds host arrays; keep, when given, receives device copies of the results.
-static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
-    int rc = check_request(h, hr, 0, "hpf_solve_host");
+// With `so` (hpf_solve_host_stats) no phasor goes back: each chunk's V_m is kept in a whole-batch device
+// array, and after the last chunk the copy-out stream reduces it with the whole-batch status array
+// (launch_batch_stats) and copies back the statistics and the flag arrays that hr asks for.
+static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep, const StatsOut* so = nullptr) {
+    int rc = check_request(h, hr, so ? 2 : 0, so ? "hpf_solve_host_stats" : "hpf_solve_host");
     if (rc || hr.B == 0) return rc;
     ENTER_DEVICE(h);
     // Pipelined in chunks of scenarios: while chunk k is being solved, chunk k+1 is copied in and
@@ -2889,10 +2980,23 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
     const size_t nd = per_scn * Bs + Bp + 3 * (Bp / 2);
     rc = grow(h, h->d_io, nd * sizeof(double), "hpf_solve_host: staging buffers");
     if (rc) return rc;
+    // statistics: whole-batch V_m [H, n, B] | THD rows [2, n, B] | limits [R] | stats [5 + K, R] | counts
+    const size_t R = n * H + 2 * n;
+    if (so) {
+        rc = grow(h, h->d_stats, ((H + 2) * n * Bs + R + (5 + so->K) * R + 2) * sizeof(double),
+                  "hpf_solve_host_stats: statistics scratch");
+        if (rc) return rc;
+    }
+    double *const dVfull = h->d_stats.get(), *const dThd = dVfull + H * n * Bs, *const dLim = dThd + 2 * n * Bs,
+           *const dStats = dLim + R;
+    int* const dCounts = so ? reinterpret_cast<int*>(dStats + (5 + so->K) * R) : nullptr;
+    BatchOut keep_vm;                    // the statistics keep V_m only: the flag arrays already sit in d_io
+    keep_vm.V_m = dVfull;
+    if (so) keep = &keep_vm;
     if (!h->st_io[0]) {
         // all or nothing: the handle takes the streams and events only when every one of them exists
         Stream st[6];
-        Event ev[2 * HPF_HOST_MAX_CHUNKS];
+        Event ev[3 * HPF_HOST_MAX_CHUNKS];
         for (auto& s : st) {
             cudaStream_t raw = nullptr;
             CK(cudaStreamCreateWithFlags(&raw, cudaStreamNonBlocking));
@@ -2900,7 +3004,7 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
         }
         for (auto& e : ev) CK(create_event(e, cudaEventDisableTiming));
         for (int i = 0; i < 6; ++i) h->st_io[i] = std::move(st[i]);
-        for (int i = 0; i < 2 * HPF_HOST_MAX_CHUNKS; ++i) h->ev_io[i] = std::move(ev[i]);
+        for (int i = 0; i < 3 * HPF_HOST_MAX_CHUNKS; ++i) h->ev_io[i] = std::move(ev[i]);
     }
     cudaStream_t s_in = h->st_io[0].get(), s_out = h->st_io[2].get();
     const int cmp_stream[4] = {1, 3, 4, 5};
@@ -2962,32 +3066,50 @@ static int solve_host_impl(hpf_t* h, const SolveReq& hr, const BatchOut* keep) {
         e = cudaEventRecord(h->ev_io[HPF_HOST_MAX_CHUNKS + k].get(), s_cmp);
         if (tl) cudaEventRecord(tle[3 * k + 1].get(), s_cmp);
         if (e == cudaSuccess) e = cudaStreamWaitEvent(s_out, h->ev_io[HPF_HOST_MAX_CHUNKS + k].get(), 0);
-        if (e == cudaSuccess) e = cp2d(ho.V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
-        if (e == cudaSuccess) e = cp2d(ho.V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
+        if (e == cudaSuccess && !so) e = cp2d(ho.V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
+        if (e == cudaSuccess && !so) e = cp2d(ho.V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToHost, s_out);
         if (e == cudaSuccess && ho.I_inj && q)
             e = cp2d(ho.I_inj + b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToHost, s_out);
         if (e == cudaSuccess && k == nchunk - 1) {       // s_out has waited for every chunk by now
-            e = cudaMemcpyAsync(ho.err_h, dErr_all, Bs * sizeof(double), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.n_iter_f, di_all, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.n_iter_h, di_all + Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(ho.status, di_all + 2 * Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            // (the statistics host solve copies back only the flag arrays it is given)
+            if (ho.err_h) e = cudaMemcpyAsync(ho.err_h, dErr_all, Bs * sizeof(double), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess && ho.n_iter_f) e = cudaMemcpyAsync(ho.n_iter_f, di_all, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess && ho.n_iter_h) e = cudaMemcpyAsync(ho.n_iter_h, di_all + Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+            if (e == cudaSuccess && ho.status) e = cudaMemcpyAsync(ho.status, di_all + 2 * Bp, Bs * sizeof(int), cudaMemcpyDeviceToHost, s_out);
         }
         if (tl) cudaEventRecord(tle[3 * k + 2].get(), s_out);
         if (e == cudaSuccess && keep) {
             // also leave the results on the device in the full [rows, B] layout (device-to-device
             // 2-D copies on the compute stream, ~20 us for the whole batch)
             e = cp2d(keep->V_m + b0, p8, dVm, w8, w8, n * H, cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess) e = cp2d(keep->V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->V_a) e = cp2d(keep->V_a + b0, p8, dVa, w8, w8, n * H, cudaMemcpyDeviceToDevice, s_cmp);
             if (e == cudaSuccess && keep->I_inj && ho.I_inj && q)
                 e = cp2d(keep->I_inj + b0, p16, dInj, w16, w16, q * H, cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(keep->err_h + b0, dErr, Bc * sizeof(double), cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(keep->n_iter_f + b0, di_f, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(keep->n_iter_h + b0, di_h, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
-            if (e == cudaSuccess) e = cudaMemcpyAsync(keep->status + b0, di_s, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->err_h) e = cudaMemcpyAsync(keep->err_h + b0, dErr, Bc * sizeof(double), cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->n_iter_f) e = cudaMemcpyAsync(keep->n_iter_f + b0, di_f, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->n_iter_h) e = cudaMemcpyAsync(keep->n_iter_h + b0, di_h, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
+            if (e == cudaSuccess && keep->status) e = cudaMemcpyAsync(keep->status + b0, di_s, Bc * sizeof(int), cudaMemcpyDeviceToDevice, s_cmp);
+        }
+        if (e == cudaSuccess && so) {
+            // the keep copies run on the compute stream AFTER the chunk's "solved" event: the statistics
+            // wait for an event recorded behind them
+            e = cudaEventRecord(h->ev_io[2 * HPF_HOST_MAX_CHUNKS + k].get(), s_cmp);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(s_out, h->ev_io[2 * HPF_HOST_MAX_CHUNKS + k].get(), 0);
         }
         if (e != cudaSuccess) break;
     }
-    if (!rc && e != cudaSuccess) rc = fail(h, HPF_E_CUDA, std::string("hpf_solve_host: ") + cudaGetErrorString(e));
+    if (!rc && e == cudaSuccess && so) {
+        // s_out has waited for every chunk's V_m copy: reduce the whole batch, copy back the results
+        if (so->limits) e = cudaMemcpyAsync(dLim, so->limits, R * sizeof(double), cudaMemcpyHostToDevice, s_out);
+        if (e == cudaSuccess)
+            rc = launch_batch_stats(h, hr.B, dVfull, di_all + 2 * Bp, so->K, so->quantiles, so->limits ? dLim : nullptr,
+                                    dCounts, dStats, dThd, s_out);
+        if (!rc && e == cudaSuccess)
+            e = cudaMemcpyAsync(so->stats, dStats, (5 + so->K) * R * sizeof(double), cudaMemcpyDeviceToHost, s_out);
+        if (!rc && e == cudaSuccess) e = cudaMemcpyAsync(so->counts, dCounts, 4 * sizeof(int), cudaMemcpyDeviceToHost, s_out);
+    }
+    if (!rc && e != cudaSuccess)
+        rc = fail(h, HPF_E_CUDA, std::string(so ? "hpf_solve_host_stats: " : "hpf_solve_host: ") + cudaGetErrorString(e));
     for (auto& s : h->st_io) {
         const cudaError_t e2 = cudaStreamSynchronize(s.get());
         if (!rc && e2 != cudaSuccess) rc = fail(h, HPF_E_CUDA, std::string("hpf_solve_host: ") + cudaGetErrorString(e2));
@@ -3033,6 +3155,29 @@ int hpf_solve_host_keep(hpf_t* h, int B, const double* P, const double* Q, const
     k.V_m = dV_m; k.V_a = dV_a; k.I_inj = (double2*)dI_inj; k.err_h = derr_h;
     k.n_iter_f = dn_iter_f; k.n_iter_h = dn_iter_h; k.status = dstatus;
     return solve_host_impl(h, r, &k);
+}
+
+int hpf_solve_host_stats(hpf_t* h, int B, const double* P, const double* Q, const double* I_N, double thresh_f,
+                         int max_iter_f, double thresh_h, int max_iter_h, int K, const double* quantiles,
+                         const double* limits, int* status_counts, double* stats, int* n_iter_f, int* n_iter_h,
+                         double* err_h, int* status) {
+    if (!h) return HPF_E_INVALID;
+    int rc = check_stats_args(h, B, K, quantiles, status_counts, stats, "hpf_solve_host_stats");
+    if (rc) return rc;
+    SolveReq r;
+    r.B = B; r.P = P; r.Q = Q; r.I_N = (const double2*)I_N;
+    r.thresh_f = thresh_f; r.max_f = max_iter_f; r.thresh_h = thresh_h; r.max_h = max_iter_h;
+    r.out.n_iter_f = n_iter_f; r.out.n_iter_h = n_iter_h; r.out.err_h = err_h; r.out.status = status;
+    StatsOut so;
+    so.K = K; so.quantiles = quantiles; so.limits = limits; so.counts = status_counts; so.stats = stats;
+    rc = solve_host_impl(h, r, nullptr, &so);
+    if (rc || B > 0) return rc;
+    // an empty batch: no scenario included
+    const size_t R = (size_t)h->n * h->H + 2 * h->n;
+    for (int i = 0; i < 4; ++i) status_counts[i] = 0;
+    for (size_t p = 0; p < (size_t)(5 + K); ++p)
+        for (size_t i = 0; i < R; ++i) stats[p * R + i] = p == 4 ? 0.0 : std::numeric_limits<double>::quiet_NaN();
+    return HPF_OK;
 }
 
 static int mismatch_impl(hpf_t* h, int B, const double* V_m, const double* V_a, const double* P, const double* Q,

@@ -70,6 +70,56 @@ class BatchResult:
         return out
 
 
+@dataclass
+class BatchStats:
+    """Statistics of a batch (hpf_batch_stats / hpf_solve_host_stats) over R = n*H + 2n rows: V_m of
+    order harmonics[h] at bus i (row h*n + i), THD_F (row n*H + i), THD_R (row n*H + n + i).
+    ``planes`` [5 + K, R]: mean, std (population), min, max, exceed (count above the limit), then one
+    nearest-rank quantile per level of ``quantiles``.  Device tensors from ``batch_stats``, numpy
+    arrays from ``solve_host_stats`` (which also puts the optional flag arrays in ``flags``)."""
+    status_counts: object      # [4] int32: scenarios per HPF_ST_* value
+    quantiles: tuple
+    planes: object             # [5 + K, R] f64
+    n: int
+    H: int
+    flags: dict = None
+
+    STATS = ("mean", "std", "min", "max", "exceed")
+
+    def plane(self, stat):
+        """[R] row of a statistic: one of STATS or a quantile level given to the call."""
+        if isinstance(stat, str):
+            return self.planes[self.STATS.index(stat)]
+        return self.planes[5 + [float(p) for p in self.quantiles].index(float(stat))]
+
+    def V_m(self, stat):
+        """[H, n] for V_m."""
+        return self.plane(stat)[:self.n * self.H].reshape(self.H, self.n)
+
+    def THD_F(self, stat):
+        """[n] for THD_F."""
+        return self.plane(stat)[self.n * self.H:self.n * self.H + self.n]
+
+    def THD_R(self, stat):
+        """[n] for THD_R."""
+        return self.plane(stat)[self.n * self.H + self.n:]
+
+
+def stats_limit_rows(limits, n, H):
+    """{"V_m": [H, n] or broadcastable, "THD_F" / "THD_R": [n] or scalar} -> [R] float64 rows (a missing
+    key = +inf: never exceeded), or None for no limits."""
+    if limits is None:
+        return None
+    unknown = set(limits) - {"V_m", "THD_F", "THD_R"}
+    if unknown:
+        raise ValueError("unknown limit keys %s" % sorted(unknown))
+    inf = np.inf
+    vm = np.broadcast_to(np.asarray(limits.get("V_m", inf), np.float64), (H, n))
+    tf = np.broadcast_to(np.asarray(limits.get("THD_F", inf), np.float64), (n,))
+    tr = np.broadcast_to(np.asarray(limits.get("THD_R", inf), np.float64), (n,))
+    return np.ascontiguousarray(np.concatenate([vm.ravel(), tf, tr]))
+
+
 def result_slab_layout(H, n, q, B):
     """Byte offsets of the result fields in ONE contiguous slab (multi-GPU runs gather and copy
     the slab with one collective / one D2H instead of seven): -> (dict name -> (offset, shape,
@@ -223,6 +273,57 @@ class BatchSolver:
         out = self._f64(2, self.net.n, B)
         _lib.check(self._h, self.lib.hpf_thd(self._h, B, _ptr(V_m), _ptr(out), self._stream()))
         return out
+
+    def _quantile_levels(self, quantiles):
+        q = np.ascontiguousarray(np.asarray(quantiles, dtype=np.float64).ravel())
+        if q.size > _lib.HPF_STATS_MAX_Q:
+            raise ValueError("at most %d quantile levels" % _lib.HPF_STATS_MAX_Q)
+        return q
+
+    def batch_stats(self, V_m, status=None, quantiles=(0.5, 0.95), limits=None) -> BatchStats:
+        """Statistics of V_m [H, n, B] and its THD over the converged scenarios (all of them when
+        ``status`` is None), on the device (hpf_batch_stats).  ``limits``: see stats_limit_rows."""
+        n = self.net
+        V_m = self._dev(V_m, torch.float64)
+        if tuple(V_m.shape[:2]) != (n.H, n.n) or V_m.dim() != 3:
+            raise ValueError("V_m must be [H, n, B]")
+        B = V_m.shape[2]
+        if status is not None:
+            status = self._dev(status, torch.int32)
+            if tuple(status.shape) != (B,):
+                raise ValueError("status must be [B]")
+        q = self._quantile_levels(quantiles)
+        lim = stats_limit_rows(limits, n.n, n.H)
+        lim = None if lim is None else self._dev(lim, torch.float64)
+        R = n.n * n.H + 2 * n.n
+        counts, planes = self._i32(4), self._f64(5 + q.size, R)
+        _lib.check(self._h, self.lib.hpf_batch_stats(self._h, B, _ptr(V_m), _ptr(status), int(q.size), _np_d(q),
+                                                     _ptr(lim), _ptr(counts), _ptr(planes), self._stream()))
+        return BatchStats(counts, tuple(float(p) for p in q), planes, n.n, n.H)
+
+    def solve_host_stats(self, P, Q, I_N, thresh_f=1e-6, max_iter_f=30, thresh_h=1e-4, max_iter_h=50,
+                         quantiles=(0.5, 0.95), limits=None, want_flags=False) -> BatchStats:
+        """hpf_solve_host_stats: numpy in, statistics out (numpy); only the inputs and a few KB of
+        statistics cross the host link.  ``want_flags=True`` also returns the per-scenario n_iter_f,
+        n_iter_h, err_h and status in ``flags``."""
+        n = self.net
+        P = np.ascontiguousarray(P, dtype=np.float64)
+        Q = np.ascontiguousarray(Q, dtype=np.float64)
+        B = P.shape[1]
+        I_N = np.ascontiguousarray(I_N, dtype=np.complex128) if n.q > 0 else np.zeros(0, np.complex128)
+        q = self._quantile_levels(quantiles)
+        lim = stats_limit_rows(limits, n.n, n.H)
+        R = n.n * n.H + 2 * n.n
+        counts, planes = np.empty(4, np.int32), np.empty((5 + q.size, R), np.float64)
+        flags = dict(n_iter_f=np.empty(B, np.int32), n_iter_h=np.empty(B, np.int32), err_h=np.empty(B, np.float64),
+                     status=np.empty(B, np.int32)) if want_flags else None
+        vp = lambda a: C.c_void_p(None if a is None else a.ctypes.data)
+        f = flags or {}
+        _lib.check(self._h, self.lib.hpf_solve_host_stats(
+            self._h, B, vp(P), vp(Q), vp(I_N), thresh_f, max_iter_f, thresh_h, max_iter_h,
+            int(q.size), _np_d(q), vp(lim), vp(counts), vp(planes),
+            vp(f.get("n_iter_f")), vp(f.get("n_iter_h")), vp(f.get("err_h")), vp(f.get("status"))))
+        return BatchStats(counts, tuple(float(p) for p in q), planes, n.n, n.H, flags)
 
     # -- inputs ------------------------------------------------------------------------
     def prepare(self, P, Q, I_N=None):

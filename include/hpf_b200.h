@@ -67,7 +67,7 @@ typedef struct hpf_handle hpf_t;
 #define HPF_ST_NONFINITE    3   /* NaN/Inf in the mismatch or the state            */
 
 /* ABI version of this header: bumped on any signature change. */
-#define HPF_ABI_VERSION 11
+#define HPF_ABI_VERSION 12
 int hpf_abi_version(void);
 
 /* Lifetime.  `device` is the CUDA ordinal the handle is bound to. */
@@ -267,6 +267,50 @@ int hpf_norton_wn(hpf_t* h, int B, const double* I_N, double* wN, void* stream);
  *   in : V_m [H, n, B];  out: thd [2, n, B]  (plane 0 = THD_F, plane 1 = THD_R)
  */
 int hpf_thd(hpf_t* h, int B, const double* V_m, double* thd, void* stream);
+
+/*
+ * Batch statistics of a solved batch, on the device: for a network of n buses and H orders the
+ * R = n*H + 2n rows are  row h*n + i = V_m of order harmonics[h] at bus i (the V_m layout),
+ * row n*H + i = THD_F of bus i, row n*H + n + i = THD_R of bus i (THD exactly as hpf_thd writes it).
+ * A scenario is included when status[b] == HPF_ST_CONVERGED; status == NULL includes all of them;
+ * n_valid = number included.
+ *   in : V_m [H, n, B] (device), status [B] (device) or NULL, limits [R] (device) or NULL,
+ *        quantiles [K] (host), 0 <= K <= HPF_STATS_MAX_Q, each in [0, 1]
+ *   out: status_counts int[4] (device): scenarios per HPF_ST_* value ({B, 0, 0, 0} without status);
+ *        stats [5 + K, R] doubles (device), one plane per statistic:
+ *          0 mean, 1 population std (ddof 0, two passes: mean, then squared deviations), 2 min, 3 max,
+ *          4 exceed = included scenarios with x > limits[r] (0 without limits or for limit +inf),
+ *          5 + k = quantile p_k: the included value of rank max(1, ceil(p_k * n_valid)) in ascending
+ *          order (nearest rank, numpy's method="inverted_cdf"; p = 0 gives min, p = 1 max) - an exact
+ *          order statistic, no interpolation.
+ *        Values are ordered by their bit patterns (-0 below +0).  n_valid == 0 (or B == 0): planes 0-3
+ *        and the quantiles are NaN, exceed 0.
+ * The same inputs give the same bits on every call and stream (no floating-point atomics; sums run in
+ * an order fixed by B and the launch shape).  Uses the handle's scratch (THD rows), so it goes through
+ * the handle's ordering like hpf_solve; the first call with a larger B than before grows that scratch
+ * (device synchronisation + reallocation) like the other grow-only buffers.
+ */
+#define HPF_STATS_MAX_Q 16
+int hpf_batch_stats(hpf_t* h, int B, const double* V_m, const int* status,
+                    int K, const double* quantiles, const double* limits,
+                    int* status_counts, double* stats, void* stream);
+
+/*
+ * hpf_solve_host that returns the statistics of hpf_batch_stats instead of the per-scenario phasors:
+ * copies the inputs in (chunk-pipelined like hpf_solve_host), solves, reduces on the device and copies
+ * back only status_counts int[4] and stats [5 + K, R] - a few KB instead of V_m, V_a and I_inj.  Every
+ * buffer here is HOST memory, limits [R] (or NULL) included; quantiles and limits mean what they mean
+ * in hpf_batch_stats.  n_iter_f, n_iter_h, err_h,
+ * status [B] may each be NULL (then not copied back).  Bit-identical to hpf_batch_stats over the V_m and
+ * status that hpf_solve_host_keep leaves on the device for the same inputs and chunk plan - and so, where
+ * the chunked solve equals hpf_solve (the 4-bus paths), to hpf_solve followed by hpf_batch_stats.
+ * Synchronises.
+ */
+int hpf_solve_host_stats(hpf_t* h, int B, const double* P, const double* Q, const double* I_N,
+                         double thresh_f, int max_iter_f, double thresh_h, int max_iter_h,
+                         int K, const double* quantiles, const double* limits,
+                         int* status_counts, double* stats,
+                         int* n_iter_f, int* n_iter_h, double* err_h, int* status);
 
 /*
  * Post-processing after the path: per-bus current spectra I[h][i] = sum_j Y(h)[i][j] V[h][j] (what
