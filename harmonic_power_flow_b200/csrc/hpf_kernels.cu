@@ -18,6 +18,7 @@
 #include <memory>
 #include <new>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/hpf_b200.h"
@@ -1281,19 +1282,65 @@ static bool fits_smem_lu(const hpf_t* h, const DevNet& net) {
            scn_smem_bytes(net.n, net.H, net.q, net.N, true) <= (size_t)h->smem_optin;
 }
 
+// ---- kernel launches --------------------------------------------------------------------
+// A kernel takes up to 48 KB of dynamic shared memory by default; beyond that it must be allowed per kernel.
 template <class K>
-static int prep_kernel(hpf_t* h, K kernel, size_t smem, const char* who, int* ctas_per_sm,
-                       int threads = HPF_THREADS) {
+static cudaError_t allow_smem(K kernel, size_t smem) {
+    if (smem <= 48 * 1024) return cudaSuccess;
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+}
+
+// CTAs of `kernel` the device holds at once with `threads` threads and `smem` B of dynamic shared
+// memory -> *ctas.  `who`: the entry point named in the error messages.
+template <class K>
+static int resident_ctas(hpf_t* h, K kernel, int threads, size_t smem, const char* who, long long* ctas) {
     if (smem > (size_t)h->smem_optin)
         return fail(h, HPF_E_UNSUPPORTED,
                     std::string(who) + ": system too large for the shared-memory path (needs " +
                         std::to_string(smem) + " B of shared memory per CTA, device offers " +
                         std::to_string(h->smem_optin) + ")");
-    CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CK(allow_smem(kernel, smem));
     int occ = 0;
     CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem));
     if (occ < 1) return fail(h, HPF_E_UNSUPPORTED, std::string(who) + ": kernel does not fit on an SM");
-    *ctas_per_sm = occ;
+    *ctas = (long long)occ * h->sm_count;
+    return HPF_OK;
+}
+
+// Grid of a kernel whose CTAs loop over `items` work items: the resident CTAs, at most one per item and
+// at least one; a work-queue kernel (`queue`) also at most $HPF_MAX_CTAS.
+static unsigned fill_grid(const hpf_t* h, long long ctas, long long items, bool queue) {
+    long long g = ctas < items ? ctas : items;
+    if (queue && h->max_ctas && g > h->max_ctas) g = h->max_ctas;
+    return (unsigned)(g < 1 ? 1 : g);
+}
+
+// Grid, block, dynamic shared memory and stream of one launch; cluster > 0: thread-block clusters of
+// that many CTAs along x
+struct LaunchCfg {
+    dim3 grid, block;
+    size_t smem;
+    cudaStream_t st;
+    int cluster = 0;
+};
+
+// The one place that launches a kernel.  The launch counts 1 (hpf_launch_count) and is checked at once;
+// its error is consumed so that it does not stay behind as the runtime's last error.
+template <class... P, class... A>
+static int launch(hpf_t* h, void (*kernel)(P...), const LaunchCfg& c, A&&... args) {
+    CK(allow_smem(kernel, c.smem));
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeClusterDimension;
+    attr.val.clusterDim.x = (unsigned)c.cluster; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = c.grid; cfg.blockDim = c.block; cfg.dynamicSmemBytes = c.smem; cfg.stream = c.st;
+    cfg.attrs = &attr; cfg.numAttrs = c.cluster > 0 ? 1 : 0;
+    const cudaError_t e = cudaLaunchKernelEx(&cfg, kernel, std::forward<A>(args)...);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(h, HPF_E_CUDA, std::string("kernel launch: ") + cudaGetErrorString(e));
+    }
+    h->launches++;
     return HPF_OK;
 }
 
@@ -1333,11 +1380,10 @@ static auto with_lu_kind(int kind, F&& f) {
 
 // Flat start (HG:183) of the harmonic rows h = 2..H of a batch whose fundamental stage ran on the
 // one-harmonic view.
-static void flat_start_harmonics(hpf_t* h, int n, int H, int B, double* V_m, double* V_a, cudaStream_t st) {
+static int flat_start_harmonics(hpf_t* h, int n, int H, int B, double* V_m, double* V_a, cudaStream_t st) {
     const size_t cnt = (size_t)(H - 1) * n * B;
-    flat_start_fill_kernel<<<(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st>>>(
-        V_m + (size_t)n * B, V_a + (size_t)n * B, cnt);
-    h->launches++;
+    return launch(h, flat_start_fill_kernel, {(unsigned)((cnt + 255) / 256 < 65535 * 8 ? (cnt + 255) / 256 : 65535 * 8), 256, 0, st},
+                  V_m + (size_t)n * B, V_a + (size_t)n * B, cnt);
 }
 
 // ---- solve requests -------------------------------------------------------------------
@@ -1421,13 +1467,11 @@ static int solve_common(hpf_t* h, int mode, const SolveReq& r, cudaStream_t st) 
     const LuPlan lu = lu_plan(h, net);
     const auto kernel = with_lu_kind(lu.kind, [](auto k) { return solve_kernel<decltype(k)::value>; });
     const int threads = lu.kind ? HPF_THREADS_GMEM : HPF_THREADS;
-    int occ = 0;
-    int rc = prep_kernel(h, kernel, lu.smem, who, &occ, threads);
+    long long ctas = 0;
+    int rc = resident_ctas(h, kernel, threads, lu.smem, who, &ctas);
     if (rc) return rc;
     CK(cudaMemsetAsync(h->d_counter.get() + r.slot, 0, sizeof(int), st));
-    long long grid = (long long)occ * h->sm_count;
-    if (grid > r.B) grid = r.B;
-    if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
+    const unsigned grid = fill_grid(h, ctas, r.B, true);
     double* workspace = nullptr;
     if (lu.kind) {
         rc = grow(h, h->d_work, (size_t)grid * lub_ld(net.N) * (net.N + 1) * sizeof(double),
@@ -1436,11 +1480,10 @@ static int solve_common(hpf_t* h, int mode, const SolveReq& r, cudaStream_t st) 
         workspace = h->d_work.get();
     }
     if (h->profiling) { CK(cudaEventRecord(h->ev[1].get(), st)); }
-    kernel<<<(unsigned)grid, threads, lu.smem, st>>>(net, solve_args(h, r, mode, lu, workspace));
-    if (net.H != H_full) flat_start_harmonics(h, net.n, H_full, r.B, r.out.V_m, r.out.V_a, st);
+    rc = launch(h, kernel, {grid, threads, lu.smem, st}, net, solve_args(h, r, mode, lu, workspace));
+    if (!rc && net.H != H_full) rc = flat_start_harmonics(h, net.n, H_full, r.B, r.out.V_m, r.out.V_a, st);
+    if (rc) return rc;
     if (h->profiling) { CK(cudaEventRecord(h->ev[2].get(), st)); h->ev_valid = 2; }
-    h->launches++;
-    CK(cudaGetLastError());
     return HPF_OK;
 }
 
@@ -1469,45 +1512,38 @@ static int launch_zgemm(hpf_t* h, int M, int N, int K, const double2* A, size_t 
 // read for nn > gj_single_max).
 static int gj_invert(hpf_t* h, double2* A, int nn, int* ipiv, int* info, double* pr, double2* tmp, cudaStream_t st,
                      double2* FR = nullptr) {
-    if (nn <= h->gj_single_max) {
-        cinv_gj_kernel<<<1, 1024, 0, st>>>(nn, A, ipiv, info, pr);
-        h->launches++;
-    } else if (FR && !h->gj_unblocked) {
+    if (nn <= h->gj_single_max) return launch(h, cinv_gj_kernel, {1, 1024, 0, st}, nn, A, ipiv, info, pr);
+    const unsigned g1 = (nn + 255) / 256;
+    int rc;
+    if (FR && !h->gj_unblocked) {
         // blocked: panels of GJB_NB pivots, the rest of the matrix updated by one tensor-core GEMM per panel
         double2 *rowk = tmp, *pinv = tmp + 2 * (size_t)nn;
         double2 *F = FR, *R = FR + (size_t)nn * GJB_NB, *pinv_all = R + (size_t)GJB_NB * nn;
-        const int g1 = (nn + 255) / 256;
         for (int j0 = 0; j0 < nn; j0 += GJB_NB) {
             const int nb = nn - j0 < GJB_NB ? nn - j0 : GJB_NB, j1 = j0 + nb;
             int ge = (nn + 3) / 4;
             if (ge > h->sm_count * 8) ge = h->sm_count * 8;
             for (int k = j0; k < j1; ++k) {
-                gjb_pivot_row_kernel<<<1, 1024, 0, st>>>(nn, k, j0, j1, A, ipiv, info, pr, pinv, rowk, F, pinv_all);
-                gjb_col_elim_kernel<<<ge, dim3(GJB_NB, 4), 0, st>>>(nn, k, j0, j1, A, rowk, pinv, F);
+                if ((rc = launch(h, gjb_pivot_row_kernel, {1, 1024, 0, st}, nn, k, j0, j1, A, ipiv, info, pr, pinv, rowk, F,
+                                 pinv_all))) return rc;
+                if ((rc = launch(h, gjb_col_elim_kernel, {(unsigned)ge, dim3(GJB_NB, 4), 0, st}, nn, k, j0, j1, A, rowk, pinv,
+                                 F))) return rc;
             }
-            gjb_rows_kernel<<<g1, 256, 0, st>>>(nn, j0, nb, A, ipiv, F, pinv_all, R);
-            h->launches += 2LL * nb + 1;
-            int rc = launch_zgemm(h, nn, nn, nb, F, (size_t)GJB_NB, R, (size_t)nn, A, (size_t)nn, st, true);
-            if (rc) return rc;
+            if ((rc = launch(h, gjb_rows_kernel, {g1, 256, 0, st}, nn, j0, nb, A, ipiv, F, pinv_all, R))) return rc;
+            if ((rc = launch_zgemm(h, nn, nn, nb, F, (size_t)GJB_NB, R, (size_t)nn, A, (size_t)nn, st, true))) return rc;
         }
-        gjm_unpermute_kernel<<<g1, 256, 0, st>>>(nn, A, ipiv);
-        h->launches++;
     } else {
         double2 *rowk = tmp, *colk = tmp + nn, *pinv = tmp + 2 * (size_t)nn;
-        const int g1 = (nn + 255) / 256;
-        int gy = (h->sm_count * 8 + g1 - 1) / g1;
-        if (gy > nn) gy = nn;
+        unsigned gy = (h->sm_count * 8 + g1 - 1) / g1;
+        if (gy > (unsigned)nn) gy = nn;
         for (int k = 0; k < nn; ++k) {
-            gjm_pivot_kernel<<<1, 1024, 0, st>>>(nn, k, A, ipiv, info, pr, pinv);
-            gjm_row_kernel<<<g1, 256, 0, st>>>(nn, k, A, ipiv, pinv, rowk);
-            gjm_col_kernel<<<g1, 256, 0, st>>>(nn, k, A, colk);
-            gjm_elim_kernel<<<dim3(g1, gy), 256, 0, st>>>(nn, k, A, rowk, colk);
+            if ((rc = launch(h, gjm_pivot_kernel, {1, 1024, 0, st}, nn, k, A, ipiv, info, pr, pinv))) return rc;
+            if ((rc = launch(h, gjm_row_kernel, {g1, 256, 0, st}, nn, k, A, ipiv, pinv, rowk))) return rc;
+            if ((rc = launch(h, gjm_col_kernel, {g1, 256, 0, st}, nn, k, A, colk))) return rc;
+            if ((rc = launch(h, gjm_elim_kernel, {dim3(g1, gy), 256, 0, st}, nn, k, A, rowk, colk))) return rc;
         }
-        gjm_unpermute_kernel<<<g1, 256, 0, st>>>(nn, A, ipiv);
-        h->launches += 4LL * nn + 1;
     }
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, gjm_unpermute_kernel, {g1, 256, 0, st}, nn, A, ipiv);
 }
 
 template <class T>
@@ -1553,18 +1589,15 @@ static int setup_woodbury(hpf_t* h, const DevNet& net, cudaStream_t st, int* inf
     if (!rc) rc = alloc_async(h, pr, (size_t)2 * (H + 1), st, who);
     if (rc) return rc;
     tick("allocations");
-    wb_blocks_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv.get());
-    h->launches++;
+    const unsigned g8 = h->sm_count * 8;
+    rc = launch(h, wb_blocks_kernel, {g8, 256, 0, st}, net, Dinv.get());
     for (int hh = 0; hh < H && !rc; ++hh) {
         double2* blk = hh == 0 ? Dinv.get() : Dinv.get() + (size_t)q * q + (size_t)(hh - 1) * n * n;
         rc = gj_invert(h, blk, hh == 0 ? q : n, ipiv.get(), info.get() + hh, pr.get() + 2 * hh, tmp.get(), st, FR.get());
     }
     tick("block inversions D_h");
-    if (!rc) {
-        wb_capacitance_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, Dinv.get(), Mx.get());
-        h->launches++;
-        rc = gj_invert(h, Mx.get(), qH, ipiv.get(), info.get() + H, pr.get() + 2 * H, tmp.get(), st, FR.get());
-    }
+    if (!rc) rc = launch(h, wb_capacitance_kernel, {g8, 256, 0, st}, net, Dinv.get(), Mx.get());
+    if (!rc) rc = gj_invert(h, Mx.get(), qH, ipiv.get(), info.get() + H, pr.get() + 2 * H, tmp.get(), st, FR.get());
     tick("capacitance matrix M: build + invert");
     // W_NL = (D^-1 E) M^-1, one GEMM per harmonic block: rows of block h x the rows (k, h) of M^-1
     for (int hh = 0; hh < H && !rc; ++hh) {
@@ -1577,15 +1610,9 @@ static int setup_woodbury(hpf_t* h, const DevNet& net, cudaStream_t st, int* inf
     }
     // T = D_0^-1 Y_0[nl, lin];  U = YN E^T D^-1 A_ZF;  G = W_NL U + [T; 0]
     if (!rc) rc = launch_zgemm(h, q, m, q, Dinv.get(), (size_t)q, net.Y + (size_t)m * n, (size_t)n, T.get(), (size_t)m, st);
-    if (!rc) {
-        wb_coupling_rhs_kernel<<<h->sm_count * 4, 256, 0, st>>>(net, T.get(), U.get());
-        h->launches++;
-        rc = launch_zgemm(h, nZ, m, qH, WNL, (size_t)qH, U.get(), (size_t)m, Gz, (size_t)m, st);
-    }
-    if (!rc) {
-        wb_finish_G_kernel<<<h->sm_count * 8, 256, 0, st>>>(nZ, m, q, T.get(), Gz, GzT);
-        h->launches++;
-    }
+    if (!rc) rc = launch(h, wb_coupling_rhs_kernel, {(unsigned)h->sm_count * 4, 256, 0, st}, net, T.get(), U.get());
+    if (!rc) rc = launch_zgemm(h, nZ, m, qH, WNL, (size_t)qH, U.get(), (size_t)m, Gz, (size_t)m, st);
+    if (!rc) rc = launch(h, wb_finish_G_kernel, {g8, 256, 0, st}, nZ, m, q, T.get(), Gz, GzT);
     tick("W_NL, G (tensor-core GEMMs)");
     if (rc) return rc;
     std::vector<int> hinfo((size_t)H + 1);
@@ -1744,22 +1771,17 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
     SK(AZF, (size_t)nZ * net.m * sizeof(double2));
     SK(ipiv, (size_t)(nZ + 2) * sizeof(int));
     SK(pr, 2 * sizeof(double));
-    struct_assemble_kernel<<<h->sm_count * 8, 256, 0, st>>>(net, sb.Ainv.get(), AZF.get());
-    h->launches++;
+    int rc = launch(h, struct_assemble_kernel, {(unsigned)h->sm_count * 8, 256, 0, st}, net, sb.Ainv.get(), AZF.get());
+    if (rc) return rc;
     if (nZ > h->gj_single_max) SK(tmp, ((size_t)2 * nZ + 1) * sizeof(double2));
-    const int rcg = gj_invert(h, sb.Ainv.get(), nZ, ipiv.get(), ipiv.get() + nZ, pr.get(), tmp.get(), st);
-    if (rcg) return rcg;
-    {
-        const size_t tot = (size_t)nZ * net.m;
-        struct_G_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(nZ, net.m, net.q < nZ ? net.q : nZ,
-                                                                       sb.Ainv.get(), AZF.get(), sb.Gz.get(), sb.GzT.get());
-        h->launches++;
-    }
-    if (qH > 0) {
-        const size_t tot = (size_t)nZ * qH;
-        struct_WNL_kernel<<<(unsigned)((tot + 127) / 128), 128, 0, st>>>(net, nZ, sb.Ainv.get(), sb.WNL.get());
-        h->launches++;
-    }
+    rc = gj_invert(h, sb.Ainv.get(), nZ, ipiv.get(), ipiv.get() + nZ, pr.get(), tmp.get(), st);
+    if (!rc)
+        rc = launch(h, struct_G_kernel, {(unsigned)(((size_t)nZ * net.m + 127) / 128), 128, 0, st}, nZ, net.m,
+                    net.q < nZ ? net.q : nZ, sb.Ainv.get(), AZF.get(), sb.Gz.get(), sb.GzT.get());
+    if (!rc && qH > 0)
+        rc = launch(h, struct_WNL_kernel, {(unsigned)(((size_t)nZ * qH + 127) / 128), 128, 0, st}, net, nZ, sb.Ainv.get(),
+                    sb.WNL.get());
+    if (rc) return rc;
     int info = -1;
     double prh[2] = {0.0, 0.0};
     cudaError_t e = cudaMemcpyAsync(&info, ipiv.get() + nZ, sizeof(int), cudaMemcpyDeviceToHost, st);
@@ -1790,14 +1812,9 @@ static int ensure_struct(hpf_t* h, cudaStream_t st) {
 static int launch_zgemm(hpf_t* h, int M, int N, int K, const double2* A, size_t lda, const double2* B, size_t ldb,
                         double2* C, size_t ldc, cudaStream_t st, bool subtract, const int* n_dev) {
     if (M <= 0 || N <= 0) return HPF_OK;
-    CK(cudaFuncSetAttribute(zgemm_dmma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZG_SMEM_BYTES));
-    CK(cudaFuncSetAttribute(zgemm_dmma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ZG_SMEM_BYTES));
     const dim3 grid((unsigned)((N + ZG_BN - 1) / ZG_BN), (unsigned)((M + ZG_BM - 1) / ZG_BM));
-    if (subtract) zgemm_dmma_kernel<true><<<grid, 256, ZG_SMEM_BYTES, st>>>(M, N, K, A, lda, B, ldb, C, ldc, n_dev);
-    else zgemm_dmma_kernel<false><<<grid, 256, ZG_SMEM_BYTES, st>>>(M, N, K, A, lda, B, ldb, C, ldc, n_dev);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, subtract ? zgemm_dmma_kernel<true> : zgemm_dmma_kernel<false>, {grid, 256, ZG_SMEM_BYTES, st},
+                  M, N, K, A, lda, B, ldb, C, ldc, n_dev);
 }
 
 // The generic Norton contraction w_N = W_NL I_N runs on the tensor cores for batches of at least one
@@ -1822,53 +1839,39 @@ static int launch_wn(hpf_t* h, const DevNet& net, const StructNet& sn, int B, co
     const int qH = net.q * net.H;
     if (qH == 0) { CK(cudaMemsetAsync(wa.wN, 0, (size_t)sn.nZ * B * sizeof(double2), st)); return HPF_OK; }
     if (h->shape && h->struct_state == 1 && !h->hWNL.empty()) {
-        with_shape(h->shape, [&](auto d) {
+        return with_shape(h->shape, [&](auto d) {
             using D = decltype(d);
             static_assert(sizeof(WnConsts<D>) + sizeof(WnArgs) <= 32000, "kernel parameter space");
             WnConsts<D> C;
             memcpy(C.W, h->hWNL.data(), sizeof(C.W));
-            wn_lane_kernel<D><<<(unsigned)((B + 127) / 128), 128, 0, st>>>(C, wa);
-            return 0;
+            return launch(h, wn_lane_kernel<D>, {(unsigned)((B + 127) / 128), 128, 0, st}, C, wa);
         });
-        h->launches++;
-        CK(cudaGetLastError());
-        return HPF_OK;
     }
     if (wn_use_dmma(h, sn.nZ, qH, B))
         return launch_zgemm(h, sn.nZ, B, qH, sn.WNL, (size_t)qH, I_N, (size_t)B, wa.wN, (size_t)B, st);
     const size_t smem = (size_t)(qH < HPF_WN_UCH ? qH : HPF_WN_UCH) * HPF_T * sizeof(double2) + 16;
-    int occ = 0;
-    rc = prep_kernel(h, wn_tile_kernel, smem, "hpf_solve", &occ, 256);
+    long long ctas = 0;
+    rc = resident_ctas(h, wn_tile_kernel, 256, smem, "hpf_solve", &ctas);
     if (rc) return rc;
-    const long long tiles = ((long long)B + HPF_T - 1) / HPF_T;
-    long long grid = (long long)occ * h->sm_count;
-    if (grid > tiles) grid = tiles;
+    const unsigned grid = fill_grid(h, ctas, ((long long)B + HPF_T - 1) / HPF_T, false);
     // few tiles (large networks, small batches): spread the row groups over grid.y as well
     const long long groups = (sn.nZ + 8 * HPF_WN_RPW - 1) / (8 * HPF_WN_RPW);
-    long long gy = ((long long)occ * h->sm_count + grid - 1) / grid;
+    long long gy = (ctas + grid - 1) / grid;
     if (gy > groups) gy = groups;
     if (gy < 1) gy = 1;
-    wn_tile_kernel<<<dim3((unsigned)grid, (unsigned)gy), 256, smem, st>>>(net, sn, sn.WNL, wa);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, wn_tile_kernel, {dim3(grid, (unsigned)gy), 256, smem, st}, net, sn, sn.WNL, wa);
 }
 
 template <int NW, int MINB, class D>
 static int launch_harm_t(hpf_t* h, const DevNet& net, const StructNet& sn, const HarmTileArgs& ha,
                          bool persistent, cudaStream_t st) {
     const size_t smem = harm_tile_smem_bytes(net.n, net.H, net.m, net.c, net.q, NW, sn.yn_elems);
-    int occ = 0;
-    int rc = prep_kernel(h, harm_tile_kernel<NW, MINB, D>, smem, "hpf_solve", &occ, NW * 32);
+    long long ctas = 0;
+    const int rc = resident_ctas(h, harm_tile_kernel<NW, MINB, D>, NW * 32, smem, "hpf_solve", &ctas);
     if (rc) return rc;
     const long long tiles = ((long long)ha.B + HPF_T - 1) / HPF_T;
-    long long grid = tiles;
-    if (persistent && grid > (long long)occ * h->sm_count) grid = (long long)occ * h->sm_count;
-    if (persistent && h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
-    harm_tile_kernel<NW, MINB, D><<<(unsigned)grid, NW * 32, smem, st>>>(net, sn, ha);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    const unsigned grid = persistent ? fill_grid(h, ctas, tiles, true) : (unsigned)tiles;
+    return launch(h, harm_tile_kernel<NW, MINB, D>, {grid, NW * 32, smem, st}, net, sn, ha);
 }
 
 template <class D>
@@ -1877,17 +1880,11 @@ static int launch_harm_hw(hpf_t* h, const HarmTileArgs& ha, cudaStream_t st) {
     constexpr int threads = D::H * 32;
     auto go = [&](auto kernel, const auto* C) -> int {
         static_assert(sizeof(*C) + sizeof(HarmTileArgs) <= 32000, "kernel parameter space");
-        int occ = 0;
-        int rc = prep_kernel(h, kernel, smem, "hpf_solve", &occ, threads);
+        long long ctas = 0;
+        const int rc = resident_ctas(h, kernel, threads, smem, "hpf_solve", &ctas);
         if (rc) return rc;
         const long long tiles = ((long long)ha.B + HPF_T - 1) / HPF_T;
-        long long grid = (long long)occ * h->sm_count;
-        if (grid > tiles) grid = tiles;
-        if (h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
-        kernel<<<(unsigned)grid, threads, smem, st>>>(*C, ha);
-        h->launches++;
-        CK(cudaGetLastError());
-        return HPF_OK;
+        return launch(h, kernel, {fill_grid(h, ctas, tiles, true), threads, smem, st}, *C, ha);
     };
     if (h->coupled) return go(harm_hw_kernel<D, true>, reinterpret_cast<const HwConsts<D, true>*>(h->hw_consts.data()));
     return go(harm_hw_kernel<D, false>, reinterpret_cast<const HwConsts<D, false>*>(h->hw_consts.data()));
@@ -1911,12 +1908,10 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
             return harm_cta_kernel<decltype(k)::value ? HPF_THREADS_GMEM : HPF_THREADS, decltype(k)::value == 2>;
         });
         const int threads = gst ? gthreads : HPF_THREADS;
-        int occ = 0;
-        int rc = prep_kernel(h, kernel, smem, "hpf_solve", &occ, threads);
+        long long ctas = 0;
+        int rc = resident_ctas(h, kernel, threads, smem, "hpf_solve", &ctas);
         if (rc) return rc;
-        long long grid = ha.B;
-        if ((persistent || gst) && grid > (long long)occ * h->sm_count) grid = (long long)occ * h->sm_count;
-        if (persistent && h->max_ctas && grid > h->max_ctas) grid = h->max_ctas;
+        const unsigned grid = persistent || gst ? fill_grid(h, ctas, ha.B, persistent) : (unsigned)ha.B;
         HarmTileArgs ha2 = ha;
         ha2.gstate = nullptr; ha2.gstate_stride = 0; ha2.lub_doubles = (int)lubd;
         if (gst) {
@@ -1926,10 +1921,7 @@ static int launch_harm(hpf_t* h, const DevNet& net, const StructNet& sn, const H
             if (rc) return rc;
             ha2.gstate = h->d_gstate.get(); ha2.gstate_stride = stride;
         }
-        kernel<<<(unsigned)grid, threads, smem, st>>>(net, sn, ha2);
-        h->launches++;
-        CK(cudaGetLastError());
-        return HPF_OK;
+        return launch(h, kernel, {grid, threads, smem, st}, net, sn, ha2);
     }
     if (h->shape && !h->hw_consts.empty() && !h->harm_tile_only && !ha.step_only && persistent)
         return with_shape(h->shape, [&](auto d) { return launch_harm_hw<decltype(d)>(h, ha, st); });
@@ -2000,76 +1992,49 @@ static void ls_carve_ints(LsArgs& la, char* p, int S) {
     la.perm = ip;
 }
 
-template <class K>
-static int ls_grid(hpf_t* h, K kernel, int threads, size_t smem, long long items, int* grid) {
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int occ = 0;
-    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, threads, smem));
-    if (occ < 1) return fail(h, HPF_E_UNSUPPORTED, "hpf_solve: lock-step kernel does not fit on an SM");
-    long long g = (long long)occ * h->sm_count;
-    if (g > items) g = items;
-    if (g < 1) g = 1;
-    *grid = (int)g;
-    return HPF_OK;
-}
-
 // Batched LU with partial pivoting + solve of the systems [ld x (N+1)] of all active slots
 // (ls_panel -> ls_swap_trsm -> ls_update per 32-column panel, ls_backsub).
 static int launch_ls_lu(hpf_t* h, const LsArgs& la, int cur, int N, int nwave, cudaStream_t st) {
     const size_t cap = (size_t)h->smem_optin;
+    // every kernel of the LU takes (la, cur, N, ...) and runs one CTA per item, at most the resident CTAs
+    auto go = [&](auto kernel, int threads, size_t smem, long long items, auto... args) -> int {
+        long long ctas = 0;
+        const int rc = resident_ctas(h, kernel, threads, smem, "hpf_solve", &ctas);
+        if (rc) return rc;
+        return launch(h, kernel, {fill_grid(h, ctas, items, false), (unsigned)threads, smem, st}, la, cur, N, args...);
+    };
     auto panel = [&](int k0, int left) -> int {
         const int rows = N - k0, nb = rows < LS_NB ? rows : LS_NB;
         // all-register when every row has a thread, else sub-panels of 8 columns; staged in shared memory when it fits
         const size_t want = LS_PANEL_FIXED_BYTES + (size_t)rows * nb * sizeof(double);
         const int staged = want <= cap ? 1 : 0;
         const size_t psm = staged ? want : (size_t)LS_PANEL_FIXED_BYTES;
-        int grid = 0, rc;
-        if (rows <= 512) {
-            const int T = rows <= 128 ? 128 : rows <= 256 ? 256 : 512;
-            rc = ls_grid(h, ls_panel_kernel<1, 32>, T, psm, nwave, &grid);
-            if (rc) return rc;
-            ls_panel_kernel<1, 32><<<grid, T, psm, st>>>(la, cur, N, k0, staged, left);
-        } else if (rows <= 1024) {
-            rc = ls_grid(h, ls_panel_kernel<2, 8>, 512, psm, nwave, &grid);
-            if (rc) return rc;
-            ls_panel_kernel<2, 8><<<grid, 512, psm, st>>>(la, cur, N, k0, staged, left);
-        } else {
-            rc = ls_grid(h, ls_panel_kernel<4, 8>, 512, psm, nwave, &grid);
-            if (rc) return rc;
-            ls_panel_kernel<4, 8><<<grid, 512, psm, st>>>(la, cur, N, k0, staged, left);
-        }
+        const int rc = rows <= 512 ? go(ls_panel_kernel<1, 32>, rows <= 128 ? 128 : rows <= 256 ? 256 : 512, psm, nwave, k0, staged, left)
+                     : rows <= 1024 ? go(ls_panel_kernel<2, 8>, 512, psm, nwave, k0, staged, left)
+                                    : go(ls_panel_kernel<4, 8>, 512, psm, nwave, k0, staged, left);
+        if (rc) return rc;
         g_ls_timer.mark(4);
-        h->launches++;
         return HPF_OK;
     };
     auto swap_trsm = [&](int k0, int pair) -> int {
         const int nb = (N - k0) < LS_NB ? (N - k0) : LS_NB, cr = k0 + nb;
         const int nchunk = (N + 1 - cr + LS_ST - 1) / LS_ST;
-        int grid = 0;
-        int rc = ls_grid(h, ls_swap_trsm_kernel, LS_ST, 0, (long long)nwave * nchunk, &grid);
+        const int rc = go(ls_swap_trsm_kernel, LS_ST, 0, (long long)nwave * nchunk, k0, pair);
         if (rc) return rc;
-        ls_swap_trsm_kernel<<<grid, LS_ST, 0, st>>>(la, cur, N, k0, pair);
         g_ls_timer.mark(5);
-        h->launches++;
         return HPF_OK;
     };
     auto update = [&](int K, int kb, int rlo, int clo, int chi) -> int {
         if (rlo >= N || clo > chi) return HPF_OK;
-        int grid = 0, rc;
-        auto go = [&](auto kernel, int TR, int TC, int NT) -> int {
+        auto tiles = [&](auto kernel, int TR, int TC, int NT) -> int {
             const size_t usm = ((size_t)K * (TR + 4) + (size_t)TC * (K + 4)) * sizeof(double);
-            const long long ntr = (N - rlo + TR - 1) / TR, ntc = (chi + 1 - clo + TC - 1) / TC;
-            (void)ntc;
-            rc = ls_grid(h, kernel, NT, usm, (long long)nwave * ntr, &grid);   // (strips: row tiles of the matrices)
-            if (rc) return rc;
-            kernel<<<grid, NT, usm, st>>>(la, cur, N, kb, rlo, clo, chi);
-            return HPF_OK;
+            const long long ntr = (N - rlo + TR - 1) / TR;          // (strips: row tiles of the matrices)
+            return go(kernel, NT, usm, (long long)nwave * ntr, kb, rlo, clo, chi);
         };
-        if (K == 64) rc = go(ls_update_kernel<64, 64, 64, 128, 3>, 64, 64, 128);
-        else rc = go(ls_update_kernel<32, 128, 128, 256, 2>, 128, 128, 256);
+        const int rc = K == 64 ? tiles(ls_update_kernel<64, 64, 64, 128, 3>, 64, 64, 128)
+                               : tiles(ls_update_kernel<32, 128, 128, 256, 2>, 128, 128, 256);
         if (rc) return rc;
         g_ls_timer.mark(6);
-        h->launches++;
         return HPF_OK;
     };
     int rc;
@@ -2093,13 +2058,8 @@ static int launch_ls_lu(hpf_t* h, const LsArgs& la, int cur, int N, int nwave, c
         if ((rc = update(64, k0, c2, c2, N))) return rc;
         k0 = c2;
     }
-    int grid = 0;
-    rc = ls_grid(h, ls_backsub_kernel, 256, 0, nwave, &grid);
-    if (rc) return rc;
-    ls_backsub_kernel<<<grid, 256, 0, st>>>(la, cur, N);
+    if ((rc = go(ls_backsub_kernel, 256, 0, nwave))) return rc;
     g_ls_timer.mark(7);
-    h->launches++;
-    CK(cudaGetLastError());
     return HPF_OK;
 }
 
@@ -2145,16 +2105,14 @@ static int lu_solve_batched(hpf_t* h, int N, int B, const double* J, size_t stri
     for (int b0 = 0; b0 < B; b0 += S) {
         la.b0 = b0;
         la.nwave = (B - b0 < S) ? B - b0 : S;
-        ls_init_kernel<<<(S + 255) / 256, 256, 0, st>>>(la);
-        const long long items = (long long)la.nwave * nt * nt;
-        ls_lu_load_kernel<<<(unsigned)std::min<long long>(items, (long long)h->sm_count * 8), 256, 0, st>>>(la, N, J, stride, f);
-        rc = launch_ls_lu(h, la, 0, N, la.nwave, st);
-        if (rc) return rc;
-        const long long tot = (long long)la.nwave * N;
-        ls_lu_store_kernel<<<(unsigned)std::min<long long>((tot + 255) / 256, (long long)h->sm_count * 8), 256, 0, st>>>(la, N, dx, info);
-        h->launches += 3;
+        const long long items = (long long)la.nwave * nt * nt, tot = (long long)la.nwave * N;
+        if ((rc = launch(h, ls_init_kernel, {(unsigned)(S + 255) / 256, 256, 0, st}, la))) return rc;
+        if ((rc = launch(h, ls_lu_load_kernel, {(unsigned)std::min<long long>(items, (long long)h->sm_count * 8), 256, 0, st},
+                         la, N, J, stride, f))) return rc;
+        if ((rc = launch_ls_lu(h, la, 0, N, la.nwave, st))) return rc;
+        if ((rc = launch(h, ls_lu_store_kernel, {(unsigned)std::min<long long>((tot + 255) / 256, (long long)h->sm_count * 8),
+                                                 256, 0, st}, la, N, dx, info))) return rc;
     }
-    CK(cudaGetLastError());
     return HPF_OK;
 }
 
@@ -2195,37 +2153,31 @@ static int launch_lockstep_fund(hpf_t* h, const SolveReq& r, cudaStream_t st) {
         la.state = reinterpret_cast<double*>(p);  p += state_stride * sizeof(double) * (size_t)S;
         ls_carve_ints(la, p, S);
     }
-    int g_mis = 0, g_jac = 0;
-    rc = ls_grid(h, ls_fund_mismatch_kernel, 256, 0, S, &g_mis);
-    if (rc) return rc;
-    rc = ls_grid(h, ls_fund_jac_kernel, 256, 0, S, &g_jac);
-    if (rc) return rc;
+    long long c_mis = 0, c_jac = 0;
+    if ((rc = resident_ctas(h, ls_fund_mismatch_kernel, 256, 0, "hpf_solve", &c_mis))) return rc;
+    if ((rc = resident_ctas(h, ls_fund_jac_kernel, 256, 0, "hpf_solve", &c_jac))) return rc;
+    const unsigned g_mis = fill_grid(h, c_mis, S, false), g_jac = fill_grid(h, c_jac, S, false);
     g_ls_timer.on = getenv("HPF_LS_TIMING") != nullptr && !stream_capturing(st);
     g_ls_timer.st = st;
     for (int b0 = 0; b0 < B; b0 += S) {
         la.b0 = b0;
         la.nwave = (B - b0 < S) ? B - b0 : S;
-        ls_init_kernel<<<(S + 255) / 256, 256, 0, st>>>(la);
-        h->launches++;
+        if ((rc = launch(h, ls_init_kernel, {(unsigned)(S + 255) / 256, 256, 0, st}, la))) return rc;
         g_ls_timer.mark(0);
         for (int it = 0; it <= max_f; ++it) {
             const int cur = it & 1, nxt = cur ^ 1;
-            ls_fund_mismatch_kernel<<<g_mis, 256, 0, st>>>(nf, la, cur, it == 0);
-            ls_compact_kernel<<<1, 1024, 0, st>>>(la, cur);
-            h->launches += 2;
+            if ((rc = launch(h, ls_fund_mismatch_kernel, {g_mis, 256, 0, st}, nf, la, cur, it == 0))) return rc;
+            if ((rc = launch(h, ls_compact_kernel, {1, 1024, 0, st}, la, cur))) return rc;
             g_ls_timer.mark(1);
             if (it == max_f) break;
-            ls_fund_jac_kernel<<<g_jac, 256, 0, st>>>(nf, la, nxt);
-            h->launches++;
+            if ((rc = launch(h, ls_fund_jac_kernel, {g_jac, 256, 0, st}, nf, la, nxt))) return rc;
             g_ls_timer.mark(3);
-            rc = launch_ls_lu(h, la, nxt, Nf, la.nwave, st);
-            if (rc) return rc;
+            if ((rc = launch_ls_lu(h, la, nxt, Nf, la.nwave, st))) return rc;
         }
     }
-    if (H_full > 1) flat_start_harmonics(h, nf.n, H_full, B, r.out.V_m, r.out.V_a, st);
+    if (H_full > 1 && (rc = flat_start_harmonics(h, nf.n, H_full, B, r.out.V_m, r.out.V_a, st))) return rc;
     g_ls_timer.report("fundamental stage");
     g_ls_timer.on = false;
-    CK(cudaGetLastError());
     return HPF_OK;
 }
 
@@ -2252,50 +2204,40 @@ static int launch_lockstep(hpf_t* h, const DevNet& net, const StructNet& sn, con
         ls_carve_ints(la, p, S);
     }
     la.mat_stride = mat_stride; la.state_stride = state_stride; la.ldb = lub_ld(nx);
-    int g_mis = 0, g_bor = 0;
-    rc = ls_grid(h, ls_mismatch_kernel, 256, 0, S, &g_mis);
-    if (rc) return rc;
+    long long c_mis = 0, c_bor = 0;
+    if ((rc = resident_ctas(h, ls_mismatch_kernel, 256, 0, "hpf_solve", &c_mis))) return rc;
+    if ((rc = resident_ctas(h, ls_border_kernel, 256, 0, "hpf_solve", &c_bor))) return rc;
     const long long btiles = (long long)((m - 1 + 31) / 32) * ((nx + 1 + 31) / 32);
-    rc = ls_grid(h, ls_border_kernel, 256, 0, (long long)S * btiles, &g_bor);
-    if (rc) return rc;
-    const int g_el = (int)std::min<long long>(((long long)S * m + 255) / 256, (long long)h->sm_count * 8);
+    const unsigned g_mis = fill_grid(h, c_mis, S, false), g_bor = fill_grid(h, c_bor, (long long)S * btiles, false);
+    const unsigned g_el = (unsigned)std::min<long long>(((long long)S * m + 255) / 256, (long long)h->sm_count * 8);
     g_ls_timer.on = getenv("HPF_LS_TIMING") != nullptr && !stream_capturing(st);
     g_ls_timer.st = st;
     for (int b0 = 0; b0 < r.B; b0 += S) {
         la.b0 = b0;
         la.nwave = (r.B - b0 < S) ? r.B - b0 : S;
-        ls_init_kernel<<<(S + 255) / 256, 256, 0, st>>>(la);
-        h->launches++;
+        if ((rc = launch(h, ls_init_kernel, {(unsigned)(S + 255) / 256, 256, 0, st}, la))) return rc;
         g_ls_timer.mark(0);
         for (int it = 0; it <= r.max_h; ++it) {
             const int cur = it & 1, nxt = cur ^ 1;
-            ls_mismatch_kernel<<<g_mis, 256, 0, st>>>(net, sn, la, cur, it == 0);
-            ls_compact_kernel<<<1, 1024, 0, st>>>(la, cur);
-            h->launches += 2;
+            if ((rc = launch(h, ls_mismatch_kernel, {g_mis, 256, 0, st}, net, sn, la, cur, it == 0))) return rc;
+            if ((rc = launch(h, ls_compact_kernel, {1, 1024, 0, st}, la, cur))) return rc;
             g_ls_timer.mark(1);
             if (it == r.max_h) break;
-            ls_pack_vf_kernel<<<g_el, 256, 0, st>>>(net, la, nxt);
-            h->launches++;
-            if (q > 0) {
-                rc = launch_zgemm(h, q, la.nwave, m, sn.G, (size_t)m, la.X, (size_t)S, la.U0, (size_t)S, st, false, la.nact + nxt);
-                if (rc) return rc;
-            }
+            if ((rc = launch(h, ls_pack_vf_kernel, {g_el, 256, 0, st}, net, la, nxt))) return rc;
+            if (q > 0 && (rc = launch_zgemm(h, q, la.nwave, m, sn.G, (size_t)m, la.X, (size_t)S, la.U0, (size_t)S, st, false,
+                                            la.nact + nxt))) return rc;
             g_ls_timer.mark(2);
-            ls_border_kernel<<<g_bor, 256, 0, st>>>(net, sn, la, nxt);
-            h->launches++;
+            if ((rc = launch(h, ls_border_kernel, {g_bor, 256, 0, st}, net, sn, la, nxt))) return rc;
             g_ls_timer.mark(3);
-            rc = launch_ls_lu(h, la, nxt, nx, la.nwave, st);
-            if (rc) return rc;
-            ls_uf_kernel<<<g_el, 256, 0, st>>>(net, sn, la, nxt);
-            h->launches++;
-            rc = launch_zgemm(h, nZ, la.nwave, m, sn.G, (size_t)m, la.X, (size_t)S, la.GX, (size_t)S, st, false, la.nact + nxt);
-            if (rc) return rc;
+            if ((rc = launch_ls_lu(h, la, nxt, nx, la.nwave, st))) return rc;
+            if ((rc = launch(h, ls_uf_kernel, {g_el, 256, 0, st}, net, sn, la, nxt))) return rc;
+            if ((rc = launch_zgemm(h, nZ, la.nwave, m, sn.G, (size_t)m, la.X, (size_t)S, la.GX, (size_t)S, st, false,
+                                   la.nact + nxt))) return rc;
             g_ls_timer.mark(8);
         }
     }
     g_ls_timer.report("harmonic stage");
     g_ls_timer.on = false;
-    CK(cudaGetLastError());
     return HPF_OK;
 }
 
@@ -2344,20 +2286,15 @@ static int solve_structured(hpf_t* h, const SolveReq& r, cudaStream_t st) {
         const size_t smem = per_warp * warps;
         const FundTileArgs fa = fund_tile_args(r);
         const long long tiles = ((long long)B + HPF_T - 1) / HPF_T;
-        auto launch = [&](auto kernel) -> int {
-            CK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            int occ = 0;
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kernel, warps * 32, smem));
-            if (occ < 1) return fail(h, HPF_E_UNSUPPORTED, "hpf_solve: fundamental tile kernel does not fit");
-            long long grid = (tiles + warps - 1) / warps;
-            if (grid > (long long)occ * h->sm_count) grid = (long long)occ * h->sm_count;
-            kernel<<<(unsigned)grid, warps * 32, smem, st>>>(net, fa);
-            return HPF_OK;
-        };
-        const int rcf = with_dims(h->fund_shape, [&](auto d) { return launch(fund_tile_kernel<decltype(d)>); });
+        const int rcf = with_dims(h->fund_shape, [&](auto d) {
+            const auto kernel = fund_tile_kernel<decltype(d)>;
+            long long ctas = 0;
+            const int rc = resident_ctas(h, kernel, warps * 32, smem, "hpf_solve", &ctas);
+            if (rc) return rc;
+            return launch(h, kernel, {fill_grid(h, ctas, (tiles + warps - 1) / warps, false), (unsigned)warps * 32, smem, st},
+                          net, fa);
+        });
         if (rcf) return rcf;
-        h->launches++;
-        CK(cudaGetLastError());
     }
     if (h->profiling) { CK(cudaEventRecord(h->ev[1].get(), st)); }
     // per-scenario constant w_N = A_ZZ^-1 I_N,Z, then the harmonic stage
@@ -2404,9 +2341,7 @@ static int launch_mismatch_lane(hpf_t* h, const MismatchArgs& a, cudaStream_t st
         for (int t = 0; t < per; ++t) C.YNk[k * per + t] = h->hYN[(size_t)h->hdev[k] * per + t];
     const int threads = HPF_LANE_THREADS;
     const unsigned grid = (unsigned)(((long long)a.B + threads - 1) / threads);
-    if (h->coupled) mismatch_lane_kernel<D, true><<<grid, threads, 0, st>>>(C, a);
-    else mismatch_lane_kernel<D, false><<<grid, threads, 0, st>>>(C, a);
-    return HPF_OK;
+    return launch(h, h->coupled ? mismatch_lane_kernel<D, true> : mismatch_lane_kernel<D, false>, {grid, threads, 0, st}, C, a);
 }
 
 extern "C" {
@@ -2568,11 +2503,10 @@ static int build_Y_impl(hpf_t* h, double* Y_out, void* stream) {
     ENTER_DEVICE(h);
     cudaStream_t st = (cudaStream_t)stream;
     const int total = h->n * h->H;
-    ybus_kernel<<<(total + 127) / 128, 128, 0, st>>>(h->n, h->H, h->L, h->d_harm.get(), h->d_from.get(), h->d_to.get(),
-                                                      h->d_R.get(), h->d_X.get(), h->d_G.get(), h->d_B.get(), h->d_Xsh.get(),
-                                                      h->d_tau.get(), h->d_phase.get(), h->y_flags, h->d_Y.get());
-    h->launches++;
-    CK(cudaGetLastError());
+    const int rc = launch(h, ybus_kernel, {(unsigned)(total + 127) / 128, 128, 0, st}, h->n, h->H, h->L, h->d_harm.get(),
+                          h->d_from.get(), h->d_to.get(), h->d_R.get(), h->d_X.get(), h->d_G.get(), h->d_B.get(),
+                          h->d_Xsh.get(), h->d_tau.get(), h->d_phase.get(), h->y_flags, h->d_Y.get());
+    if (rc) return rc;
     if (Y_out)
         CK(cudaMemcpyAsync(Y_out, h->d_Y.get(), (size_t)h->H * h->n * h->n * sizeof(double2),
                            cudaMemcpyDeviceToDevice, st));
@@ -2606,11 +2540,8 @@ int hpf_thd(hpf_t* h, int B, const double* V_m, double* thd, void* stream) {
     if (!V_m || !thd) return fail(h, HPF_E_INVALID, "hpf_thd: NULL buffer");
     ENTER_DEVICE(h);
     const size_t total = (size_t)h->n * B;
-    thd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(h->n, h->H, h->d_harm.get(), B,
-                                                                                    V_m, thd);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, thd_kernel, {(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream}, h->n, h->H, h->d_harm.get(),
+                  B, V_m, thd);
 }
 
 int hpf_bus_currents(hpf_t* h, int B, const double* V_m, const double* V_a, double* I_bus, void* stream) {
@@ -2621,11 +2552,8 @@ int hpf_bus_currents(hpf_t* h, int B, const double* V_m, const double* V_a, doub
     ENTER_DEVICE(h);
     const DevNet net = devnet(h);
     const size_t total = (size_t)net.nH * B;
-    bus_currents_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
-        net, B, V_m, V_a, (double2*)I_bus);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, bus_currents_kernel, {(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream}, net, B, V_m, V_a,
+                  (double2*)I_bus);
 }
 
 int hpf_set_profiling(hpf_t* h, int enabled) {
@@ -2799,20 +2727,15 @@ int hpf_ne_extract(hpf_t* h, int D, int N, const double* Vf, const double* Vh, c
         return fail(h, HPF_E_INVALID, "hpf_ne_extract: NULL buffer");
     ENTER_DEVICE(h);
     const size_t smem = ne_extract_smem_bytes(N);
-    int occ = 0;
-    int rc = prep_kernel(h, ne_extract_kernel, smem, "hpf_ne_extract", &occ, 256);
+    long long ctas = 0;
+    const int rc = resident_ctas(h, ne_extract_kernel, 256, smem, "hpf_ne_extract", &ctas);
     if (rc) return rc;
     NeExtractArgs a;
     a.D = D; a.N = N;
     a.Vf = (const double2*)Vf; a.Vh = (const double2*)Vh; a.I_f = (const double2*)I_f; a.I_h = (const double2*)I_h;
     a.Y_N_c = (double2*)Y_N_c; a.I_N_c = (double2*)I_N_c; a.Y_N_uc = (double2*)Y_N_uc; a.I_N_uc = (double2*)I_N_uc;
     a.info = info;
-    long long grid = (long long)occ * h->sm_count;
-    if (grid > D) grid = D;
-    ne_extract_kernel<<<(unsigned)grid, 256, smem, (cudaStream_t)stream>>>(a);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, ne_extract_kernel, {fill_grid(h, ctas, D, false), 256, smem, (cudaStream_t)stream}, a);
 }
 
 int hpf_fund_solve(hpf_t* h, int B, const double* P, const double* Q, double thresh_f, int max_iter_f,
@@ -2864,26 +2787,15 @@ static int launch_batch_stats(hpf_t* h, int B, const double* V_m, const int* sta
     const int n = h->n, nH = n * h->H, R = nH + 2 * n;
     if (B > 0) {
         const size_t total = (size_t)n * B;
-        thd_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(n, h->H, h->d_harm.get(), B, V_m, thd);
-        h->launches++;
-        CK(cudaGetLastError());
+        const int rc = launch(h, thd_kernel, {(unsigned)((total + 255) / 256), 256, 0, st}, n, h->H, h->d_harm.get(), B, V_m, thd);
+        if (rc) return rc;
     }
     StatsArgs a;
     a.B = B; a.R = R; a.nH = nH; a.K = K;
     a.V_m = V_m; a.thd = thd; a.status = status; a.limits = limits; a.counts = counts; a.stats = stats;
     for (int k = 0; k < HPF_STATS_MAX_Q; ++k) a.q[k] = k < K ? quantiles[k] : 0.0;
     const int cs = stats_cluster(h, R, B);
-    const size_t smem = stats_smem_bytes(K);
-    if (smem > 48 * 1024) CK(cudaFuncSetAttribute(stats_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(cs * R)); cfg.blockDim = dim3(HPF_STATS_THREADS);
-    cfg.dynamicSmemBytes = smem; cfg.stream = st; cfg.attrs = attr; cfg.numAttrs = 1;
-    CK(cudaLaunchKernelEx(&cfg, stats_kernel, a));
-    h->launches++;
-    return HPF_OK;
+    return launch(h, stats_kernel, {(unsigned)(cs * R), HPF_STATS_THREADS, stats_smem_bytes(K), st, cs}, a);
 }
 
 extern "C" {
@@ -3193,36 +3105,23 @@ static int mismatch_impl(hpf_t* h, int B, const double* V_m, const double* V_a, 
     a.B = B; a.V_m = V_m; a.V_a = V_a; a.P = P; a.Q = Q; a.I_N = (const double2*)I_N;
     a.f = f; a.err = err; a.I_inj = (double2*)I_inj;
     const int yn_elems = h->n_dev * (h->coupled ? h->H * h->H : h->H);
-    size_t smem = tile_smem_bytes(net.n, net.H, net.q, net.m, yn_elems);
-    int occ = 0;
-    if (h->shape && !h->mismatch_tile) {
-        rc = with_shape(h->shape, [&](auto d) { return launch_mismatch_lane<decltype(d)>(h, a, (cudaStream_t)stream); });
-        if (rc) return rc;
-    } else if (smem <= (size_t)h->smem_optin) {
-        const long long tiles = ((long long)B + HPF_TILE - 1) / HPF_TILE;
-        auto launch = [&](auto kernel) -> int {
-            int rc2 = prep_kernel(h, kernel, smem, "hpf_mismatch", &occ);
-            if (rc2) return rc2;
-            // one CTA per 32-scenario tile: the hardware scheduler balances the tail (a persistent
-            // grid of occ*SMs CTAs quantises 2048 tiles into 4 rounds of 592, 13 % idle)
-            long long grid = tiles;
-            (void)occ;
-            kernel<<<(unsigned)grid, HPF_THREADS, smem, (cudaStream_t)stream>>>(net, a, yn_elems);
-            return HPF_OK;
-        };
-        rc = with_dims(h->shape, [&](auto d) { return launch(mismatch_tile_kernel<decltype(d)>); });
-        if (rc) return rc;
-    } else {
-        smem = scn_smem_bytes(net.n, net.H, net.q, net.N, false);
-        rc = prep_kernel(h, mismatch_cta_kernel, smem, "hpf_mismatch", &occ);
-        if (rc) return rc;
-        long long grid = (long long)occ * h->sm_count;
-        if (grid > B) grid = B;
-        mismatch_cta_kernel<<<(unsigned)grid, HPF_THREADS, smem, (cudaStream_t)stream>>>(net, a);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t smem = tile_smem_bytes(net.n, net.H, net.q, net.m, yn_elems);
+    if (h->shape && !h->mismatch_tile)
+        return with_shape(h->shape, [&](auto d) { return launch_mismatch_lane<decltype(d)>(h, a, st); });
+    if (smem <= (size_t)h->smem_optin) {
+        // one CTA per 32-scenario tile: the hardware scheduler balances the tail (a persistent
+        // grid of occ*SMs CTAs quantises 2048 tiles into 4 rounds of 592, 13 % idle)
+        const unsigned tiles = (unsigned)(((long long)B + HPF_TILE - 1) / HPF_TILE);
+        return with_dims(h->shape, [&](auto d) {
+            return launch(h, mismatch_tile_kernel<decltype(d)>, {tiles, HPF_THREADS, smem, st}, net, a, yn_elems);
+        });
     }
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    const size_t csmem = scn_smem_bytes(net.n, net.H, net.q, net.N, false);
+    long long ctas = 0;
+    rc = resident_ctas(h, mismatch_cta_kernel, HPF_THREADS, csmem, "hpf_mismatch", &ctas);
+    if (rc) return rc;
+    return launch(h, mismatch_cta_kernel, {fill_grid(h, ctas, B, false), HPF_THREADS, csmem, st}, net, a);
 }
 
 int hpf_mismatch(hpf_t* h, int B, const double* V_m, const double* V_a, const double* P, const double* Q,
@@ -3241,25 +3140,15 @@ static int jacobian_impl(hpf_t* h, int B, const double* V_m, const double* V_a, 
     const DevNet net = devnet(h);
     JacobianArgs a;
     a.B = B; a.V_m = V_m; a.V_a = V_a; a.J = J; a.stride = hpf_jacobian_stride(h);
-    size_t smem = jac_smem_bytes(net.n, net.H, net.q, net.N, a.stride);
-    int occ = 0;
-    if (smem <= (size_t)h->smem_optin) {
-        rc = prep_kernel(h, jacobian_kernel, smem, "hpf_jacobian", &occ, HPF_JAC_THREADS);
-        if (rc) return rc;
-        long long grid = (long long)occ * h->sm_count;
-        if (grid > B) grid = B;
-        jacobian_kernel<<<(unsigned)grid, HPF_JAC_THREADS, smem, (cudaStream_t)stream>>>(net, a);
-    } else {
-        smem = scn_smem_bytes(net.n, net.H, net.q, net.N, false);
-        rc = prep_kernel(h, jacobian_gmem_kernel, smem, "hpf_jacobian", &occ);
-        if (rc) return rc;
-        long long grid = (long long)occ * h->sm_count;
-        if (grid > B) grid = B;
-        jacobian_gmem_kernel<<<(unsigned)grid, HPF_THREADS, smem, (cudaStream_t)stream>>>(net, a);
-    }
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    const size_t smem = jac_smem_bytes(net.n, net.H, net.q, net.N, a.stride);
+    const bool in_smem = smem <= (size_t)h->smem_optin;
+    const auto kernel = in_smem ? jacobian_kernel : jacobian_gmem_kernel;
+    const int threads = in_smem ? HPF_JAC_THREADS : HPF_THREADS;
+    const size_t ksmem = in_smem ? smem : scn_smem_bytes(net.n, net.H, net.q, net.N, false);
+    long long ctas = 0;
+    rc = resident_ctas(h, kernel, threads, ksmem, "hpf_jacobian", &ctas);
+    if (rc) return rc;
+    return launch(h, kernel, {fill_grid(h, ctas, B, false), (unsigned)threads, ksmem, (cudaStream_t)stream}, net, a);
 }
 
 int hpf_jacobian(hpf_t* h, int B, const double* V_m, const double* V_a, double* J, void* stream) {
@@ -3280,23 +3169,19 @@ static int lu_solve_impl(hpf_t* h, int B, const double* J, const double* f, doub
     a.lu_classic = h->lu_classic;
     const auto kernel = with_lu_kind(lu.kind, [](auto k) { return lu_solve_kernel<decltype(k)::value>; });
     const int threads = lu.kind ? HPF_THREADS_GMEM : HPF_THREADS;
-    int occ = 0;
-    rc = prep_kernel(h, kernel, lu.smem, "hpf_lu_solve", &occ, threads);
+    long long ctas = 0;
+    rc = resident_ctas(h, kernel, threads, lu.smem, "hpf_lu_solve", &ctas);
     if (rc) return rc;
     if (lu.kind && use_lockstep(h, net.N, B))
         return lu_solve_batched(h, net.N, B, J, a.stride, f, dx, info, (cudaStream_t)stream);
-    long long grid = (long long)occ * h->sm_count;
-    if (grid > B) grid = B;
+    const unsigned grid = fill_grid(h, ctas, B, false);
     a.workspace = nullptr;
     if (lu.kind) {
         rc = grow(h, h->d_work, (size_t)grid * lub_ld(net.N) * (net.N + 1) * sizeof(double), "hpf_lu_solve: LU workspace");
         if (rc) return rc;
         a.workspace = h->d_work.get();
     }
-    kernel<<<(unsigned)grid, threads, lu.smem, (cudaStream_t)stream>>>(net, a);
-    h->launches++;
-    CK(cudaGetLastError());
-    return HPF_OK;
+    return launch(h, kernel, {grid, (unsigned)threads, lu.smem, (cudaStream_t)stream}, net, a);
 }
 
 int hpf_lu_solve(hpf_t* h, int B, const double* J, const double* f, double* dx, int* info, void* stream) {

@@ -250,65 +250,13 @@ __global__ void gjm_elim_kernel(int n, int k, double2* __restrict__ A, const dou
 }
 
 // ---- blocked variant (panels of GJB_NB pivots): the pivot steps of a panel touch only the panel's
-// columns [j0, j1) (the three kernels below); every other column receives the panel's GJB_NB rank-1
+// columns [j0, j1) (gjb_pivot_row_kernel, gjb_col_elim_kernel); every other column receives the panel's GJB_NB rank-1
 // updates at once, A -= F R, as one complex GEMM on the tensor cores (hpf_zgemm.cuh).  With column k
 // of the pivot step reset to e_k, a Gauss-Jordan step IS a rank-1 update A -= f r^T over all rows when
 // f_k = a_kk - 1 (a_kk the pivot), f_i = a_ik otherwise, r = (row k) / a_kk:
 //   F [n x NB]  f of every step of the panel (rows interchanged along with the matrix rows),
 //   R [NB x n]  the scaled pivot rows on the other columns: R_t = (a_{k_t,:} - sum_{s<t} F[k_t][s] R_s) / a_kk.
 #define GJB_NB 64
-
-// pivot row of step t = k - j0 on the panel's columns; earlier columns of F follow the interchange
-__global__ void gjb_row_kernel(int n, int k, int j0, int j1, double2* __restrict__ A, const int* __restrict__ ipiv,
-                               const double2* __restrict__ pinv_in, double2* __restrict__ rowk,
-                               double2* __restrict__ F, double2* __restrict__ pinv_all) {
-    const int j = j0 + blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= j1) return;
-    const int p = ipiv[k], t = k - j0;
-    const double2 pinv = pinv_in[0];
-    const double2 tk = A[(size_t)k * n + j], tp = A[(size_t)p * n + j];
-    const double2 a = (j == k) ? make_double2(1.0, 0.0) : tp;
-    const double2 v = cmul(a, pinv);
-    A[(size_t)k * n + j] = v;
-    if (p != k) A[(size_t)p * n + j] = tk;
-    rowk[j - j0] = v;
-    const int s = j - j0;
-    if (s < t && p != k) {                                   // F rows k <-> p of the panel's earlier steps
-        const double2 fk = F[(size_t)k * GJB_NB + s], fp = F[(size_t)p * GJB_NB + s];
-        F[(size_t)k * GJB_NB + s] = fp;
-        F[(size_t)p * GJB_NB + s] = fk;
-    }
-    if (j == k) pinv_all[t] = pinv;
-}
-
-// column k after the interchange: multipliers of the panel's own elimination + column t of F
-__global__ void gjb_col_kernel(int n, int k, int j0, const double2* __restrict__ A, const int* __restrict__ ipiv,
-                               const double2* __restrict__ pinv_in, double2* __restrict__ colk,
-                               double2* __restrict__ F) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const double2 a = A[(size_t)i * n + k];
-    colk[i] = (i == k) ? make_double2(0.0, 0.0) : a;
-    double2 f = a;
-    if (i == k) {                                            // a_kk - 1 (row k already holds 1 / a_kk at column k)
-        const double2 piv = crecip(pinv_in[0]);
-        f = make_double2(piv.x - 1.0, piv.y);
-    }
-    F[(size_t)i * GJB_NB + (k - j0)] = f;
-}
-
-__global__ void gjb_elim_kernel(int n, int k, int j0, int j1, double2* __restrict__ A, const double2* __restrict__ rowk,
-                                const double2* __restrict__ colk) {
-    const int j = j0 + threadIdx.x;                          // blockDim.x = GJB_NB
-    if (j >= j1) return;
-    const double2 r = rowk[j - j0];
-    for (int i = blockIdx.x * blockDim.y + threadIdx.y; i < n; i += gridDim.x * blockDim.y) {
-        if (i == k) continue;
-        const double2 f = colk[i];
-        double2* a = A + (size_t)i * n + j;
-        *a = (j == k) ? cneg(cmul(f, r)) : csub(*a, cmul(f, r));
-    }
-}
 
 // The two kernels of a blocked pivot step (the set-up is bound by the NUMBER of launches - ~6 us each,
 // 12,400 pivots for the 1000-bus configuration - so pivot search + pivot row are one launch, multiplier
@@ -357,7 +305,7 @@ gjb_pivot_row_kernel(int n, int k, int j0, int j1, double2* __restrict__ A, int*
         }
     }
     __syncthreads();
-    // pivot row on the panel's columns (see gjb_row_kernel)
+    // pivot row of step t = k - j0 on the panel's columns; earlier columns of F follow the interchange
     const int j = j0 + tid;
     if (j < j1) {
         const int p = sp, t = k - j0;
